@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- one advect+project frame of the HNanoSolver hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0). A "step" is one full frame over one synthetic sparse smoke domain:
   metric  : active voxel-updates/s  (N_voxels / frame time), BASELINE.json's metric
@@ -224,6 +224,21 @@ def frame_quality(sim) -> dict:
             "div_rms_after": float(np.sqrt(d / max(sim.n, 1)))}
 
 
+DUMP_VOXELS = 1 << 20     # 8 B of index + 4 B per float of velocity and scalars each: 40 MB with config 4's five scalar fields
+
+
+def dump_outputs(directory: str, sim, names) -> None:
+    """--dump-outputs: what the last timed frame hands back, the velocity (N, 3) and each scalar field (N), as float32 .npy files, at
+    DUMP_VOXELS voxels drawn with a fixed seed (all of them on smaller domains); voxel_index.npy (float64) says which voxels."""
+    os.makedirs(directory, exist_ok=True)
+    n = sim.n
+    idx = np.arange(n) if n <= DUMP_VOXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_VOXELS, replace=False))
+    np.save(os.path.join(directory, "voxel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(directory, "velocity.npy"), sim.velocity()[idx])
+    for i, name in enumerate(names):
+        np.save(os.path.join(directory, f"{name}.npy"), sim.scalar(i)[idx])
+
+
 # ----------------------------------------------------------------------------------------------------------------
 # CPU baseline (oracle port) on a bounded sample
 # ----------------------------------------------------------------------------------------------------------------
@@ -269,6 +284,8 @@ def main():
                     help="pressure solve of the timed frame: the reference's I red-black SOR iterations (default; bit-exact with the reference) or "
                          "multigrid V-cycles to a relative Poisson residual of 1e-4 (default for --workload c3, BASELINE.json config 3)")
     ap.add_argument("--mg-cycles", type=int, default=0, help="fixed number of V(2,2) cycles instead of solving to 1e-4")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the velocity and scalar fields of the last timed frame (a seeded sample of voxels) to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -280,6 +297,8 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: hnanosolver_b200 has no CPU fallback")
     torch.cuda.set_device(local_rank)
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        raise SystemExit("--dump-outputs: single-GPU runs of this implementation only")
     if args.impl == "reference":  # rank 0 alone times the reference; the other ranks leave without joining a process group
         return reference_arm(args, rank, world)
     if world > 1:
@@ -351,6 +370,8 @@ def main():
     launches = int(_lib.lib().hns_launch_count())
     packed_launches = int(_lib.lib().hns_packed_advection_launches() - packed0)
     clocks = sampler.stop(tc0, tc1)
+    if args.dump_outputs:       # every timed frame starts from the same inputs: the state now holds the last one's result
+        dump_outputs(args.dump_outputs, sim, names)
     ms_step = ms_total / args.steps
     value = N / (ms_step * 1e-3)
     solve_quality = frame_quality(sim)          # relative Poisson residual + ||div u_new|| of the frame just timed

@@ -1,5 +1,13 @@
 """Shared helpers of the parity tests."""
+import importlib.util
+import os
+
 import numpy as np
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+_spec = importlib.util.spec_from_file_location("make_golden", os.path.join(GOLDEN, "make_golden.py"))
+make_golden = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(make_golden)
 
 # Tolerance of the north star: advected / projected fields within 1e-5 relative of the reference kernels.
 # "Relative" is measured against the field's max magnitude (a voxel-wise relative error is meaningless at zero crossings).
@@ -39,3 +47,89 @@ def nanovdb_compare_mask(nbytes: int, num_tiles: int) -> np.ndarray:
         tile = root + 96 + 32 * t
         m[tile + 20:tile + 32] = False      # padding after state + the untouched tile value
     return m
+
+
+class Golden:
+    """One fixture of tests/golden (make_golden.compact): the reference's inputs, regenerated and checked against their digests, and
+    its outputs, each held as values at a sample of voxels plus the SHA-256 of the whole array."""
+
+    def __init__(self, name: str):
+        z = np.load(os.path.join(GOLDEN, f"ref_{name}.npz"))
+        self._z = {k: z[k] for k in z.files}
+        self._arrays = {k: v for k, v in self._z.items() if "." not in k}
+        for k, v in make_golden.case_arrays(name).items():
+            assert make_golden.digest(v) == self.sha256(k), f"regenerated input {k} is not the one the reference was given"
+            self._arrays[k] = v
+
+    def __contains__(self, key: str) -> bool:
+        return key in self._arrays or key + ".sha256" in self._z
+
+    def __getitem__(self, key: str) -> np.ndarray:
+        """a parameter, the index grid or an input; outputs are only compared, through check / matches"""
+        return self._arrays[key]
+
+    def sha256(self, key: str) -> str:
+        return str(self._z[key + ".sha256"])
+
+    def matches(self, a, key: str) -> bool:
+        """`a` equals output `key` value for value (+0.0 == -0.0)"""
+        return make_golden.digest(a) == self.sha256(key)
+
+    def check(self, a, key: str, what: str):
+        """assert_close of `a` and output `key` on the stored sample of voxels, then bitwise equality of the whole array"""
+        a = np.asarray(a)
+        assert_close(a[self._z["sample_index"]], self._z[key + ".sample"], what)
+        assert self.matches(a, key), f"{what}: equal on the sample of {self._z['sample_index'].size} voxels but not everywhere (SHA-256 differs)"
+
+
+class Recording:
+    """Outputs of the reference's own kernels and launchers by key (tests/golden/ref_recorded.npz), each held as its values at a seeded
+    sample of rows plus the SHA-256 of the whole array, and per key the digest of the inputs they were computed from.
+
+    With HNS_RECORD_REFERENCE=1 and the reference build present (oracle/_ref), `record` stores the reference's own output and `save`
+    merges what a run recorded into the file. The file as committed was recorded on a B200 from this project's CUDA path at a state
+    whose kernels, input generator and test inputs equal those of commit a7bb57e, where every one of these comparisons had passed bit
+    for bit against the live reference (profiles/r2f_gpu_tests_final.log). Its vorticity outputs for the two cases the golden fixtures
+    share (random28 = soup, sphere32 = sphere) agree bit for bit with those fixtures, which come from the reference itself."""
+
+    SAMPLE = 32
+
+    def __init__(self, path: str):
+        self.path = path
+        self.recording = os.environ.get("HNS_RECORD_REFERENCE") == "1"
+        self._z = {}
+        if os.path.exists(path):
+            z = np.load(path)
+            self._z = {k: z[k] for k in z.files}
+
+    @classmethod
+    def _rows(cls, n: int) -> np.ndarray:
+        return np.sort(np.random.default_rng(7).choice(n, min(n, cls.SAMPLE), replace=False))
+
+    @staticmethod
+    def _inputs_digest(arrays) -> str:
+        return make_golden.digest(np.array([make_golden.digest(a) for a in arrays]))
+
+    def record_inputs(self, key: str, arrays):
+        self._z[key + "/inputs.sha256"] = np.array(self._inputs_digest(arrays))
+
+    def record(self, want, key: str):
+        want = np.asarray(want)
+        self._z[key + ".sample"], self._z[key + ".sha256"] = want[self._rows(len(want))], np.array(make_golden.digest(want))
+
+    def check_inputs(self, key: str, arrays):
+        """the recorded outputs under `key` apply only to the inputs they were computed from"""
+        assert key + "/inputs.sha256" in self._z, f"no recorded reference outputs for {key}"
+        assert self._inputs_digest(arrays) == str(self._z[key + "/inputs.sha256"]), \
+            f"{key}: the inputs differ from those the recorded reference outputs were computed from (input generator or numpy changed)"
+
+    def check(self, a, key: str, what: str):
+        a = np.asarray(a)
+        idx = self._rows(len(a))
+        assert key + ".sha256" in self._z, f"{what}: no recorded reference output {key}"
+        assert_close(a[idx], self._z[key + ".sample"], what)
+        assert make_golden.digest(a) == str(self._z[key + ".sha256"]), \
+            f"{what}: equal on the sample of {idx.size} rows but not everywhere (SHA-256 differs)"
+
+    def save(self):
+        np.savez_compressed(self.path, **self._z)

@@ -1,6 +1,7 @@
 """GPU parity tests: the CUDA path, called through the C ABI (hnanosolver_b200.launchers -> ctypes -> libhns_b200.so), against
-(1) the CPU oracle, (2) the committed golden fixtures, (3) the unmodified reference kernels / launchers running live on the
-same GPU (oracle/_ref/libhns_ref.so, when it travelled with the snapshot), and (4) size-independent properties at full size.
+(1) the CPU oracle, (2) the committed golden fixtures, (3) the unmodified reference kernels / launchers: live on the same GPU when
+their build (oracle/_ref/libhns_ref.so) is present, else what they computed on the same inputs (tests/golden/ref_recorded.npz), and
+(4) size-independent properties at full size.
 
 Bar (north star): index topology bit-exact; fields within 1e-5 relative (helpers.REL_TOL) of the reference kernels.
 """
@@ -10,15 +11,56 @@ import numpy as np
 import pytest
 
 import hnanosolver_b200 as H
-from helpers import REL_TOL, assert_close, nanovdb_compare_mask, rel_err
+from helpers import GOLDEN, Golden, Recording, assert_close, nanovdb_compare_mask, rel_err
 from hnanosolver_b200 import synth
 from hnanosolver_b200.grid_data import FLOAT, VEC3F, GridIndexedData
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
-needs_ref = pytest.mark.skipif(not O.ref_gpu_available(), reason="oracle/_ref/libhns_ref.so not present")
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 PARAMS6 = np.array([0.5, 2.0, 1.5, 0.1, 0.0, 1.0], np.float32)
+RECORDED = Recording(os.path.join(GOLDEN, "ref_recorded.npz"))
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _save_recording():
+    yield
+    if RECORDED.recording:
+        RECORDED.save()
+
+
+class Reference:
+    """The reference's outputs under `key` (test, case, parameters) for `inputs`: `live()` runs its own kernels and launchers when their
+    build is present (and, with HNS_RECORD_REFERENCE=1, records what they return); otherwise the recording of what they computed from
+    the same inputs stands in (helpers.Recording)."""
+
+    def __init__(self, key: str, live, inputs):
+        self.key, self.want = key, None
+        if O.ref_gpu_available():
+            self.want = live()
+            if RECORDED.recording:
+                RECORDED.record_inputs(key, inputs)
+        elif RECORDED.recording:
+            pytest.fail("recording the reference's outputs needs its build (oracle/_ref/libhns_ref.so)")
+        else:
+            RECORDED.check_inputs(key, inputs)
+
+    def check(self, got, name: str, what: str):
+        if self.want is None:
+            RECORDED.check(got, f"{self.key}/{name}", what)
+            return
+        assert_close(got, self.want[name], what)
+        if RECORDED.recording:
+            RECORDED.record(self.want[name], f"{self.key}/{name}")
+
+
+def _copies(rd):
+    return {k: v.copy() for k, v in rd.blocks.items()}
+
+
+def _masked_nanovdb(buf):
+    """voxelsToGrid's buffer with the bytes it leaves uninitialised zeroed (helpers.nanovdb_compare_mask)"""
+    T = int(np.frombuffer(buf[672 + 40:672 + 44].tobytes(), np.uint32)[0])
+    return np.where(nanovdb_compare_mask(buf.size, T), buf, 0).astype(np.uint8)
 
 
 def small_cases():
@@ -61,20 +103,19 @@ def test_index_grid_matches_oracle_bit_exact(case):
     assert np.array_equal(g.get_values(w.coords), np.arange(1, w.num_voxels + 1, dtype=np.uint64))
 
 
-@needs_ref
 def test_index_grid_matches_reference_voxelsToGrid(case):
     w = case
     g = H.create_index_grid_from_origins(w.origins, w.voxel_size)
-    rd = O.RefData(w.coords)
-    rg = O.RefGrid(rd, w.voxel_size)
-    ref, mine = rg.buffer(), g.nanovdb_buffer()
-    assert ref.size == mine.size
-    T = int(np.frombuffer(ref[672 + 40:672 + 44].tobytes(), np.uint32)[0])
-    bad = np.nonzero((ref != mine) & nanovdb_compare_mask(ref.size, T))[0]
-    assert bad.size == 0, f"NanoVDB buffer differs from voxelsToGrid at bytes {bad[:16]}"
     rng = np.random.default_rng(1)
     q = np.concatenate([w.coords[::2], w.coords[::3] + rng.integers(-12, 13, size=w.coords[::3].shape).astype(np.int32)])
-    assert np.array_equal(g.get_values(q), rg.get_values(q))
+
+    def live():
+        rg = O.RefGrid(O.RefData(w.coords), w.voxel_size)
+        return dict(nanovdb=_masked_nanovdb(rg.buffer()), values=rg.get_values(q))
+
+    ref = Reference(f"index_grid/{w.name}", live, [w.coords, q])
+    ref.check(_masked_nanovdb(g.nanovdb_buffer()), "nanovdb", "NanoVDB buffer vs voxelsToGrid")
+    ref.check(g.get_values(q), "values", "getValue")
 
 
 def test_neighbor_table(case):
@@ -133,28 +174,35 @@ def test_sweep_direction_does_not_change_the_bits(case):
         assert np.array_equal(a[k], b[k]), k
 
 
-@needs_ref
-def test_frame_stages_match_reference_kernels(case):
-    w = case
-    I = 9
+def _ref_frame(w, iterations):
+    """the reference's north-star frame on its own kernels: adv, div, p, vel, scalar{i} and the divergence norm of vel"""
     rd = O.RefData(w.coords)
     rd.add_vec3("vel", w.velocity)
     for n, a in zip(w.scalar_names, w.scalars):
         rd.add_float(n, a)
     rg = O.RefGrid(rd, w.voxel_size)
     rf = O.RefFrame(rd, rg, w.scalar_names)
-    rf.run(I, w.dt, w.voxel_size, 1)
+    rf.run(iterations, w.dt, w.voxel_size, 1)
     want = rf.download()
+    want.update({f"scalar{i}": s for i, s in enumerate(want.pop("scalars"))}, div_norm=_div_norm(w, want["vel"]))
+    return want
+
+
+def _div_norm(w, vel):
+    return np.array([np.sqrt(np.mean(O.OracleIndex(w.coords).divergence(vel, w.voxel_size).astype(np.float64) ** 2))])
+
+
+def test_frame_stages_match_reference_kernels(case):
+    w = case
+    I = 9
     got = run_product_frame(w, I)
+    ref = Reference(f"frame/{w.name}", lambda: _ref_frame(w, I), [w.coords, w.velocity, *w.scalars])
     for k in ("adv", "div", "p", "vel"):
-        assert_close(got[k], want[k], k)
+        ref.check(got[k], k, k)
     for i in range(len(w.scalars)):
-        assert_close(got["scalars"][i], want["scalars"][i], f"scalar {i}")
+        ref.check(got["scalars"][i], f"scalar{i}", f"scalar {i}")
     # divergence L2 norm of the projected velocity agrees with the reference's (BASELINE.md parity gate)
-    ix = O.OracleIndex(w.coords)
-    n_got = np.sqrt(np.mean(ix.divergence(got["vel"], w.voxel_size).astype(np.float64) ** 2))
-    n_ref = np.sqrt(np.mean(ix.divergence(want["vel"], w.voxel_size).astype(np.float64) ** 2))
-    assert abs(n_got - n_ref) <= REL_TOL * n_ref
+    ref.check(_div_norm(w, got["vel"]), "div_norm", "||div u|| of the projected velocity")
 
 
 def test_far_samples_take_the_tree_walk_path():
@@ -265,22 +313,27 @@ def test_compute_sim_equals_the_resident_frame_bitwise(case, order):
         assert np.array_equal(d.pValues(FLOAT, k), sim.scalar(i)), k
 
 
-@needs_ref
-def test_compute_sim_matches_reference_compute_sim(case):
-    w = case
-    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
+def _ref_compute_sim(w, fields, iterations, params, has_collision=False):
+    """the reference's CreateIndexGrid + Compute_Sim on a copy of the sidecar: every block afterwards"""
     rd = O.RefData(w.coords)
     rd.add_vec3("vel", w.velocity)
     for k, v in fields.items():
         rd.add_float(k, v)
     rg = O.RefGrid(rd, w.voxel_size)
-    O.ref_compute_sim(rd, rg, 8, w.dt, w.voxel_size, PARAMS6, False)
+    O.ref_compute_sim(rd, rg, iterations, w.dt, w.voxel_size, params, has_collision)
+    return _copies(rd)
+
+
+def test_compute_sim_matches_reference_compute_sim(case):
+    w = case
+    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
     d = _sidecar(w, fields)
     g = H.CreateIndexGrid(d, w.voxel_size)
     H.Compute_Sim(d, g, 8, w.dt, w.voxel_size, H.CombustionParams(*PARAMS6.tolist()), False)
-    assert_close(d.pValues(VEC3F, "vel"), rd.blocks["vel"], "Compute_Sim velocity")
+    ref = Reference(f"compute_sim/{w.name}", lambda: _ref_compute_sim(w, fields, 8, PARAMS6), [w.coords, w.velocity, *fields.values()])
+    ref.check(d.pValues(VEC3F, "vel"), "vel", "Compute_Sim velocity")
     for k in fields:
-        assert_close(d.pValues(FLOAT, k), rd.blocks[k], f"Compute_Sim {k}")
+        ref.check(d.pValues(FLOAT, k), k, f"Compute_Sim {k}")
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -310,20 +363,22 @@ def test_vorticity_confinement_matches_oracle(case, scale, factor_scale):
     assert not np.array_equal(got, w.velocity) or w.num_leaves == 1
 
 
-@needs_ref
 @pytest.mark.parametrize("scale,factor_scale", VORTICITY_CASES[:4])
 def test_vorticity_confinement_matches_reference_kernel_out_of_place(case, scale, factor_scale):
     """The reference kernel itself, given separate input and output buffers (Compute() passes the same buffer twice and races)."""
     w = case
-    rd = O.RefData(w.coords)
-    rd.add_vec3("vel", w.velocity)
-    for n, a in zip(w.scalar_names, w.scalars):
-        rd.add_float(n, a)
-    rg = O.RefGrid(rd, w.voxel_size)
-    want = O.RefFrame(rd, rg, w.scalar_names).vorticity(w.dt, w.voxel_size, scale, factor_scale)
+
+    def live():
+        rd = O.RefData(w.coords)
+        rd.add_vec3("vel", w.velocity)
+        for n, a in zip(w.scalar_names, w.scalars):
+            rd.add_float(n, a)
+        rg = O.RefGrid(rd, w.voxel_size)
+        return dict(vel=O.RefFrame(rd, rg, w.scalar_names).vorticity(w.dt, w.voxel_size, scale, factor_scale))
+
     _, got = _product_vorticity(w, scale, factor_scale)
-    assert_close(got, want, "vorticityConfinement")
-    assert np.array_equal(got, want), "expected bit-exact agreement with the reference kernel"
+    ref = Reference(f"vorticity/{w.name}/{scale}/{factor_scale}", live, [w.coords, w.velocity, *w.scalars])
+    ref.check(got, "vel", "vorticityConfinement")
 
 
 def test_vorticity_identity_cases(case):
@@ -354,7 +409,6 @@ def test_compute_sim_with_vorticity_matches_oracle(case):
         assert not np.array_equal(want_vel, off_vel)
 
 
-@needs_ref
 def test_compute_sim_default_sop_vorticity_parameters_match_reference(case):
     """SOP defaults: vorticity 1, factor_scale 0.5 (SOP_HNanoSolver.cpp:73-86). The offset truncates to 0, the in-place race of the
     reference is then harmless, and both sides must agree."""
@@ -362,18 +416,13 @@ def test_compute_sim_default_sop_vorticity_parameters_match_reference(case):
     params = PARAMS6.copy()
     params[4], params[5] = 1.0, 0.5
     fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
-    rd = O.RefData(w.coords)
-    rd.add_vec3("vel", w.velocity)
-    for k, v in fields.items():
-        rd.add_float(k, v)
-    rg = O.RefGrid(rd, w.voxel_size)
-    O.ref_compute_sim(rd, rg, 6, w.dt, w.voxel_size, params, False)
     d = _sidecar(w, fields)
     g = H.CreateIndexGrid(d, w.voxel_size)
     H.Compute_Sim(d, g, 6, w.dt, w.voxel_size, H.CombustionParams(*params.tolist()), False)
-    assert_close(d.pValues(VEC3F, "vel"), rd.blocks["vel"], "Compute_Sim velocity")
+    ref = Reference(f"compute_sim_sop_default/{w.name}", lambda: _ref_compute_sim(w, fields, 6, params), [w.coords, w.velocity, *fields.values()])
+    ref.check(d.pValues(VEC3F, "vel"), "vel", "Compute_Sim velocity")
     for k in fields:
-        assert_close(d.pValues(FLOAT, k), rd.blocks[k], f"Compute_Sim {k}")
+        ref.check(d.pValues(FLOAT, k), k, f"Compute_Sim {k}")
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -448,21 +497,15 @@ def test_compute_sim_with_collision_matches_oracle(case):
     assert not d0.pValues(FLOAT, "collision_sdf").any()
 
 
-@needs_ref
 def test_compute_sim_with_collision_matches_reference(case):
     w = case
     fields, d = _compute_sim_collision(w, True, iterations=7)
-    rd = O.RefData(w.coords)
-    rd.add_vec3("vel", w.velocity)
-    for k, v in fields.items():
-        rd.add_float(k, v)
-    rg = O.RefGrid(rd, w.voxel_size)
-    O.ref_compute_sim(rd, rg, 7, w.dt, w.voxel_size, PARAMS6, True)
-    assert_close(d.pValues(VEC3F, "vel"), rd.blocks["vel"], "Compute_Sim(hasCollision) velocity")
-    assert np.array_equal(d.pValues(VEC3F, "vel"), rd.blocks["vel"])
+    ref = Reference(f"compute_sim_collision/{w.name}", lambda: _ref_compute_sim(w, fields, 7, PARAMS6, True),
+                    [w.coords, w.velocity, *fields.values()])
+    ref.check(d.pValues(VEC3F, "vel"), "vel", "Compute_Sim(hasCollision) velocity")
     for k in fields:
         if k != "collision_sdf":
-            assert_close(d.pValues(FLOAT, k), rd.blocks[k], f"Compute_Sim(hasCollision) {k}")
+            ref.check(d.pValues(FLOAT, k), k, f"Compute_Sim(hasCollision) {k}")
 
 
 @pytest.mark.parametrize("name", ["soup", "sphere"])
@@ -470,8 +513,8 @@ def test_collision_against_golden_reference_outputs(name):
     path = os.path.join(GOLDEN, f"ref_{name}.npz")
     if not os.path.exists(path):
         pytest.skip("no golden fixture")
-    z = np.load(path)
-    if "collision_sdf" not in z.files:
+    z = Golden(name)
+    if "collision_sdf" not in z:
         pytest.skip("fixture predates the collision vectors")
     origins, h, dt, I = z["origins"], float(z["voxel_size"]), float(z["dt"]), int(z["iterations"])
     S = len(z["scalar_names"])
@@ -481,11 +524,11 @@ def test_collision_against_golden_reference_outputs(name):
     sim.set_collision(S)
     sim.enforce_collision()
     sim.sync()
-    assert np.array_equal(sim.velocity(), z["coll_enforce"])
+    z.check(sim.velocity(), "coll_enforce", "enforceCollisionBoundaries")
     sim.upload(z["velocity"], [z[f"scalar{i}"] for i in range(S)] + [z["collision_sdf"]])
     sim.advect_velocity(dt)
     sim.sync()
-    assert np.array_equal(sim.aux(H.Simulation.AUX_ADVECTED), z["coll_advect_vector"])
+    z.check(sim.aux(H.Simulation.AUX_ADVECTED), "coll_advect_vector", "advect_vector(hasCollision)")
     # all-in-one node
     fields = dict(density=z["scalar0"], fuel=z["comb_fuel"], waste=z["comb_waste"], temperature=z["comb_temperature"], flame=z["comb_flame"],
                   collision_sdf=z["collision_sdf"])
@@ -499,31 +542,36 @@ def test_collision_against_golden_reference_outputs(name):
         d.pValues(FLOAT, k)[:] = v
     gh = H.CreateIndexGrid(d, h)
     H.Compute_Sim(d, gh, I, dt, h, H.CombustionParams(*z["params"].tolist()), True)
-    assert np.array_equal(d.pValues(VEC3F, "vel"), z["compute_sim_coll_vel"])
+    z.check(d.pValues(VEC3F, "vel"), "compute_sim_coll_vel", "Compute_Sim(hasCollision) velocity")
     for k in fields:
         if k != "collision_sdf":
-            assert np.array_equal(d.pValues(FLOAT, k), z[f"compute_sim_coll_{k}"]), k
+            z.check(d.pValues(FLOAT, k), f"compute_sim_coll_{k}", k)
 
 
-@needs_ref
 def test_standalone_launchers_match_reference_launchers(case):
     w = case
     h, dt = w.voxel_size, w.dt
-    rd = O.RefData(w.coords)
-    rd.add_vec3("vel", w.velocity)
-    for n, s in zip(w.scalar_names, w.scalars):
-        rd.add_float(n, s)
-    O.ref_advect_index_grid(rd, dt, h)
+
+    def live():
+        rd = O.RefData(w.coords)
+        rd.add_vec3("vel", w.velocity)
+        for n, s in zip(w.scalar_names, w.scalars):
+            rd.add_float(n, s)
+        O.ref_advect_index_grid(rd, dt, h)
+        out = {"advect_" + n: rd.blocks[n].copy() for n in w.scalar_names}
+        rd = O.RefData(w.coords)
+        rd.add_vec3("vel", w.velocity)
+        O.ref_project_non_divergent(rd, 10, h)
+        return dict(out, project=rd.blocks["vel"].copy())
+
+    ref = Reference(f"launchers/{w.name}", live, [w.coords, w.velocity, *w.scalars])
     d = _sidecar(w, dict(zip(w.scalar_names, w.scalars)))
     H.AdvectIndexGrid(d, dt, h)
     for n in w.scalar_names:
-        assert_close(d.pValues(FLOAT, n), rd.blocks[n], f"AdvectIndexGrid {n}")
-    rd = O.RefData(w.coords)
-    rd.add_vec3("vel", w.velocity)
-    O.ref_project_non_divergent(rd, 10, h)
+        ref.check(d.pValues(FLOAT, n), "advect_" + n, f"AdvectIndexGrid {n}")
     d = _sidecar(w, {})
     H.ProjectNonDivergent(d, 10, h)
-    assert_close(d.pValues(VEC3F, "vel"), rd.blocks["vel"], "ProjectNonDivergent")
+    ref.check(d.pValues(VEC3F, "vel"), "project", "ProjectNonDivergent")
 
 
 def test_compute_sim_errors():
@@ -552,7 +600,7 @@ def test_against_golden_reference_outputs(name):
     path = os.path.join(GOLDEN, f"ref_{name}.npz")
     if not os.path.exists(path):
         pytest.skip("fixture not committed")
-    z = np.load(path)
+    z = Golden(name)
     h, dt, I = float(z["voxel_size"]), float(z["dt"]), int(z["iterations"])
     g = H.create_index_grid_from_origins(z["origins"], h)
     ref = z["nanovdb"]
@@ -564,18 +612,18 @@ def test_against_golden_reference_outputs(name):
     sim.upload(z["velocity"], [z[f"scalar{i}"] for i in range(S)])
     sim.step(I, dt)
     sim.sync()
-    assert_close(sim.aux(2), z["frame_adv"], "advect_vector")
-    assert_close(sim.aux(0), z["frame_div"], "divergence")
-    assert_close(sim.aux(1), z["frame_p"], "pressure")
-    assert_close(sim.velocity(), z["frame_vel"], "projected velocity")
+    z.check(sim.aux(2), "frame_adv", "advect_vector")
+    z.check(sim.aux(0), "frame_div", "divergence")
+    z.check(sim.aux(1), "frame_p", "pressure")
+    z.check(sim.velocity(), "frame_vel", "projected velocity")
     for i in range(S):
-        assert_close(sim.scalar(i), z[f"frame_scalar{i}"], f"scalar {i}")
+        z.check(sim.scalar(i), f"frame_scalar{i}", f"scalar {i}")
     fields = dict(density=z["scalar0"], fuel=z["comb_fuel"], waste=z["comb_waste"], temperature=z["comb_temperature"], flame=z["comb_flame"])
     d = GridIndexedData.from_arrays(z["coords"], z["velocity"], "vel", **fields)
     H.Compute_Sim(d, H.CreateIndexGrid(d, h), I, dt, h, H.CombustionParams(*z["params"].tolist()), False)
-    assert_close(d.pValues(VEC3F, "vel"), z["compute_sim_vel"], "Compute_Sim velocity")
+    z.check(d.pValues(VEC3F, "vel"), "compute_sim_vel", "Compute_Sim velocity")
     for k in fields:
-        assert_close(d.pValues(FLOAT, k), z[f"compute_sim_{k}"], f"Compute_Sim {k}")
+        z.check(d.pValues(FLOAT, k), f"compute_sim_{k}", f"Compute_Sim {k}")
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -597,26 +645,28 @@ def test_config2_full_frame_matches_oracle():
         assert_close(got["scalars"][i], want["scalars"][i], f"scalar {i}")
 
 
-@needs_ref
 def test_config4_full_frame_matches_reference_kernels(c4):
     w = c4
-    coords = synth.dense_coords(w.origins)
-    rd = O.RefData(coords)
-    rd.add_vec3("vel", w.velocity)
-    for n, a in zip(w.scalar_names, w.scalars):
-        rd.add_float(n, a)
-    rg = O.RefGrid(rd, w.voxel_size)
-    rf = O.RefFrame(rd, rg, w.scalar_names)
-    rf.run(40, w.dt, w.voxel_size, 1)
-    want = rf.download()
+
+    def live():
+        rd = O.RefData(synth.dense_coords(w.origins))
+        rd.add_vec3("vel", w.velocity)
+        for n, a in zip(w.scalar_names, w.scalars):
+            rd.add_float(n, a)
+        rg = O.RefGrid(rd, w.voxel_size)
+        rf = O.RefFrame(rd, rg, w.scalar_names)
+        rf.run(40, w.dt, w.voxel_size, 1)
+        want = rf.download()
+        return dict(want, **{f"scalar{i}": s for i, s in enumerate(want.pop("scalars"))})
+
     got = run_product_frame(w, 40)
+    ref = Reference(f"frame/{w.name}", live, [w.origins, w.velocity, *w.scalars])
     for k in ("adv", "div", "p", "vel"):
-        assert_close(got[k], want[k], k)
+        ref.check(got[k], k, k)
     for i in range(2):
-        assert_close(got["scalars"][i], want["scalars"][i], f"scalar {i}")
+        ref.check(got["scalars"][i], f"scalar{i}", f"scalar {i}")
 
 
-@needs_ref
 def test_config4_all_in_one_frame_matches_reference_compute_sim(c4):
     """What bench.py times: the FULL HNanoSolver frame (combustion + buoyancy, S = 5 float blocks, I = 40) on the 512^3 sparse smoke,
     through the launcher pair CreateIndexGrid + Compute_Sim, against the unmodified reference's own CreateIndexGrid + Compute_Sim on
@@ -624,17 +674,22 @@ def test_config4_all_in_one_frame_matches_reference_compute_sim(c4):
     w = c4
     fields = dict(density=w.scalars[0], **synth.combustion_fields(w))
     coords = synth.dense_coords(w.origins)
-    rd = O.RefData(coords)
-    rd.add_vec3("vel", w.velocity)
-    for k, v in fields.items():
-        rd.add_float(k, v)
-    O.ref_cook_frame(rd, 40, w.dt, w.voxel_size, PARAMS6)
+
+    def live():
+        rd = O.RefData(coords)
+        rd.add_vec3("vel", w.velocity)
+        for k, v in fields.items():
+            rd.add_float(k, v)
+        O.ref_cook_frame(rd, 40, w.dt, w.voxel_size, PARAMS6)
+        return _copies(rd)
+
+    ref = Reference(f"cook/{w.name}", live, [coords, w.velocity, *fields.values()])
     d = GridIndexedData.from_arrays(coords, w.velocity.copy(), "vel", **{k: v.copy() for k, v in fields.items()})
     g = H.CreateIndexGrid(d, w.voxel_size)
     H.Compute_Sim(d, g, 40, w.dt, w.voxel_size, H.CombustionParams(*PARAMS6.tolist()), False)
-    assert_close(d.pValues(VEC3F, "vel"), rd.blocks["vel"], "Compute_Sim velocity")
+    ref.check(d.pValues(VEC3F, "vel"), "vel", "Compute_Sim velocity")
     for k in fields:
-        assert_close(d.pValues(FLOAT, k), rd.blocks[k], f"Compute_Sim {k}")
+        ref.check(d.pValues(FLOAT, k), k, f"Compute_Sim {k}")
 
 
 def test_config1_reference_host_path_case():

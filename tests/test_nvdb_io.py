@@ -12,7 +12,7 @@ from hnanosolver_b200 import synth
 from hnanosolver_b200.grid_data import FLOAT, VEC3F, GridIndexedData
 from oracle import oracle as O
 
-needs_refhost = pytest.mark.skipif(not O.ref_host_available(), reason="oracle/_ref/libref_host.so not built (needs /root/reference)")
+needs_refhost = pytest.mark.skipif(not O.ref_host_available(), reason="needs oracle/_ref/libref_host.so, built only from the original project's sources (oracle/Makefile REF)")
 
 
 def _cases():

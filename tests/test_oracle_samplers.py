@@ -5,7 +5,7 @@ import pytest
 
 from oracle import oracle as O
 
-needs_refhost = pytest.mark.skipif(not O.ref_host_available(), reason="oracle/_ref/libref_host.so not built (needs /root/reference)")
+needs_refhost = pytest.mark.skipif(not O.ref_host_available(), reason="needs oracle/_ref/libref_host.so, built only from the original project's sources (oracle/Makefile REF)")
 
 
 def _line(axis, n=15):
