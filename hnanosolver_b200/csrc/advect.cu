@@ -561,6 +561,7 @@ __global__ void __launch_bounds__(512) k_advect_scalars_cold(GridView g, const f
 // The packed groups (float4[L][512], same voxel order as the brick fields) are produced by the kernel that writes the fields anyway
 // (subtractPressureGradient writes {u, v, w, scalar 0}, combustion writes {fuel, waste, temperature, flame}) or by k_pack4.
 // Arithmetic, operand order and the cold path are those of the second generation: results are bit-identical.
+// In the frame with combustion, k_advect_vector4 also carries the combustion field update and writes group 1 itself (kCombustion).
 // =================================================================================================================================
 constexpr int kCells = kRX * kRX * kRZ;                         // 3136 cells, 49 KB per group
 constexpr size_t kRegions4 = 2 * kCells * sizeof(float4);        // double buffer: 98 KB per CTA, two CTAs per SM
@@ -674,10 +675,14 @@ __device__ __forceinline__ float limited(float mn, float mx, float first, float 
 	return fmaxf(fminf(mn, first), fminf(corrected, fmaxf(mx, first)));
 }
 
-template <bool kCollision>
+// kCombustion: combustion_oxygen rides along (the frame's own pass would stream 2.5 GB through HBM at 40 M voxels, while this kernel,
+// bound by the shared-memory pipe, leaves about 70 % of the HBM bandwidth idle): for every work item each thread also updates its own
+// voxel of the leaf from the frame's input fields (combustion_voxel, kernels.cuh). The loads are issued before the sampling and consumed
+// after it, on every path through the item, the cold exits included.
+template <bool kCollision, bool kCombustion = false>
 __global__ void __launch_bounds__(512, 2) k_advect_vector4(GridView g, const float4* __restrict__ vel4, float* __restrict__ ou, float* __restrict__ ov,
                                                            float* __restrict__ ow, float sdt, const float* __restrict__ sdf,
-                                                           uint8_t* __restrict__ cold) {
+                                                           uint8_t* __restrict__ cold, const __grid_constant__ CombustionJob cj) {
 	extern __shared__ __align__(128) float4 region4[];
 	int(*meta)[kMeta] = reinterpret_cast<int(*)[kMeta]>(region4 + 2 * kCells);
 	const Items items = cta_items2(g);
@@ -702,6 +707,18 @@ __global__ void __launch_bounds__(512, 2) k_advect_vector4(GridView g, const flo
 		const float4* __restrict__ r = region4 + (k & 1) * kCells;
 		const int* m = meta[k % 3];
 		const uint32_t leaf = uint32_t(m[kMetaLeaf]);
+		const uint32_t self = leaf * 512u + uint32_t(tid);
+		float4 comb_in;
+		if constexpr (kCombustion) comb_in = make_float4(__ldg(cj.in[0] + self), __ldg(cj.in[1] + self), __ldg(cj.in[2] + self), __ldg(cj.in[3] + self));
+		auto combust = [&] {
+			if constexpr (kCombustion) {
+				float4 o;
+				const float burn = combustion_voxel(comb_in, cj.temp_gain, o);
+				cj.out[0][self] = o.x, cj.out[1][self] = o.y, cj.out[2][self] = o.z, cj.out[3][self] = o.w;
+				cj.grp1[self] = o;
+				cj.burn[self] = burn;
+			}
+		};
 		const float4 c0 = r[oc];
 		const int ox = m[kMetaOx], oy = m[kMetaOx + 1], oz = m[kMetaOx + 2];
 		const float px = float(ox + x), py = float(oy + y), pz = float(oz + z);
@@ -712,6 +729,7 @@ __global__ void __launch_bounds__(512, 2) k_advect_vector4(GridView g, const flo
 		int cb;
 		if (!footprint4(bi - ox, bj - oy, bk - oz, cb)) {
 			cold[leaf] = 1;
+			combust();
 			continue;
 		}
 		const float4 f = tri_lerp4(r, cb, bx - float(bi), by - float(bj), bz - float(bk));
@@ -721,12 +739,13 @@ __global__ void __launch_bounds__(512, 2) k_advect_vector4(GridView g, const flo
 		int cf;
 		if (!footprint4(fi - ox, fj - oy, fk - oz, cf)) {
 			cold[leaf] = 1;
+			combust();
 			continue;
 		}
 		const float4 b = tri_lerp4(r, cf, fx - float(fi), fy - float(fj), fz - float(fk));
 		const float cu = fmaf(0.5f, c0.x - b.x, f.x), cv = fmaf(0.5f, c0.y - b.y, f.y), cw = fmaf(0.5f, c0.z - b.z, f.z);  // :399-400
 		const float4 n0 = r[oc - kCX], n1 = r[oc + kCX], n2 = r[oc - kCY], n3 = r[oc + kCY], n4 = r[oc - 1], n5 = r[oc + 1];
-		const uint32_t self = leaf * 512u + uint32_t(tid);
+		combust();
 		ou[self] = limited(min7(c0.x, n0.x, n1.x, n2.x, n3.x, n4.x, n5.x), max7(c0.x, n0.x, n1.x, n2.x, n3.x, n4.x, n5.x), f.x, cu);  // :402-429
 		ov[self] = limited(min7(c0.y, n0.y, n1.y, n2.y, n3.y, n4.y, n5.y), max7(c0.y, n0.y, n1.y, n2.y, n3.y, n4.y, n5.y), f.y, cv);
 		ow[self] = limited(min7(c0.z, n0.z, n1.z, n2.z, n3.z, n4.z, n5.z), max7(c0.z, n0.z, n1.z, n2.z, n3.z, n4.z, n5.z), f.z, cw);
@@ -893,7 +912,7 @@ void ensure_attrs(DeviceInfo& d) {
 	opt_in(k_advect_scalars2<0, false>), opt_in(k_advect_scalars2<1, false>);
 	opt_in(k_advect_scalars2<0, true>), opt_in(k_advect_scalars2<1, true>);
 	static_assert(kAdvect4Smem >= kAdvectSmem, "opt_in asks for the second generation's size");
-	opt_in(k_advect_vector4<false>, kAdvect4Smem), opt_in(k_advect_vector4<true>, kAdvect4Smem);
+	opt_in(k_advect_vector4<false>, kAdvect4Smem), opt_in(k_advect_vector4<true>, kAdvect4Smem), opt_in(k_advect_vector4<false, true>, kAdvect4Smem);
 	opt_in(k_advect_scalars4<0, false>, kAdvect4Smem), opt_in(k_advect_scalars4<1, false>, kAdvect4Smem);
 	opt_in(k_advect_scalars4<0, true>, kAdvect4Smem), opt_in(k_advect_scalars4<1, true>, kAdvect4Smem);
 	d.attrs = true;
@@ -940,7 +959,7 @@ int set_packed_advection(int on) { return packed_switch().exchange(on ? 1 : 0); 
 uint64_t packed_advection_launches() { return g_packed_launches.load(); }
 
 void launch_advect_vector(const GridView& g, const float* const vel[3], float* const out[3], float dt, float inv_dx, cudaStream_t st, const float* sdf,
-                          uint8_t* cold, const AdvectGroups* grp) {
+                          uint8_t* cold, const AdvectGroups* grp, const CombustionJob* comb) {
 	if (!g.count()) return;
 	DeviceInfo& d = device_info();
 	ensure_attrs(d);
@@ -950,11 +969,14 @@ void launch_advect_vector(const GridView& g, const float* const vel[3], float* c
 	if (grp && grp->g[0] && (grp->valid & 1u) && packed_advection()) {  // group 0 holds this velocity: the third generation
 		g_packed_launches.fetch_add(1, std::memory_order_relaxed);
 		if (sdf) {
-			HNS_LAUNCH(k_advect_vector4<true>, grid, 512, kAdvect4Smem, st, g, grp->g[0], out[0], out[1], out[2], sdt, sdf, cold);
+			HNS_LAUNCH(k_advect_vector4<true>, grid, 512, kAdvect4Smem, st, g, grp->g[0], out[0], out[1], out[2], sdt, sdf, cold, CombustionJob{});
 			HNS_LAUNCH(k_advect_vector_cold<true>, cold_grid, 512, 0, st, g, vel[0], vel[1], vel[2], out[0], out[1], out[2], sdt, sdf, cold);
 			launch_collision_boundary(g, out, out, sdf, inv_dx, 1.5f, 1, st);
 		} else {
-			HNS_LAUNCH(k_advect_vector4<false>, grid, 512, kAdvect4Smem, st, g, grp->g[0], out[0], out[1], out[2], sdt, sdf, cold);
+			if (comb)
+				HNS_LAUNCH((k_advect_vector4<false, true>), grid, 512, kAdvect4Smem, st, g, grp->g[0], out[0], out[1], out[2], sdt, sdf, cold, *comb);
+			else
+				HNS_LAUNCH(k_advect_vector4<false>, grid, 512, kAdvect4Smem, st, g, grp->g[0], out[0], out[1], out[2], sdt, sdf, cold, CombustionJob{});
 			HNS_LAUNCH(k_advect_vector_cold<false>, cold_grid, 512, 0, st, g, vel[0], vel[1], vel[2], out[0], out[1], out[2], sdt, sdf, cold);
 		}
 		return;

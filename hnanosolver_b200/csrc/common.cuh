@@ -212,6 +212,7 @@ struct hns_state {
 	const float* grp0_s0 = nullptr;                                          // the scalar buffer in group 0's fourth lane
 	const float* grp1_src[4] = {nullptr, nullptr, nullptr, nullptr};         // the buffers group 1 mirrors
 	bool grp_dist = false;  // a sharded frame (dist.cu) re-packs the ghost leaves of the groups after its exchanges
+	float* burn = nullptr;  // float[n], allocated on first use: combustion's burn per voxel from advect_vector to the divergence (api.cu, frame)
 	float* vort[4] = {nullptr, nullptr, nullptr, nullptr};  // vorticity confinement scratch, allocated on first use: output planes u, v, w and |curl|
 	// optional combustion + buoyancy stage of the all-in-one frame
 	bool comb_enabled = false;

@@ -143,9 +143,13 @@ void launch_soa_to_aos(const float* u, const float* v, const float* w, float* ao
 // divergence  (reference Kernel.cu:499-519)
 //   xp = (c.x + u(+x).x) * 0.5 ... ; div = (xp - xm + yp - ym + zp - zm) * inv_dx ; inactive neighbour -> 0
 // =============================================================================================================
+// kBurn: combustion's expansion term too (reference Kernel.cu:963), from the burn values the combustion side job of advect_vector wrote
+// (advect.cu): d = fma(burn, expansion, d) on the divergence rounded to float, as when combustion_oxygen reads it back; burn = -1 (no
+// oxygen) leaves d alone, so an exact -0.0 stays -0.0 there
+template <bool kBurn>
 __global__ void __launch_bounds__(256) k_divergence(GridView g, const float* __restrict__ u, const float* __restrict__ v,
                                                     const float* __restrict__ w, float* __restrict__ div_red, float* __restrict__ div_blk,
-                                                    float inv_dx) {
+                                                    float inv_dx, const float* __restrict__ burn, float expansion) {
 	RowCtx c;
 	if (!make_row_ctx(g, c)) return;
 	const uint64_t self = c.self();
@@ -164,12 +168,22 @@ __global__ void __launch_bounds__(256) k_divergence(GridView g, const float* __r
 		const float yp = (cv.v[z] + vyp.v[z]) * 0.5f, ym = (cv.v[z] + vym.v[z]) * 0.5f;
 		const float zp = (cw.v[z] + (z < 7 ? cw.v[z < 7 ? z + 1 : 7] : wzp)) * 0.5f;
 		const float zm = (cw.v[z] + (z > 0 ? cw.v[z > 0 ? z - 1 : 0] : wzm)) * 0.5f;
-		o.v[z] = (xp - xm + yp - ym + zp - zm) * inv_dx;
+		if constexpr (kBurn) o.v[z] = __fmul_rn(xp - xm + yp - ym + zp - zm, inv_dx);  // not contracted into the fma below
+		else o.v[z] = (xp - xm + yp - ym + zp - zm) * inv_dx;
+	}
+	if constexpr (kBurn) {
+		const Row8 b = ld_row(burn, self);
+#pragma unroll
+		for (int z = 0; z < 8; ++z)
+			if (b.v[z] != -1.0f) o.v[z] = fmaf(b.v[z], expansion, o.v[z]);
 	}
 	st_split(div_red, div_blk, c, o);
 }
-void launch_divergence(const GridView& g, const float* const vel[3], float* const div[2], float inv_dx, cudaStream_t st) {
-	if (g.count()) HNS_LAUNCH(k_divergence, (g.count() + 3) / 4, 256, 0, st, g, vel[0], vel[1], vel[2], div[0], div[1], inv_dx);
+void launch_divergence(const GridView& g, const float* const vel[3], float* const div[2], float inv_dx, cudaStream_t st, const float* burn,
+                       float expansion) {
+	if (!g.count()) return;
+	HNS_LAUNCH((burn ? k_divergence<true> : k_divergence<false>), (g.count() + 3) / 4, 256, 0, st, g, vel[0], vel[1], vel[2], div[0], div[1], inv_dx, burn,
+	           expansion);
 }
 
 // =============================================================================================================
@@ -177,12 +191,14 @@ void launch_divergence(const GridView& g, const float* const vel[3], float* cons
 // =============================================================================================================
 // kGroup: the projected velocity also goes, together with the scalar field `s0` (or 0), into the packed group the advection kernels
 // stage from (advect.cu, third generation): float4 {u, v, w, s0} per voxel.
-template <bool kGroup>
+// kBuoyancy: temperature_buoyancy first, on the v this thread reads: the value its own pass would have stored, with the same two
+// roundings; that v also goes back to by.vy (= v: a thread reads and writes only its own row).
+template <bool kGroup, bool kBuoyancy>
 __global__ void __launch_bounds__(256) k_subtract_gradient(GridView g, const float* __restrict__ u, const float* __restrict__ v,
                                                            const float* __restrict__ w, const float* __restrict__ p_red,
                                                            const float* __restrict__ p_blk, float* __restrict__ ou, float* __restrict__ ov,
                                                            float* __restrict__ ow, float inv_dx, float4* __restrict__ grp0,
-                                                           const float* __restrict__ s0) {
+                                                           const float* __restrict__ s0, const Buoyancy by) {
 	RowCtx c;
 	if (!make_row_ctx(g, c)) return;
 	const uint64_t self = c.self();
@@ -196,7 +212,15 @@ __global__ void __launch_bounds__(256) k_subtract_gradient(GridView g, const flo
 	// z = 7 of the -z leaf has parity (x+y+7): colour red iff s is odd; z = 0 of the +z leaf is red iff s is even
 	const float pzm = (i = c.zminus()) >= 0 ? __ldg((s ? p_red : p_blk) + (split_idx(uint64_t(i) & ~uint64_t(7)) + 3)) : 0.f;
 	const float pzp = (i = c.zplus()) >= 0 ? __ldg((s ? p_blk : p_red) + split_idx(uint64_t(i))) : 0.f;
-	const Row8 cu = ld_row(u, self), cv = ld_row(v, self), cw = ld_row(w, self);
+	const Row8 cu = ld_row(u, self), cw = ld_row(w, self);
+	Row8 cv = ld_row(v, self);
+	if constexpr (kBuoyancy) {
+		const Row8 T = ld_row(by.temp, self);
+#pragma unroll
+		for (int z = 0; z < 8; ++z)
+			if (T.v[z] > by.ambient) cv.v[z] = fmaf(fmaxf(0.0f, (T.v[z] - by.ambient) * by.strength), by.dt, cv.v[z]);
+		st_row(by.vy, self, cv);
+	}
 	Row8 a, b, d;
 #pragma unroll
 	for (int z = 0; z < 8; ++z) {
@@ -230,14 +254,12 @@ __global__ void __launch_bounds__(256) k_subtract_gradient(GridView g, const flo
 	}
 }
 void launch_subtract_gradient(const GridView& g, const float* const vel[3], const float* const p[2], float* const out[3], float inv_dx,
-                              cudaStream_t st, float4* grp0, const float* s0) {
+                              cudaStream_t st, float4* grp0, const float* s0, const Buoyancy* buoy) {
 	if (!g.count()) return;
-	if (grp0)
-		HNS_LAUNCH(k_subtract_gradient<true>, (g.count() + 3) / 4, 256, 0, st, g, vel[0], vel[1], vel[2], p[0], p[1], out[0], out[1], out[2], inv_dx,
-		           grp0, s0);
-	else
-		HNS_LAUNCH(k_subtract_gradient<false>, (g.count() + 3) / 4, 256, 0, st, g, vel[0], vel[1], vel[2], p[0], p[1], out[0], out[1], out[2], inv_dx,
-		           grp0, s0);
+	auto k = grp0 ? (buoy ? k_subtract_gradient<true, true> : k_subtract_gradient<true, false>)
+	              : (buoy ? k_subtract_gradient<false, true> : k_subtract_gradient<false, false>);
+	HNS_LAUNCH(k, (g.count() + 3) / 4, 256, 0, st, g, vel[0], vel[1], vel[2], p[0], p[1], out[0], out[1], out[2], inv_dx, grp0, s0,
+	           buoy ? *buoy : Buoyancy{});
 }
 
 // =============================================================================================================
@@ -532,23 +554,13 @@ __global__ void __launch_bounds__(256) k_combustion_buoyancy_packed(const float*
                                                                     uint64_t n, bool update_div, bool buoyancy) {
 	const uint64_t t = blockIdx.x * uint64_t(256) + threadIdx.x;
 	if (t >= n) return;
-	float f = fuel[t];
-	const float wv = waste[t], T = temp[t], fl = flame[t];
-	if (f < 0.001f) f = 0.0f;
-	const float oxygen = 1.0f - f - wv;
-	float4 o = make_float4(f, wv, T, fl);
-	if (!(oxygen < 0.0f)) {
-		const float burn = fminf(oxygen, f);
-		o.x = f - burn;
-		o.y = fmaf(burn, 2.0f, wv);
-		o.w = fmaxf(fl, fminf(1.0f, burn * 10.0f));
-		o.z = fmaf(burn, temp_gain, T);
-		if (update_div) {
-			const uint32_t v = uint32_t(t) & 511u;
-			const bool black = (((v >> 6) + (v >> 3) + v) & 1u) != 0;
-			float* d = (black ? div_blk : div_red) + ((t >> 3) << 2) + ((v & 7u) >> 1);
-			*d = fmaf(burn, expansion, *d);
-		}
+	float4 o;
+	const float burn = combustion_voxel(make_float4(fuel[t], waste[t], temp[t], flame[t]), temp_gain, o);
+	if (update_div && burn != -1.0f) {
+		const uint32_t v = uint32_t(t) & 511u;
+		const bool black = (((v >> 6) + (v >> 3) + v) & 1u) != 0;
+		float* d = (black ? div_blk : div_red) + ((t >> 3) << 2) + ((v & 7u) >> 1);
+		*d = fmaf(burn, expansion, *d);
 	}
 	oFuel[t] = o.x, oWaste[t] = o.y, oTemp[t] = o.z, oFlame[t] = o.w;
 	grp[t] = o;
