@@ -3,6 +3,9 @@ import importlib.util
 import os
 
 import numpy as np
+import pytest
+
+from oracle import oracle as O
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 _spec = importlib.util.spec_from_file_location("make_golden", os.path.join(GOLDEN, "make_golden.py"))
@@ -133,3 +136,41 @@ class Recording:
 
     def save(self):
         np.savez_compressed(self.path, **self._z)
+
+
+RECORDED = Recording(os.path.join(GOLDEN, "ref_recorded.npz"))
+
+
+class Reference:
+    """The reference's outputs under `key` (test, case, parameters) for `inputs`: `live()` runs its own kernels and launchers when their
+    build is present (and, with HNS_RECORD_REFERENCE=1, records what they return); otherwise the recording of what they computed from
+    the same inputs stands in (Recording). A module that builds one saves RECORDED when it is done recording."""
+
+    def __init__(self, key: str, live, inputs):
+        self.key, self.want = key, None
+        if O.ref_gpu_available():
+            self.want = live()
+            if RECORDED.recording:
+                RECORDED.record_inputs(key, inputs)
+        elif RECORDED.recording:
+            pytest.fail("recording the reference's outputs needs its build (oracle/_ref/libhns_ref.so)")
+        else:
+            RECORDED.check_inputs(key, inputs)
+
+    def check(self, got, name: str, what: str):
+        if self.want is None:
+            RECORDED.check(got, f"{self.key}/{name}", what)
+            return
+        assert_close(got, self.want[name], what)
+        if RECORDED.recording:
+            RECORDED.record(self.want[name], f"{self.key}/{name}")
+
+
+def combustion_fields(n, seed=123):
+    """fuel / waste / temperature / flame of the small cases: fuel in about 40 % of the voxels, element 0 zero"""
+    rng = np.random.default_rng(seed)
+    f = dict(fuel=(rng.random(n) * (rng.random(n) < 0.4)).astype(np.float32), waste=(0.3 * rng.random(n)).astype(np.float32),
+             temperature=rng.random(n).astype(np.float32), flame=(0.2 * rng.random(n)).astype(np.float32))
+    for a in f.values():
+        a[0] = 0.0
+    return f

@@ -11,14 +11,13 @@ import numpy as np
 import pytest
 
 import hnanosolver_b200 as H
-from helpers import GOLDEN, Golden, Recording, assert_close, nanovdb_compare_mask, rel_err
+from helpers import GOLDEN, RECORDED, Golden, Reference, assert_close, combustion_fields, nanovdb_compare_mask, rel_err
 from hnanosolver_b200 import synth
 from hnanosolver_b200.grid_data import FLOAT, VEC3F, GridIndexedData
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 PARAMS6 = np.array([0.5, 2.0, 1.5, 0.1, 0.0, 1.0], np.float32)
-RECORDED = Recording(os.path.join(GOLDEN, "ref_recorded.npz"))
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -26,31 +25,6 @@ def _save_recording():
     yield
     if RECORDED.recording:
         RECORDED.save()
-
-
-class Reference:
-    """The reference's outputs under `key` (test, case, parameters) for `inputs`: `live()` runs its own kernels and launchers when their
-    build is present (and, with HNS_RECORD_REFERENCE=1, records what they return); otherwise the recording of what they computed from
-    the same inputs stands in (helpers.Recording)."""
-
-    def __init__(self, key: str, live, inputs):
-        self.key, self.want = key, None
-        if O.ref_gpu_available():
-            self.want = live()
-            if RECORDED.recording:
-                RECORDED.record_inputs(key, inputs)
-        elif RECORDED.recording:
-            pytest.fail("recording the reference's outputs needs its build (oracle/_ref/libhns_ref.so)")
-        else:
-            RECORDED.check_inputs(key, inputs)
-
-    def check(self, got, name: str, what: str):
-        if self.want is None:
-            RECORDED.check(got, f"{self.key}/{name}", what)
-            return
-        assert_close(got, self.want[name], what)
-        if RECORDED.recording:
-            RECORDED.record(self.want[name], f"{self.key}/{name}")
 
 
 def _copies(rd):
@@ -267,19 +241,10 @@ def test_launchers_match_oracle(case):
     assert_close(d.pValues(VEC3F, "vel"), ix.project_non_divergent(w.velocity, 5, h)[0], "ProjectNonDivergent")
 
 
-def _combustion_fields(n, seed=123):
-    rng = np.random.default_rng(seed)
-    f = dict(fuel=(rng.random(n) * (rng.random(n) < 0.4)).astype(np.float32), waste=(0.3 * rng.random(n)).astype(np.float32),
-             temperature=rng.random(n).astype(np.float32), flame=(0.2 * rng.random(n)).astype(np.float32))
-    for a in f.values():
-        a[0] = 0.0
-    return f
-
-
 def test_compute_sim_matches_oracle(case):
     w = case
     ix = O.OracleIndex(w.coords)
-    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
+    fields = dict(density=w.scalars[0], **combustion_fields(w.num_voxels))
     want_vel, want = ix.compute_sim(w.velocity, fields, 5, w.dt, w.voxel_size, PARAMS6)
     d = _sidecar(w, fields)
     g = H.CreateIndexGrid(d, w.voxel_size)
@@ -296,7 +261,7 @@ def test_compute_sim_equals_the_resident_frame_bitwise(case, order):
     follow behind the gradient pass (api.cu::frame, FrameDeps). The resident frame runs the reference's step order on fields that are
     all there. Independent steps in another order: every bit must agree, whatever the order of the float blocks."""
     w = case
-    comb = _combustion_fields(w.num_voxels)
+    comb = combustion_fields(w.num_voxels)
     fields = {k: (w.scalars[0] if k == "density" else comb[k]) for k in order}
     d = _sidecar(w, {k: v.copy() for k, v in fields.items()})
     g = H.CreateIndexGrid(d, w.voxel_size)
@@ -326,7 +291,7 @@ def _ref_compute_sim(w, fields, iterations, params, has_collision=False):
 
 def test_compute_sim_matches_reference_compute_sim(case):
     w = case
-    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
+    fields = dict(density=w.scalars[0], **combustion_fields(w.num_voxels))
     d = _sidecar(w, fields)
     g = H.CreateIndexGrid(d, w.voxel_size)
     H.Compute_Sim(d, g, 8, w.dt, w.voxel_size, H.CombustionParams(*PARAMS6.tolist()), False)
@@ -396,7 +361,7 @@ def test_compute_sim_with_vorticity_matches_oracle(case):
     params = PARAMS6.copy()
     params[4], params[5] = 0.8, 1.0
     ix = O.OracleIndex(w.coords)
-    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
+    fields = dict(density=w.scalars[0], **combustion_fields(w.num_voxels))
     want_vel, want = ix.compute_sim(w.velocity, fields, 5, w.dt, w.voxel_size, params)
     off_vel, _ = ix.compute_sim(w.velocity, fields, 5, w.dt, w.voxel_size, PARAMS6)
     d = _sidecar(w, fields)
@@ -415,7 +380,7 @@ def test_compute_sim_default_sop_vorticity_parameters_match_reference(case):
     w = case
     params = PARAMS6.copy()
     params[4], params[5] = 1.0, 0.5
-    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
+    fields = dict(density=w.scalars[0], **combustion_fields(w.num_voxels))
     d = _sidecar(w, fields)
     g = H.CreateIndexGrid(d, w.voxel_size)
     H.Compute_Sim(d, g, 6, w.dt, w.voxel_size, H.CombustionParams(*params.tolist()), False)
@@ -474,7 +439,7 @@ def test_collision_kernels_match_oracle(case):
 
 
 def _compute_sim_collision(w, has_collision, iterations=5):
-    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels), collision_sdf=_collision_sdf(w))
+    fields = dict(density=w.scalars[0], **combustion_fields(w.num_voxels), collision_sdf=_collision_sdf(w))
     d = _sidecar(w, fields)
     g = H.CreateIndexGrid(d, w.voxel_size)
     H.Compute_Sim(d, g, iterations, w.dt, w.voxel_size, H.CombustionParams(*PARAMS6.tolist()), has_collision)
@@ -789,7 +754,7 @@ def test_packed_advection_is_bit_identical_over_consecutive_frames(layout):
     advect_scalars in every frame, advect_vector from the second frame on (the first one finds no group yet). `two_scalars` has no
     producer for its second group and must stay on the second generation."""
     w = synth.random_leaves(60, 4, 9, cfl=1.2, S=2)
-    comb = _combustion_fields(w.num_voxels)
+    comb = combustion_fields(w.num_voxels)
     fields, with_comb, expect = {
         "density_first": (dict(density=w.scalars[0], **comb), True, 5),
         "density_last": (dict(**comb, density=w.scalars[0]), True, 5),
@@ -886,7 +851,7 @@ def _drive(which, w, fields, iterations):
 @needs_compat
 def test_compat_library_is_a_drop_in_for_the_reference_launchers(case):
     w = case
-    fields = dict(density=w.scalars[0], **_combustion_fields(w.num_voxels))
+    fields = dict(density=w.scalars[0], **combustion_fields(w.num_voxels))
     ref = _drive("reference", w, fields, 7)
     mine = _drive("compat", w, fields, 7)
     T = int(np.frombuffer(ref["nanovdb"][672 + 40:672 + 44].tobytes(), np.uint32)[0])
