@@ -132,6 +132,12 @@ SIGNATURES = {
     "hns_state_set_pressure_solver": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float]),
     "hns_dist_bytes_sent": (C.c_uint64, [C.c_void_p]),
     "hns_dist_exchanges": (C.c_uint64, [C.c_void_p]),
+    "hns_dist_set_pressure_solver": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, c_i32p, C.c_int, C.c_int, C.c_int, C.c_float,
+                                               C.POINTER(C.c_uint8)]),
+    "hns_dist_mg_connect": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_uint8)]),
+    "hns_dist_mg_finish": (C.c_int, [C.c_void_p]),
+    "hns_dist_mg_gathers": (C.c_uint64, [C.c_void_p]),
+    "hns_dist_mg_gather_bytes": (C.c_uint64, [C.c_void_p]),
 }
 
 _lib = None

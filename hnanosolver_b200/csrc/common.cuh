@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cstdio>
 #include <string>
+#include <vector>
 
 #include "../../include/hns_b200.h"
 
@@ -178,6 +179,8 @@ GroupsCurrent groups_current(const hns_state* s);
 int groups_refresh_leaves(hns_state* s, const int32_t* ids, uint64_t n_ids, GroupsCurrent which, cudaStream_t st);
 void groups_stamp(hns_state* s, GroupsCurrent which);
 int mg_pressure_solve(hns_state* s, hns_mg* mg, int max_cycles, double rel_tol, int nu_pre, int nu_post, float omega, cudaStream_t st);  // multigrid.cu
+void mg_coarse_cycle(hns_mg* mg, float* const rhs1[2], int nu_pre, int nu_post, float omega, cudaStream_t st);
+cudaGraphExec_t mg_capture_coarse(hns_mg* mg, float* const rhs1[2], int nu_pre, int nu_post, float omega, uint64_t* launches);
 }
 // ---- opaque handle definitions ----------------------------------------------------------------------------
 struct hns_grid {
@@ -191,6 +194,45 @@ struct hns_grid {
 	int4* d_origin = nullptr;
 	int32_t* d_nbr = nullptr;
 	hns::GridView view{};
+};
+
+// multigrid hierarchy (multigrid.cu; a sharded run reads levels >= 1 of a hierarchy over the global grid, dist.cu)
+struct hns_mg {
+	struct Level {
+		hns_grid* grid = nullptr;     // level 0: the caller's grid (borrowed)
+		bool own_grid = false;
+		float* p[2] = {nullptr, nullptr};    // levels >= 1 (level 0 uses the state's pressure / divergence)
+		float* rhs[2] = {nullptr, nullptr};
+		float* diag[2] = {nullptr, nullptr};  // colour-split diagonal of the level's operator, 0 = cell outside the domain; null on level 0
+		const float* const* diag_or_null() const { return diag[0] ? diag : nullptr; }
+		int32_t* parent = nullptr;    // [L] leaf id on the next level; null on the last
+		float dx = 0.f;
+		uint64_t cells = 0;           // cells inside the domain
+	};
+	std::vector<Level> lv;
+	double* d_sums = nullptr;         // device double[2]
+	double* h_sums = nullptr;         // pinned
+	uint64_t last_nonempty_count = 0;  // of the last level: non-empty leaves, and (when that is 1) which one
+	int64_t last_nonempty_leaf = -1;
+	int coarsest_iterations = 32;
+	float coarsest_omega = 1.5f;      // a one-leaf last level is solved, not smoothed: SOR near its optimum for 8 cells per axis
+	// statistics of the last solve
+	int last_cycles = 0;
+	double last_rel_residual = -1.0;
+	// One V-cycle is ~10 launches per level, most of them on levels far too small to fill the GPU: issued one by one they cost their
+	// launch latency (measured: 1.27 of the 2.13 ms of two cycles on the 512^3 workload). The cycle is therefore captured once into a
+	// CUDA graph (on a private stream: capture executes nothing) and replayed; the key is everything the captured launches depend on.
+	struct CycleGraph {
+		cudaGraphExec_t exec = nullptr;
+		const void* state = nullptr;
+		hns::GridView view{};  // the fine level's view (pointers, counts, work list)
+		const void *p = nullptr, *rhs = nullptr;
+		int nu_pre = -1, nu_post = -1, coarsest_iterations = -1;
+		float omega = 0.f;
+		uint64_t launches = 0;
+	} graph;
+	cudaStream_t capture_stream = nullptr;
+	bool use_graph = true;  // HNS_MG_GRAPH=0: issue every launch directly (A/B switch)
 };
 
 struct hns_state {

@@ -111,7 +111,7 @@ struct hns_dist {
 	uint64_t block_bytes = 0;
 	uint32_t** d_remote_flags = nullptr;  // [n_peers] flag words in the peers' blocks
 	uint32_t** d_local_flags = nullptr;   // [n_peers] flag words in my block
-	uint32_t seq[8] = {};
+	uint32_t seq[16] = {};  // per flag channel (kCh* below)
 	uint32_t* d_err = nullptr;
 	int n_scalars = 0;
 	// timed mode: events inside one pressure half-sweep (k = 20): bs: before B, after B, after push, after signal+wait, after unpack; st: before I, after I
@@ -134,7 +134,31 @@ struct hns_dist {
 	cudaStream_t copy_stream = nullptr;  // hns_dist_cook: host <-> device transfers overlapping the frame
 	cudaEvent_t ev_copy[6] = {};
 	bool cook_overlap = true;       // HNS_COOK_OVERLAP=0: transfers and frame one after the other on the caller's stream (A/B switch)
+	// Sharded multigrid pressure solve (hns_dist_set_pressure_solver): level 0 is this rank's shard, levels >= 1 of `mg` (a hierarchy
+	// over the GLOBAL grid) are replicated -- every rank runs the coarse part of every cycle itself on the gathered level-1 rhs.
+	struct ShardedMg {
+		hns_mg* mg = nullptr;          // null: the red-black solve
+		bool ready = false;            // hns_dist_mg_finish has connected every rank
+		int cycles = 0, nu_pre = 0, nu_post = 0;
+		float omega = 1.f;
+		int32_t* d_parent = nullptr;   // [local leaves] level-1 leaf of each local leaf (global level-1 numbering)
+		uint8_t* block = nullptr;      // exposed to every rank: [flag words][level-1 rhs, cycle parity 0 (red | black)][parity 1]
+		uint64_t flag_bytes = 0, rhs_floats = 0;  // rhs_floats: one colour-split array, both halves
+		std::vector<void*> ipc;        // [world] the other ranks' blocks mapped into this process
+		float** d_gather[2] = {nullptr, nullptr};  // per parity: [world][2] red / black of every rank's level-1 rhs
+		uint32_t** d_sig = nullptr;    // [world - 1] my flag words in the other ranks' blocks
+		uint32_t** d_wait = nullptr;   // [world - 1] the other ranks' flag words in my block
+		uint32_t seq = 0;              // number of the last gather (cycles since set-up, across frames)
+		uint64_t gathers = 0, gather_bytes = 0;
+		cudaGraphExec_t graph[2] = {nullptr, nullptr};  // the coarse part, one per parity (its level-1 rhs pointer differs)
+		uint64_t graph_launches[2] = {0, 0};
+		int graph_coarsest[2] = {0, 0};
+	} smg;
 };
+
+// flag channels: 0..7 of the ghost exchanges (see dist_frame), 8 / 9 the red / black pressure exchanges of the sharded multigrid solve
+// (landing in the regions of channels 2 / 3), 10 the level-1 gather. k_wait reports a time-out as 1 + channel in the error word.
+constexpr int kChMgPressure = 8, kChMgGather = 10;
 
 // ---- layout of one peer region: [flags 128 B][ch0 velocity 3 x 512n][ch1 advected velocity 3 x 512n][ch2 red p 256n][ch3 black p 256n]
 //      [ch4 velocity + scalars (3+S) x 512n][ch5 |curl| 512n] floats, n = number of ghost leaves exchanged with that peer.
@@ -247,8 +271,11 @@ int hns_dist_create(const uint8_t* id128, int rank, int world, hns_dist** out) {
 	return HNS_OK;
 }
 
+static void mg_release(hns_dist* d);
+
 void hns_dist_destroy(hns_dist* d) {
 	if (!d) return;
+	mg_release(d);
 	for (auto& p : d->peers) cudaFree(p.d_send), cudaFree(p.d_recv), cudaFree(p.buf_send), cudaFree(p.buf_recv);
 	cudaFree(d->d_reduce);
 	cudaFree(d->d_elem0), cudaFree(d->d_owned), cudaFree(d->d_boundary), cudaFree(d->d_interior);
@@ -280,6 +307,7 @@ void hns_dist_destroy(hns_dist* d) {
 int hns_dist_set_plan(hns_dist* d, hns_state* s, int n_peers, const int* peer_ranks, const uint64_t* n_send, const int32_t* const* send_ids,
                       const uint64_t* n_recv, const int32_t* const* recv_ids, uint64_t n_owned, const int32_t* owned_ids) {
 	if (!d || !s || n_peers < 0 || (n_owned && !owned_ids)) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument");
+	mg_release(d);  // its parent table is per local leaf of the previous plan
 	{
 		// owned = boundary (in some send list) + interior; kernels then skip the ghost leaves altogether
 		std::vector<char> is_boundary(s->grid->num_leaves, 0);
@@ -520,6 +548,7 @@ int hns_dist_reset_error(hns_dist* d) {
 static int check_device_error(hns_dist* d) {
 	uint32_t e = 0;
 	if (d->d_err) HNS_CUDA(cudaMemcpy(&e, d->d_err, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+	if ((e & 0xffu) == 1u + kChMgGather) return fail(HNS_ERR_RUNTIME, "the multigrid level-1 gather timed out waiting for a rank: the frame ran on a stale coarse right-hand side");
 	if (e & 0xffu) return fail(HNS_ERR_RUNTIME, "ghost exchange timed out waiting for a peer on channel " + std::to_string((e & 0xffu) - 1) + ": the frame ran on stale ghosts");
 	if (e & 0x100u)
 		return fail(HNS_ERR_RUNTIME, "a semi-Lagrangian sample landed beyond the one-leaf ghost layer of this shard (CFL too large for a sharded run): the result may differ from the single-GPU frame");
@@ -576,6 +605,7 @@ static int exchange_channel(hns_dist* d, hns_state* s, int channel, int n_fields
 int hns_dist_exchange(hns_dist* d, hns_state* s, int n_fields, const int* fields, void* stream) {
 	if (!d || !s || n_fields <= 0 || n_fields > d->max_fields) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument");
 	if (!d->comm && d->world > 1) return fail(HNS_ERR_RUNTIME, "no NCCL communicator (hns_dist_create without an id) and the peer-memory exchange is not connected");
+	if (d->peers.empty()) return HNS_OK;  // a single rank (or one that shares no leaf): nothing to send or receive
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
 	for (auto& p : d->peers) {
 		uint64_t off = 0;
@@ -752,6 +782,113 @@ static int fused_pressure(hns_dist* d, hns_state* s, int iterations, float omega
 	return HNS_OK;
 }
 
+// `iterations` red-black iterations on the owned leaves with the ghost exchange of each swept colour, in two software-pipelined streams.
+// Interior leaves (no ghost neighbour) are swept on the caller's stream, boundary leaves and the exchange of their freshly swept colour
+// on comm_stream:
+//   caller's stream:  I_1        I_2        I_3   ...      I_k needs I_{k-1} (in order) and B_{k-1} (event)
+//   comm_stream:      B_1 x_1    B_2 x_2    B_3 x_3 ...    B_k needs B_{k-1}, x_{k-1} (in order) and I_{k-1} (event)
+// Half-sweep k reads colour c_{k-1} and writes colour c_k, so I_k and B_k/x_k never touch the same colour of the same leaf at the same
+// time, and the exchange latency disappears behind the interior sweep as long as B + x is the shorter chain. On return the caller's
+// stream has joined the exchanges: the ghosts of both colours are current. mg_flags: the multigrid solve's flag channels (peer memory).
+static int pipelined_sweeps(hns_dist* d, hns_state* s, int iterations, float omega, bool mg_flags, cudaStream_t st) {
+	GridView vb = s->grid->view, vi = s->grid->view;
+	vb.list = d->d_boundary, vb.num_list = d->n_boundary, vb.list_nbr = d->d_boundary_nbr;
+	vi.list = d->d_interior, vi.num_list = d->n_interior, vi.list_nbr = d->d_interior_nbr;
+	const float dx = s->grid->voxel_size;
+	const int fred[1] = {6}, fblk[1] = {7};
+	cudaStream_t bs = d->comm_stream;
+	int rc;
+	HNS_CUDA(cudaEventRecord(d->ev_I[1], st));  // "I_0": everything before the solve
+	HNS_CUDA(cudaEventRecord(d->ev_B[1], bs));  // "B_0": nothing
+	int k = 0;
+	for (int it = 0; it < iterations; ++it)
+		for (int color = 0; color < 2; ++color, ++k) {
+			const int cur = k & 1, prev = cur ^ 1;
+			HNS_CUDA(cudaStreamWaitEvent(bs, d->ev_I[prev], 0));
+			if (d->n_boundary) launch_rbgs_color(vb, s->div, s->p, dx, color, omega, color, bs);
+			HNS_CUDA(cudaEventRecord(d->ev_B[cur], bs));
+			HNS_CUDA(cudaStreamWaitEvent(st, d->ev_B[prev], 0));
+			if (d->n_interior) launch_rbgs_color(vi, s->div, s->p, dx, color, omega, color, st);
+			HNS_CUDA(cudaEventRecord(d->ev_I[cur], st));
+			if (!mg_flags) rc = exchange_channel(d, s, 2 + color, 1, color ? fblk : fred, bs);
+			else rc = d->peers.empty() ? HNS_OK : exchange_p2p(d, s, kChMgPressure + color, 1, color ? fblk : fred, bs, nullptr, 2 + color, 0);
+			if (rc) return rc;
+		}
+	HNS_CUDA(cudaEventRecord(d->ev_exchanged, bs));
+	HNS_CUDA(cudaStreamWaitEvent(st, d->ev_exchanged, 0));
+	return HNS_OK;
+}
+
+// The multigrid solve of a sharded frame: `cycles` V(nu_pre, nu_post) cycles whose level 0 is this rank's shard and whose levels >= 1 are
+// replicated. Every kernel sees the inputs it sees in the single-GPU v_cycle (multigrid.cu), so the owned voxels come out bit for bit
+// the same:
+//   1. pre-smoothing: pipelined_sweeps, ghosts of both colours current afterwards;
+//   2. residual + restriction over the owned leaves, stored straight into every rank's level-1 rhs (k_mg_residual<..., kGather>). A
+//      level-1 cell is 2x2x2 fine voxels of ONE fine leaf, and every fine leaf has one owner, so the ranks write disjoint octants whose
+//      union is the single-GPU level-1 rhs; octants without a fine leaf stay 0 from the allocation on (so nothing clears the array);
+//   3. signal "gather c done" to every rank, wait for every rank's;
+//   4. levels 1 .. n-1 locally (mg_coarse_cycle, a CUDA graph per parity);
+//   5. prolongation over the owned leaves (it reads only level-1 corrections, which every rank has computed identically);
+//   6. exchange of both pressure colours: the prolongation changed the owned leaves' values the peers hold as ghosts (the next red sweep
+//      reads black ghosts; with nu_post = 0 the next residual, or the gradient pass, reads both);
+//   7. post-smoothing: pipelined_sweeps.
+// Ordering of the gather (c = the global gather number, which continues across frames). The level-1 rhs is double-buffered by the
+// parity of c. Rank A stores gather c + 2 into rank B's buffer c & 1 only after A has waited for every rank's flag c + 1 (A's wait of
+// cycle c + 1 precedes its coarse solve of c + 1, which precedes its restriction of c + 2, all on one stream). B raises flag c + 1 from
+// its stream after its restriction of c + 1, which follows its coarse solve of cycle c -- the last reader of buffer c & 1. So no store
+// into a buffer can overtake the coarse solve still reading it, also between two ranks that share no ghost leaf and are otherwise not
+// held back by each other's sweeps. The flag a rank waits for in cycle c is raised after the stores of cycle c (k_signal fences them).
+// The pressure exchanges of steps 1, 6, 7 alternate red, black, red, ... on flag channels 8 / 9, so a landing region is reused only
+// after the peer has signalled the other colour, which it does after unpacking the previous use (as in the red-black solve).
+static int sharded_mg_pressure(hns_dist* d, hns_state* s, cudaStream_t st) {
+	auto& m = d->smg;
+	if (!m.ready) return fail(HNS_ERR_RUNTIME, "the sharded multigrid solver is set but not connected (hns_dist_mg_connect, hns_dist_mg_finish)");
+	hns_mg* mg = m.mg;
+	const int n = int(mg->lv.size());
+	const GridView g = s->view();
+	const float dx = s->grid->voxel_size;
+	const int np = d->world - 1;
+	const int fp[2] = {6, 7};
+	int rc;
+	for (int c = 0; c < m.cycles; ++c) {
+		if (n == 1) {  // a one-level hierarchy: plain red-black sweeps, like v_cycle
+			if ((rc = pipelined_sweeps(d, s, m.nu_pre + m.nu_post, m.omega, true, st))) return rc;
+			continue;
+		}
+		if ((rc = pipelined_sweeps(d, s, m.nu_pre, m.omega, true, st))) return rc;
+		const uint32_t seq = ++m.seq;
+		const int par = int(seq & 1u);
+		launch_mg_restrict_gather(g, s->p, s->div, dx, m.d_parent, m.d_gather[par], d->world, st);
+		if (np > 0) {
+			HNS_LAUNCH(k_signal, 1, 32, 0, st, m.d_sig, np, kChMgGather, seq);
+			HNS_LAUNCH(k_wait, 1, 32, 0, st, m.d_wait, np, kChMgGather, seq, d->d_err);
+		}
+		float* const base = reinterpret_cast<float*>(m.block + m.flag_bytes) + uint64_t(par) * m.rhs_floats;
+		float* const rhs1[2] = {base, base + m.rhs_floats / 2};
+		if (mg->use_graph) {
+			cudaGraphExec_t& G = m.graph[par];
+			if (G && m.graph_coarsest[par] != mg->coarsest_iterations) cudaGraphExecDestroy(G), G = nullptr;
+			if (!G) G = mg_capture_coarse(mg, rhs1, m.nu_pre, m.nu_post, m.omega, &m.graph_launches[par]), m.graph_coarsest[par] = mg->coarsest_iterations;
+			if (G) {
+				HNS_CUDA(cudaGraphLaunch(G, st));
+				g_launches.fetch_add(m.graph_launches[par], std::memory_order_relaxed);
+			} else {
+				mg_coarse_cycle(mg, rhs1, m.nu_pre, m.nu_post, m.omega, st);
+			}
+		} else {
+			mg_coarse_cycle(mg, rhs1, m.nu_pre, m.nu_post, m.omega, st);
+		}
+		launch_mg_prolong(g, s->p, nullptr, m.d_parent, mg->lv[1].grid->view, mg->lv[1].p, st);
+		for (int color = 0; color < 2 && !d->peers.empty(); ++color)
+			if ((rc = exchange_p2p(d, s, kChMgPressure + color, 1, fp + color, st, nullptr, 2 + color, 0))) return rc;
+		if ((rc = pipelined_sweeps(d, s, m.nu_post, m.omega, true, st))) return rc;
+		++m.gathers;
+		m.gather_bytes += uint64_t(d->n_owned) * 256u * uint64_t(np);
+	}
+	HNS_CUDA(cudaGetLastError());
+	return HNS_OK;
+}
+
 static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void* stream, cudaEvent_t* marks, const DistDeps* deps) {
 	if (!d || !s || iterations <= 0 || dt < 0.f) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument");
 	int rc;
@@ -760,7 +897,7 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 		if (marks) cudaEventRecord(marks[mark_i++], static_cast<cudaStream_t>(stream));
 	};
 	mark();
-	const int fvel[3] = {0, 1, 2}, fadv[3] = {3, 4, 5}, fred[1] = {6}, fblk[1] = {7};
+	const int fvel[3] = {0, 1, 2}, fadv[3] = {3, 4, 5};
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
 	s->grp_dist = true;  // this frame re-packs the ghost leaves of the packed advection groups itself (below)
 	if (s->skip_scalar >= 0 && s->skip_scalar != s->n_scalars - 1)
@@ -824,39 +961,15 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 	}
 	mark();
 	if ((rc = hns_state_pressure_init(s, stream))) return rc;
-	const float omega = hns_omega_compute(s->grid->voxel_size);
-	{
-		// Two software-pipelined streams. Interior leaves (no ghost neighbour) are swept on the caller's stream, boundary leaves
-		// and the exchange of their freshly swept colour on comm_stream:
-		//   caller's stream:  I_1        I_2        I_3   ...      I_k needs I_{k-1} (in order) and B_{k-1} (event)
-		//   comm_stream:      B_1 x_1    B_2 x_2    B_3 x_3 ...    B_k needs B_{k-1}, x_{k-1} (in order) and I_{k-1} (event)
-		// Half-sweep k reads colour c_{k-1} and writes colour c_k, so I_k and B_k/x_k never touch the same colour of the same leaf
-		// at the same time, and the exchange latency disappears behind the interior sweep as long as B + x is the shorter chain.
-		GridView vb = s->grid->view, vi = s->grid->view;
-		vb.list = d->d_boundary, vb.num_list = d->n_boundary, vb.list_nbr = d->d_boundary_nbr;
-		vi.list = d->d_interior, vi.num_list = d->n_interior, vi.list_nbr = d->d_interior_nbr;
-		const float dx = s->grid->voxel_size;
-		cudaStream_t bs = d->comm_stream;
+	if (d->smg.mg) {
+		if ((rc = sharded_mg_pressure(d, s, st))) return rc;
+	} else {
+		const float omega = hns_omega_compute(s->grid->voxel_size);
 		const bool fused = d->p2p && d->fused_push && d->n_boundary > 0;
 		if (fused) {
 			if ((rc = fused_pressure(d, s, iterations, omega, st, marks != nullptr))) return rc;
-		} else {
-			HNS_CUDA(cudaEventRecord(d->ev_I[1], st));  // "I_0": everything before the solve
-			HNS_CUDA(cudaEventRecord(d->ev_B[1], bs));  // "B_0": nothing
-			int k = 0;
-			for (int it = 0; it < iterations; ++it)
-				for (int color = 0; color < 2; ++color, ++k) {
-					const int cur = k & 1, prev = cur ^ 1;
-					HNS_CUDA(cudaStreamWaitEvent(bs, d->ev_I[prev], 0));
-					if (d->n_boundary) launch_rbgs_color(vb, s->div, s->p, dx, color, omega, color, bs);
-					HNS_CUDA(cudaEventRecord(d->ev_B[cur], bs));
-					HNS_CUDA(cudaStreamWaitEvent(st, d->ev_B[prev], 0));
-					if (d->n_interior) launch_rbgs_color(vi, s->div, s->p, dx, color, omega, color, st);
-					HNS_CUDA(cudaEventRecord(d->ev_I[cur], st));
-					if ((rc = exchange_channel(d, s, 2 + color, 1, color ? fblk : fred, bs))) return rc;
-				}
-			HNS_CUDA(cudaEventRecord(d->ev_exchanged, bs));
-			HNS_CUDA(cudaStreamWaitEvent(st, d->ev_exchanged, 0));
+		} else if ((rc = pipelined_sweeps(d, s, iterations, omega, false, st))) {
+			return rc;
 		}
 	}
 	mark();
@@ -885,6 +998,141 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 	d->vel_exchanged_version = s->vel_version;
 	mark();
 	return rc;
+}
+
+// ---- sharded multigrid solver: setup ------------------------------------------------------------------------------------------
+// 1. every rank: hns_dist_set_pressure_solver -> the IPC handle of its block (flag words + the two level-1 rhs arrays)
+// 2. the caller all-gathers the handles;  3. hns_dist_mg_connect for every other rank;  4. hns_dist_mg_finish
+static void mg_release(hns_dist* d) {
+	auto& m = d->smg;
+	for (void*& p : m.ipc)
+		if (p) cudaIpcCloseMemHandle(p), p = nullptr;
+	for (auto& g : m.graph)
+		if (g) cudaGraphExecDestroy(g), g = nullptr;
+	cudaFree(m.d_parent), cudaFree(m.block), cudaFree(m.d_gather[0]), cudaFree(m.d_gather[1]), cudaFree(m.d_sig), cudaFree(m.d_wait);
+	const uint64_t gathers = m.gathers, bytes = m.gather_bytes;
+	m = hns_dist::ShardedMg{};
+	m.gathers = gathers, m.gather_bytes = bytes;  // counters of the run, not of one set-up
+}
+
+int hns_dist_set_pressure_solver(hns_dist* d, hns_state* s, hns_mg* mg, const int32_t* local_to_global, int cycles, int nu_pre, int nu_post,
+                                 float omega_smooth, uint8_t* handle_out64) {
+	if (!d || !s) return fail(HNS_ERR_INVALID_ARGUMENT, "null argument");
+	if (s != d->bound_state) return fail(HNS_ERR_INVALID_ARGUMENT, "the state is not the one hns_dist_set_plan was given");
+	HNS_CUDA(cudaDeviceSynchronize());  // a frame in flight may still use what is released here
+	mg_release(d);
+	if (!mg) return HNS_OK;  // back to the red-black solve
+	if (cycles <= 0 || nu_pre < 0 || nu_post < 0 || nu_pre + nu_post == 0)
+		return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument: cycles must be > 0, nu_pre and nu_post >= 0 and not both 0");
+	if (!(omega_smooth > 0.f && omega_smooth < 2.f)) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument: omega_smooth must lie in (0, 2)");
+	if (d->world > 1 && !d->p2p)
+		return fail(HNS_ERR_UNSUPPORTED, "the sharded multigrid solve gathers the level-1 right-hand side through peer memory: connect the "
+		                                 "peer-memory exchange (hns_dist_ipc_*) first; the NCCL fallback has no such path");
+	if (d->world - 1 > 32) return fail(HNS_ERR_UNSUPPORTED, "the sharded multigrid solve supports at most 33 ranks");
+	if (d->world > 1 && !handle_out64) return fail(HNS_ERR_INVALID_ARGUMENT, "handle_out64 is null");
+	const hns_grid* local = s->grid;
+	const uint64_t Ll = local->num_leaves;
+	if (mg->lv.empty()) return fail(HNS_ERR_INVALID_ARGUMENT, "empty multigrid hierarchy");
+	const hns_grid* global = mg->lv[0].grid;
+	const uint64_t Lg = global->num_leaves;
+	if (Ll && !local_to_global) return fail(HNS_ERR_INVALID_ARGUMENT, "local_to_global is null");
+	if (global->voxel_size != local->voxel_size) return fail(HNS_ERR_INVALID_ARGUMENT, "the hierarchy's voxel size differs from the shard's");
+	if (Ll > Lg)
+		return fail(HNS_ERR_INVALID_ARGUMENT, "the hierarchy's level 0 has " + std::to_string(Lg) + " leaves, fewer than the shard's " + std::to_string(Ll) +
+		                                          ": it was not built over the global grid");
+	std::vector<char> seen(Lg, 0);
+	for (uint64_t i = 0; i < Ll; ++i) {
+		const int32_t id = local_to_global[i];
+		if (id < 0 || uint64_t(id) >= Lg)
+			return fail(HNS_ERR_INVALID_ARGUMENT, "local_to_global[" + std::to_string(i) + "] = " + std::to_string(id) + " is not a leaf of the hierarchy's level 0 (" +
+			                                          std::to_string(Lg) + " leaves)");
+		if (seen[id]++) return fail(HNS_ERR_INVALID_ARGUMENT, "local_to_global lists global leaf " + std::to_string(id) + " twice");
+	}
+	{
+		// every local leaf must BE the global leaf it is mapped to: same origin
+		std::vector<int4> go(Lg), lo(Ll);
+		if (Lg) HNS_CUDA(cudaMemcpy(go.data(), global->d_origin, Lg * sizeof(int4), cudaMemcpyDeviceToHost));
+		if (Ll) HNS_CUDA(cudaMemcpy(lo.data(), local->d_origin, Ll * sizeof(int4), cudaMemcpyDeviceToHost));
+		for (uint64_t i = 0; i < Ll; ++i) {
+			const int4 a = lo[i], b = go[local_to_global[i]];
+			if (a.x != b.x || a.y != b.y || a.z != b.z)
+				return fail(HNS_ERR_INVALID_ARGUMENT, "local leaf " + std::to_string(i) + " lies at (" + std::to_string(a.x) + ", " + std::to_string(a.y) + ", " +
+				                                          std::to_string(a.z) + ") but global leaf " + std::to_string(local_to_global[i]) +
+				                                          " of the hierarchy does not: it was built over another grid");
+		}
+	}
+	auto& m = d->smg;
+	const int n = int(mg->lv.size());
+	const uint64_t L1 = n > 1 ? mg->lv[1].grid->num_leaves : 0;
+	if (n > 1 && Ll) {
+		std::vector<int32_t> gp(Lg), lp(Ll);
+		HNS_CUDA(cudaMemcpy(gp.data(), mg->lv[0].parent, Lg * sizeof(int32_t), cudaMemcpyDeviceToHost));
+		for (uint64_t i = 0; i < Ll; ++i) lp[i] = gp[local_to_global[i]];
+		HNS_CUDA(cudaMalloc(&m.d_parent, Ll * sizeof(int32_t)));
+		HNS_CUDA(cudaMemcpy(m.d_parent, lp.data(), Ll * sizeof(int32_t), cudaMemcpyHostToDevice));
+	}
+	// flag word of rank r in every block: word 16 r + kChMgGather (k_signal / k_wait address flags[t] + channel)
+	m.flag_bytes = (uint64_t(d->world) * 16u * sizeof(uint32_t) + 255u) & ~uint64_t(255);
+	m.rhs_floats = L1 * 512u;
+	const uint64_t bytes = m.flag_bytes + 2u * m.rhs_floats * sizeof(float);
+	HNS_CUDA(cudaMalloc(&m.block, bytes));
+	HNS_CUDA(cudaMemset(m.block, 0, bytes));  // once: octants without a fine leaf stay 0, and the peers write into it from now on
+	if (handle_out64) {
+		cudaIpcMemHandle_t h;
+		HNS_CUDA(cudaIpcGetMemHandle(&h, m.block));
+		std::memcpy(handle_out64, &h, 64);
+	}
+	m.ipc.assign(size_t(d->world), nullptr);
+	m.mg = mg, m.cycles = cycles, m.nu_pre = nu_pre, m.nu_post = nu_post, m.omega = omega_smooth;
+	return HNS_OK;
+}
+
+int hns_dist_mg_connect(hns_dist* d, int rank, const uint8_t* handle64) {
+	if (!d || !handle64 || rank < 0 || rank >= d->world || rank == d->rank) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument");
+	auto& m = d->smg;
+	if (!m.block) return fail(HNS_ERR_INVALID_ARGUMENT, "hns_dist_set_pressure_solver has not been called");
+	cudaIpcMemHandle_t h;
+	std::memcpy(&h, handle64, 64);
+	if (m.ipc[rank]) cudaIpcCloseMemHandle(m.ipc[rank]), m.ipc[rank] = nullptr;
+	HNS_CUDA(cudaIpcOpenMemHandle(&m.ipc[rank], h, cudaIpcMemLazyEnablePeerAccess));
+	return HNS_OK;
+}
+
+int hns_dist_mg_finish(hns_dist* d) {
+	if (!d) return fail(HNS_ERR_INVALID_ARGUMENT, "null argument");
+	auto& m = d->smg;
+	if (!m.block) return fail(HNS_ERR_INVALID_ARGUMENT, "hns_dist_set_pressure_solver has not been called");
+	const int W = d->world;
+	std::vector<float*> gat[2] = {std::vector<float*>(2 * W), std::vector<float*>(2 * W)};
+	std::vector<uint32_t*> sig, wait;
+	for (int r = 0; r < W; ++r) {
+		uint8_t* b = r == d->rank ? m.block : static_cast<uint8_t*>(m.ipc[r]);
+		if (!b) return fail(HNS_ERR_RUNTIME, "rank " + std::to_string(r) + " is not connected (hns_dist_mg_connect)");
+		for (int par = 0; par < 2; ++par) {
+			float* rhs = reinterpret_cast<float*>(b + m.flag_bytes) + uint64_t(par) * m.rhs_floats;
+			gat[par][2 * r] = rhs, gat[par][2 * r + 1] = rhs + m.rhs_floats / 2;
+		}
+		if (r == d->rank) continue;
+		sig.push_back(reinterpret_cast<uint32_t*>(b) + 16 * d->rank);
+		wait.push_back(reinterpret_cast<uint32_t*>(m.block) + 16 * r);
+	}
+	for (int par = 0; par < 2; ++par) {
+		cudaFree(m.d_gather[par]);
+		m.d_gather[par] = nullptr;
+		HNS_CUDA(cudaMalloc(&m.d_gather[par], gat[par].size() * sizeof(float*)));
+		HNS_CUDA(cudaMemcpy(m.d_gather[par], gat[par].data(), gat[par].size() * sizeof(float*), cudaMemcpyHostToDevice));
+	}
+	cudaFree(m.d_sig), cudaFree(m.d_wait);
+	m.d_sig = m.d_wait = nullptr;
+	if (!sig.empty()) {
+		HNS_CUDA(cudaMalloc(&m.d_sig, sig.size() * sizeof(uint32_t*)));
+		HNS_CUDA(cudaMalloc(&m.d_wait, wait.size() * sizeof(uint32_t*)));
+		HNS_CUDA(cudaMemcpy(m.d_sig, sig.data(), sig.size() * sizeof(uint32_t*), cudaMemcpyHostToDevice));
+		HNS_CUDA(cudaMemcpy(m.d_wait, wait.data(), wait.size() * sizeof(uint32_t*), cudaMemcpyHostToDevice));
+	}
+	m.seq = 0;  // the blocks are fresh on every rank
+	m.ready = true;
+	return HNS_OK;
 }
 
 // after hns_dist_frame_timed: microseconds inside pressure half-sweep 20, all relative to the start of its boundary sweep:
@@ -957,6 +1205,8 @@ int hns_dist_allreduce_sum(hns_dist* d, double* inout_host, int n, void* stream)
 	return HNS_OK;
 }
 uint64_t hns_dist_bytes_sent(const hns_dist* d) { return d ? d->bytes_sent : 0; }
+uint64_t hns_dist_mg_gathers(const hns_dist* d) { return d ? d->smg.gathers : 0; }
+uint64_t hns_dist_mg_gather_bytes(const hns_dist* d) { return d ? d->smg.gather_bytes : 0; }
 uint64_t hns_dist_exchanges(const hns_dist* d) { return d ? d->exchanges : 0; }
 
 }  // extern "C"

@@ -790,12 +790,16 @@ void launch_vorticity_force(const GridView& g, const float* const vel[3], const 
 //   prolong    p += trilinear interpolation of the parents' correction   (weights 3/4, 1/4 per axis; z, then y, then x)
 // =============================================================================================================
 // kNorm: also accumulates sum r^2 and sum rhs^2 in fp64 (per-thread partial sums, warp shuffles, one atomic per warp).
-template <bool kMask, bool kRestrict, bool kNorm>
+// kGather (with kRestrict, sharded runs): the restricted octant goes to n_gather colour-split arrays, gather[2 t] / gather[2 t + 1] = red /
+// black of target t -- every rank's copy of the level-1 right-hand side, peers' ones mapped over NVLink -- instead of crhs. Plain stores:
+// the flag that publishes them is raised by a later kernel in the same stream.
+template <bool kMask, bool kRestrict, bool kNorm, bool kGather = false>
 __global__ void __launch_bounds__(256) k_mg_residual(GridView g, const float* __restrict__ p_red, const float* __restrict__ p_blk,
                                                      const float* __restrict__ rhs_red, const float* __restrict__ rhs_blk, float inv_dx2,
                                                      const float* __restrict__ diag_red, const float* __restrict__ diag_blk,
                                                      const int32_t* __restrict__ parent,
-                                                     float* __restrict__ crhs_red, float* __restrict__ crhs_blk, double* __restrict__ sums) {
+                                                     float* __restrict__ crhs_red, float* __restrict__ crhs_blk, double* __restrict__ sums,
+                                                     float* const* __restrict__ gather, int n_gather) {
 	RowCtx c;
 	if (!make_row_ctx(g, c)) return;
 	const uint64_t self = c.self();
@@ -842,8 +846,17 @@ __global__ void __launch_bounds__(256) k_mg_residual(GridView g, const float* __
 			const int X = ((o.x >> 3) & 1) * 4 + (c.x >> 1), Y = ((o.y >> 3) & 1) * 4 + (c.y >> 1), oz = (o.z >> 3) & 1;
 			const uint32_t base = uint32_t(__ldg(parent + c.leaf)) * 256u + uint32_t(X * 32 + Y * 4 + 2 * oz);
 			const bool sp = (X + Y) & 1;  // parent cells z = 4 oz + k have colour (X + Y + k) & 1
-			*reinterpret_cast<float2*>((sp ? crhs_blk : crhs_red) + base) = make_float2(q[0], q[2]);
-			*reinterpret_cast<float2*>((sp ? crhs_red : crhs_blk) + base) = make_float2(q[1], q[3]);
+			if (kGather) {
+				for (int t = 0; t < n_gather; ++t) {
+					float* const gr = gather[2 * t];
+					float* const gb = gather[2 * t + 1];
+					*reinterpret_cast<float2*>((sp ? gb : gr) + base) = make_float2(q[0], q[2]);
+					*reinterpret_cast<float2*>((sp ? gr : gb) + base) = make_float2(q[1], q[3]);
+				}
+			} else {
+				*reinterpret_cast<float2*>((sp ? crhs_blk : crhs_red) + base) = make_float2(q[0], q[2]);
+				*reinterpret_cast<float2*>((sp ? crhs_red : crhs_blk) + base) = make_float2(q[1], q[3]);
+			}
 		}
 	}
 }
@@ -856,7 +869,7 @@ void launch_mg_residual(const GridView& g, const float* const p[2], const float*
 	float* cb = coarse_rhs ? coarse_rhs[1] : nullptr;
 	const float* dr = diag ? diag[0] : nullptr;
 	const float* db = diag ? diag[1] : nullptr;
-#define HNS_MG_RES(M, R, N) HNS_LAUNCH((k_mg_residual<M, R, N>), grid, 256, 0, st, g, p[0], p[1], rhs[0], rhs[1], inv_dx2, dr, db, parent, cr, cb, sums)
+#define HNS_MG_RES(M, R, N) HNS_LAUNCH((k_mg_residual<M, R, N>), grid, 256, 0, st, g, p[0], p[1], rhs[0], rhs[1], inv_dx2, dr, db, parent, cr, cb, sums, nullptr, 0)
 	const bool R = coarse_rhs != nullptr, N = sums != nullptr;
 	if (diag) {
 		if (R && N) HNS_MG_RES(true, true, true);
@@ -868,6 +881,12 @@ void launch_mg_residual(const GridView& g, const float* const p[2], const float*
 		else HNS_MG_RES(false, false, true);
 	}
 #undef HNS_MG_RES
+}
+void launch_mg_restrict_gather(const GridView& g, const float* const p[2], const float* const rhs[2], float dx, const int32_t* parent,
+                               float* const* gather, int n_gather, cudaStream_t st) {
+	if (!g.count() || n_gather <= 0) return;
+	HNS_LAUNCH((k_mg_residual<false, true, false, true>), (g.count() + 3) / 4, 256, 0, st, g, p[0], p[1], rhs[0], rhs[1], 1.0f / (dx * dx), nullptr,
+	           nullptr, parent, nullptr, nullptr, nullptr, gather, n_gather);
 }
 
 // sum of squares of a colour-split field over the listed leaves (fp64)

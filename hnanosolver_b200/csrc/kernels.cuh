@@ -111,6 +111,10 @@ void launch_rbgs_color_masked(const GridView& g, const float* const rhs[2], floa
                               const float* const diag[2], cudaStream_t st);
 void launch_mg_residual(const GridView& g, const float* const p[2], const float* const rhs[2], float dx, const float* const diag[2], const int32_t* parent,
                         float* const coarse_rhs[2], double* sums, cudaStream_t st);
+// the fine level's residual restricted, as launch_mg_residual with a parent level, but stored into n_gather colour-split arrays: gather[2 t],
+// gather[2 t + 1] = red / black half of target t (a sharded run's level-1 right-hand side on every rank, dist.cu)
+void launch_mg_restrict_gather(const GridView& g, const float* const p[2], const float* const rhs[2], float dx, const int32_t* parent,
+                               float* const* gather, int n_gather, cudaStream_t st);
 void launch_sum_squares(const GridView& g, const float* const f[2], double* sum, cudaStream_t st);
 void launch_mg_prolong(const GridView& g, float* const p[2], const float* const diag[2], const int32_t* parent, const GridView& coarse,
                        const float* const e[2], cudaStream_t st);

@@ -7,7 +7,7 @@
 // the smoother (the same red-black update) and the acceptance gates of SURVEY.md Appendix A-9: relative Poisson residual and the
 // divergence of the projected velocity against what the reference's fixed-count solve reaches.
 //
-// Hierarchy: level k + 1 has cells of twice the size; a cell is inside the domain iff one of its 8 children is. Leaves of level k + 1
+// Hierarchy: level k + 1 has cells of twice the size; a cell is inside the domain iff all 8 of its children are. Leaves of level k + 1
 // are 2x2x2 leaves of level k, so every level is again a set of dense 8^3 bricks with a NanoVDB-ordered leaf list, a neighbour table
 // (topology.cu builds both) and colour-split p / rhs arrays -- the fine-level sweep kernel runs unchanged on every level, plus a
 // per-row byte mask for the cells of a coarse brick that lie outside the domain. The last level is a single leaf (or `max_levels`).
@@ -23,44 +23,6 @@
 #include "kernels.cuh"
 
 using namespace hns;
-
-struct hns_mg {
-	struct Level {
-		hns_grid* grid = nullptr;     // level 0: the caller's grid (borrowed)
-		bool own_grid = false;
-		float* p[2] = {nullptr, nullptr};    // levels >= 1 (level 0 uses the state's pressure / divergence)
-		float* rhs[2] = {nullptr, nullptr};
-		float* diag[2] = {nullptr, nullptr};  // colour-split diagonal of the level's operator, 0 = cell outside the domain; null on level 0
-		const float* const* diag_or_null() const { return diag[0] ? diag : nullptr; }
-		int32_t* parent = nullptr;    // [L] leaf id on the next level; null on the last
-		float dx = 0.f;
-		uint64_t cells = 0;           // cells inside the domain
-	};
-	std::vector<Level> lv;
-	double* d_sums = nullptr;         // device double[2]
-	double* h_sums = nullptr;         // pinned
-	uint64_t last_nonempty_count = 0;  // of the last level: non-empty leaves, and (when that is 1) which one
-	int64_t last_nonempty_leaf = -1;
-	int coarsest_iterations = 32;
-	float coarsest_omega = 1.5f;      // a one-leaf last level is solved, not smoothed: SOR near its optimum for 8 cells per axis
-	// statistics of the last solve
-	int last_cycles = 0;
-	double last_rel_residual = -1.0;
-	// One V-cycle is ~10 launches per level, most of them on levels far too small to fill the GPU: issued one by one they cost their
-	// launch latency (measured: 1.27 of the 2.13 ms of two cycles on the 512^3 workload). The cycle is therefore captured once into a
-	// CUDA graph (on a private stream: capture executes nothing) and replayed; the key is everything the captured launches depend on.
-	struct CycleGraph {
-		cudaGraphExec_t exec = nullptr;
-		const void* state = nullptr;
-		hns::GridView view{};  // the fine level's view (pointers, counts, work list)
-		const void *p = nullptr, *rhs = nullptr;
-		int nu_pre = -1, nu_post = -1, coarsest_iterations = -1;
-		float omega = 0.f;
-		uint64_t launches = 0;
-	} graph;
-	cudaStream_t capture_stream = nullptr;
-	bool use_graph = true;  // HNS_MG_GRAPH=0: issue every launch directly (A/B switch)
-};
 
 namespace {
 
@@ -230,45 +192,93 @@ static void residual_sums_async(const GridView& g, const float* const p[2], cons
 	launch_mg_residual(g, p, rhs, dx, nullptr, nullptr, nullptr, d_sums, st);
 }
 
-// One V(nu_pre, nu_post) cycle on the state's divergence / pressure. Level 0 relaxes the caller's p in place; on every coarser level
-// the correction starts from 0.
-static void v_cycle(hns_mg* mg, hns_state* s, int nu_pre, int nu_post, float omega, cudaStream_t st) {
+// Levels 1 .. n-1 of one V(nu_pre, nu_post) cycle (n > 1): the right-hand side of level 1 is `rhs1` (the hierarchy's own array, or a sharded
+// run's gathered copy, dist.cu); the correction starts from 0 on every level and ends up in lv[1].p, ready for the prolongation to level 0.
+void mg_coarse_cycle(hns_mg* mg, float* const rhs1[2], int nu_pre, int nu_post, float omega, cudaStream_t st) {
 	const int n = int(mg->lv.size());
-	auto P = [&](int k) -> float* const* { return k == 0 ? s->p : mg->lv[k].p; };
-	auto F = [&](int k) -> float* const* { return k == 0 ? s->div : mg->lv[k].rhs; };
-	auto view = [&](int k) { return k == 0 ? s->view() : mg->lv[k].grid->view; };
+	auto P = [&](int k) -> float* const* { return mg->lv[k].p; };
+	auto F = [&](int k) -> float* const* { return k == 1 ? rhs1 : mg->lv[k].rhs; };
 	auto smooth = [&](int k, int iters) {
-		const GridView g = view(k);
+		const GridView g = mg->lv[k].grid->view;
 		for (int it = 0; it < iters; ++it)
-			for (int color = 0; color < 2; ++color) {
-				if (k == 0) launch_rbgs_color(g, F(k), P(k), mg->lv[k].dx, color, omega, color, st);
-				else launch_rbgs_color_masked(g, F(k), P(k), mg->lv[k].dx, color, omega, mg->lv[k].diag, st);
-			}
+			for (int color = 0; color < 2; ++color) launch_rbgs_color_masked(g, F(k), P(k), mg->lv[k].dx, color, omega, mg->lv[k].diag, st);
 	};
-	for (int k = 0; k + 1 < n; ++k) {  // down
+	cudaMemsetAsync(mg->lv[1].p[0], 0, mg->lv[1].grid->num_leaves * 512 * sizeof(float), st);
+	for (int k = 1; k + 1 < n; ++k) {  // down
 		smooth(k, nu_pre);
 		hns_mg::Level& c = mg->lv[k + 1];
 		const size_t bytes = c.grid->num_leaves * 512 * sizeof(float);
 		cudaMemsetAsync(c.p[0], 0, bytes, st);
 		cudaMemsetAsync(c.rhs[0], 0, bytes, st);
-		launch_mg_residual(view(k), P(k), F(k), mg->lv[k].dx, mg->lv[k].diag_or_null(), mg->lv[k].parent, c.rhs, nullptr, st);
+		launch_mg_residual(mg->lv[k].grid->view, P(k), F(k), mg->lv[k].dx, mg->lv[k].diag_or_null(), mg->lv[k].parent, c.rhs, nullptr, st);
 	}
 	{  // coarsest
 		hns_mg::Level& c = mg->lv[n - 1];
-		if (n > 1 && mg->last_nonempty_count == 1) {
+		if (mg->last_nonempty_count == 1) {
 			// the whole level is one brick (its other leaves, if any, hold no cell of the domain and stay 0): solved inside one CTA
 			const uint64_t off = uint64_t(mg->last_nonempty_leaf) * 256u;
 			float* const p1[2] = {c.p[0] + off, c.p[1] + off};
-			const float* const f1[2] = {c.rhs[0] + off, c.rhs[1] + off};
+			const float* const f1[2] = {F(n - 1)[0] + off, F(n - 1)[1] + off};
 			const float* const d1[2] = {c.diag[0] + off, c.diag[1] + off};
 			launch_mg_coarsest(p1, f1, d1, c.dx, mg->coarsest_omega, mg->coarsest_iterations, st);
 		}
-		else smooth(n - 1, n > 1 ? mg->coarsest_iterations : nu_pre + nu_post);
+		else smooth(n - 1, mg->coarsest_iterations);
 	}
-	for (int k = n - 2; k >= 0; --k) {  // up
-		launch_mg_prolong(view(k), P(k), mg->lv[k].diag_or_null(), mg->lv[k].parent, mg->lv[k + 1].grid->view, mg->lv[k + 1].p, st);
+	for (int k = n - 2; k >= 1; --k) {  // up
+		launch_mg_prolong(mg->lv[k].grid->view, P(k), mg->lv[k].diag_or_null(), mg->lv[k].parent, mg->lv[k + 1].grid->view, mg->lv[k + 1].p, st);
 		smooth(k, nu_post);
 	}
+}
+
+// One V(nu_pre, nu_post) cycle on the state's divergence / pressure. Level 0 relaxes the caller's p in place; the coarser levels are
+// mg_coarse_cycle.
+static void v_cycle(hns_mg* mg, hns_state* s, int nu_pre, int nu_post, float omega, cudaStream_t st) {
+	const int n = int(mg->lv.size());
+	const GridView g = s->view();
+	const float dx = mg->lv[0].dx;
+	auto smooth = [&](int iters) {
+		for (int it = 0; it < iters; ++it)
+			for (int color = 0; color < 2; ++color) launch_rbgs_color(g, s->div, s->p, dx, color, omega, color, st);
+	};
+	if (n == 1) {  // a one-level hierarchy: plain red-black sweeps
+		smooth(nu_pre + nu_post);
+		return;
+	}
+	smooth(nu_pre);
+	hns_mg::Level& c = mg->lv[1];
+	cudaMemsetAsync(c.rhs[0], 0, c.grid->num_leaves * 512 * sizeof(float), st);
+	launch_mg_residual(g, s->p, s->div, dx, nullptr, mg->lv[0].parent, c.rhs, nullptr, st);
+	mg_coarse_cycle(mg, c.rhs, nu_pre, nu_post, omega, st);
+	launch_mg_prolong(g, s->p, nullptr, mg->lv[0].parent, c.grid->view, c.p, st);
+	smooth(nu_post);
+}
+
+// mg_coarse_cycle captured into a CUDA graph on the hierarchy's private stream (the caller owns the result; null when capture is not
+// possible); *launches = the kernels one replay runs
+cudaGraphExec_t mg_capture_coarse(hns_mg* mg, float* const rhs1[2], int nu_pre, int nu_post, float omega, uint64_t* launches) {
+	*launches = 0;
+	if (!mg->capture_stream && cudaStreamCreateWithFlags(&mg->capture_stream, cudaStreamNonBlocking) != cudaSuccess) {
+		cudaGetLastError();
+		return nullptr;
+	}
+	cudaGraph_t graph = nullptr;
+	const uint64_t before = g_launches.load();
+	if (cudaStreamBeginCapture(mg->capture_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
+		cudaGetLastError();
+		return nullptr;
+	}
+	mg_coarse_cycle(mg, rhs1, nu_pre, nu_post, omega, mg->capture_stream);
+	const cudaError_t e = cudaStreamEndCapture(mg->capture_stream, &graph);
+	*launches = g_launches.load() - before;
+	g_launches.fetch_sub(*launches);  // nothing ran yet: every replay counts them
+	if (e != cudaSuccess || !graph) {
+		cudaGetLastError();
+		return nullptr;
+	}
+	cudaGraphExec_t exec = nullptr;
+	if (cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) exec = nullptr, cudaGetLastError();
+	cudaGraphDestroy(graph);
+	return exec;
 }
 
 // the captured cycle for this (state, parameters), or null when graphs are off / capture is not possible
@@ -337,7 +347,7 @@ extern "C" {
 
 int hns_state_pressure_solve_mg(hns_state* s, hns_mg* mg, int max_cycles, double rel_tol, int nu_pre, int nu_post, float omega_smooth, void* stream) {
 	if (!s || !mg || max_cycles <= 0 || nu_pre < 0 || nu_post < 0 || nu_pre + nu_post == 0) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument");
-	if (s->active) return fail(HNS_ERR_UNSUPPORTED, "the multigrid solve is single-GPU (a sharded state has ghost leaves)");
+	if (s->active) return fail(HNS_ERR_UNSUPPORTED, "this entry point solves single-GPU states (a sharded state has ghost leaves): sharded frames take a multigrid solver through hns_dist_set_pressure_solver");
 	if (!s->n) return HNS_OK;
 	return mg_pressure_solve(s, mg, max_cycles, rel_tol, nu_pre, nu_post, omega_smooth, static_cast<cudaStream_t>(stream));
 }

@@ -269,6 +269,8 @@ class ShardedSimulation:
 
             e = C.c_uint32()
             _lib.check(_lib.lib().hns_dist_error(self._dist, C.byref(e)))
+            if e.value & 0xff == 11:
+                raise RuntimeError("the multigrid level-1 gather timed out waiting for a rank: the frame ran on a stale coarse right-hand side")
             if e.value & 0xff:
                 raise RuntimeError(f"ghost exchange timed out waiting for a peer on channel {(e.value & 0xff) - 1}: the frame ran on stale ghosts")
             if e.value & 0x100:
@@ -297,6 +299,51 @@ class ShardedSimulation:
         from . import _lib
 
         return int(_lib.lib().hns_dist_bytes_sent(self._dist)) if self.native else self.ex.bytes_sent
+
+    def set_pressure_solver(self, global_origins, cycles: int = 2, nu_pre: int = 2, nu_post: int = 2, omega_smooth: float = 1.15,
+                            max_levels: int = 0) -> None:
+        """Collective. frame() / cook() / frame_timed() then solve the pressure with `cycles` sharded V(nu_pre, nu_post) multigrid cycles
+        (hns_dist_set_pressure_solver) instead of the red-black sweeps: level 0 is this shard, the coarse levels -- a Multigrid over the
+        GLOBAL leaf origins `global_origins` (NanoVDB order, as given to make_plan) -- are replicated on every rank. The owned voxels equal
+        Simulation.set_pressure_solver(Multigrid(global grid, max_levels), ...) on one GPU bit for bit. global_origins=None switches
+        back to red-black. Needs the native frame and, with more than one rank, the peer-memory exchange."""
+        import ctypes as C
+
+        from . import _lib
+        from . import launchers as H
+
+        if not self.native:
+            raise NotImplementedError("the sharded multigrid solve needs the native sharded frame (native=True)")
+        L = _lib.lib()
+        if global_origins is None:
+            _lib.check(L.hns_dist_set_pressure_solver(self._dist, self.sim._h, None, None, 0, 0, 0, 0.0, None))
+            self._mg = None
+            return
+        grid = H.create_index_grid_from_origins(global_origins, self.voxel_size)
+        mg = H.Multigrid(grid, max_levels)
+        l2g = np.ascontiguousarray(self.plan.local_ids, np.int32)
+        handle = (C.c_uint8 * 64)()
+        _lib.check(L.hns_dist_set_pressure_solver(self._dist, self.sim._h, mg._h, l2g.ctypes.data_as(_lib.c_i32p), int(cycles), int(nu_pre),
+                                                  int(nu_post), float(omega_smooth), handle))
+        self._mg = (grid, mg)   # the library uses the hierarchy (and it the grid) until the next call
+        if self.plan.world > 1:
+            import torch.distributed as tdist
+
+            handles = [None] * self.plan.world
+            tdist.all_gather_object(handles, bytes(handle))
+            for r, hb in enumerate(handles):
+                if r != self.plan.rank:
+                    _lib.check(L.hns_dist_mg_connect(self._dist, r, (C.c_uint8 * 64).from_buffer_copy(hb)))
+        _lib.check(L.hns_dist_mg_finish(self._dist))
+        if self.plan.world > 1:
+            tdist.barrier()
+
+    @property
+    def mg_gathers(self) -> tuple[int, int]:
+        """(V-cycles that gathered the level-1 right-hand side, bytes this rank stored into the other ranks' copies)"""
+        from . import _lib
+
+        return int(_lib.lib().hns_dist_mg_gathers(self._dist)), int(_lib.lib().hns_dist_mg_gather_bytes(self._dist))
 
     def set_combustion(self, names, params):
         self.sim.set_combustion(True, names.index("fuel"), names.index("waste"), names.index("temperature"), names.index("flame"), params)
@@ -387,10 +434,13 @@ class ShardedSimulation:
 # ------------------------------------------------------------------------------------------------------------------
 def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), fill: float = 0.35, seed: int = 7, iterations: int = 12,
                          frames: int = 2, collision: bool = False, vorticity=(0.0, 1.0), cook: bool = False, combustion: bool = True,
-                         native: bool = True):
+                         native: bool = True, multigrid: dict | None = None):
     """Collective. Runs `frames` sharded frames of a small sparse box and, on rank 0, the same frames on ONE GPU over the whole
     domain; compares the owned voxels of every rank (velocity, every scalar, pressure) with np.array_equal.
-    Returns (ok, report) on rank 0 and (None, None) elsewhere. Two frames exercise the reuse of the velocity ghosts across frames."""
+    Returns (ok, report) on rank 0 and (None, None) elsewhere. Two frames exercise the reuse of the velocity ghosts across frames.
+    multigrid = dict(cycles, nu_pre, nu_post, omega, max_levels, red_black_frames): both sides solve the pressure with that many V-cycles
+    (ShardedSimulation.set_pressure_solver against Simulation.set_pressure_solver over the whole domain); red_black_frames > 0 then
+    switches both back to red-black for that many more frames."""
     import torch
     import torch.distributed as tdist
 
@@ -414,12 +464,20 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
         names, gfields = names + ["collision_sdf"], gfields + [sdf]
     NS = len(gfields)
     P = H.CombustionParams(0.5, 2.0, 1.5, 0.1, float(vorticity[0]), float(vorticity[1]))
+    mgc = None
+    if multigrid is not None:
+        mgc = dict(cycles=2, nu_pre=2, nu_post=2, omega=1.15, max_levels=0, red_black_frames=0)
+        mgc.update(multigrid)
     sh = ShardedSimulation(plan, np.ascontiguousarray(go[plan.local_ids]), wg.voxel_size, NS, device, native=native)
     try:
         if collision:
             sh.sim.set_collision(NS - 1)
         if combustion:
             sh.set_combustion(names, P)
+        if mgc is not None:
+            sh.set_pressure_solver(go, mgc["cycles"], mgc["nu_pre"], mgc["nu_post"], mgc["omega"], mgc["max_levels"])
+        gathers_before = sh.mg_gathers if native else (0, 0)
+        rb_frames = mgc["red_black_frames"] if mgc is not None else 0
         m = np.repeat(plan.owned_local, 512)
         lv, lf = np.ascontiguousarray(wg.velocity[lo]), [np.ascontiguousarray(f[lo]) for f in gfields]
         packed_before = _lib.lib().hns_packed_advection_launches()
@@ -430,15 +488,26 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
                 a[~m] = np.float32(-7.0)
             for _ in range(frames):
                 sh.cook(lv, lf, iterations, wg.dt)
+            if rb_frames:
+                sh.set_pressure_solver(None)
+                for _ in range(rb_frames):
+                    sh.cook(lv, lf, iterations, wg.dt)
             mine = [lv[m]] + [a[m] for a in lf] + [sh.sim.aux(1)[m]]
         else:
             sh.upload(lv, lf)
             for _ in range(frames):
                 sh.frame(iterations, wg.dt)
+            if rb_frames:
+                torch.cuda.synchronize()
+                sh.check_errors()
+                sh.set_pressure_solver(None)
+                for _ in range(rb_frames):
+                    sh.frame(iterations, wg.dt)
             torch.cuda.synchronize()
             sh.check_errors()
             mine = [sh.sim.velocity()[m]] + [sh.sim.scalar(i)[m] for i in range(NS)] + [sh.sim.aux(1)[m]]
         packed_launches = int(_lib.lib().hns_packed_advection_launches() - packed_before)   # third-generation advection launches of this rank
+        gathers = [a - b for a, b in zip(sh.mg_gathers, gathers_before)] if native else [0, 0]
         gathered = [None] * world
         tdist.all_gather_object(gathered, mine)
         ok, report = None, None
@@ -450,8 +519,16 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
                 sim.set_collision(NS - 1)
             if combustion:
                 sim.set_combustion(True, 1, 2, 3, 4, P)
+            ref_mg = None
+            if mgc is not None:
+                ref_mg = H.Multigrid(g, mgc["max_levels"])
+                sim.set_pressure_solver(ref_mg, mgc["cycles"], mgc["nu_pre"], mgc["nu_post"], mgc["omega"])
             for _ in range(frames):
                 sim.step(iterations, wg.dt)
+            if rb_frames:
+                sim.set_pressure_solver(None)
+                for _ in range(rb_frames):
+                    sim.step(iterations, wg.dt)
             sim.sync()
             ref = [sim.velocity()] + [sim.scalar(i) for i in range(NS)] + [sim.aux(1)]
             if cook and collision:
@@ -466,8 +543,8 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
                              + (f", max|diff| {np.abs(got.astype(np.float64) - ref[k]).max():.3e}, first leaves {np.unique(bad // 512)[:6].tolist()}" if bad.size else "") + ")")
             report = dict(ok=ok, leaves=int(go.shape[0]), world=world, frames=frames, iterations=iterations, p2p=bool(getattr(sh, "p2p", False)),
                           native=native, collision=collision, vorticity=list(vorticity), cook=cook, exchanges_per_frame=sh.exchanges // max(frames, 1),
-                          packed_advection_launches=packed_launches,
-                          fields=lines)
+                          packed_advection_launches=packed_launches, multigrid=mgc, mg_gathers=gathers[0], mg_gather_bytes=gathers[1],
+                          mg_levels=ref_mg.num_levels if ref_mg is not None else 0, fields=lines)
             del sim
         tdist.barrier()
         return ok, report

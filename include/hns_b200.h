@@ -253,9 +253,9 @@ int hns_state_residual_sums(hns_state* s, double* out2, void* stream);
 /* *out = sum of squares of the divergence (reference kernel `divergence`, src/Cuda/Kernel.cu:499-519) of the current velocity
  * (of_advected = 0) or of the advected velocity (1). OVERWRITES the state's divergence field. Synchronous. */
 int hns_state_divergence_sum_squares(hns_state* s, int of_advected, double* out, void* stream);
-/* Multigrid hierarchy over an index grid: level k+1 has cells twice the size of level k, a cell belongs to the domain iff one of its 8
- * children does, leaves of level k+1 are 2x2x2 leaves of level k; coarsening stops at a single leaf (or after max_levels; <= 0: no cap).
- * The grid must outlive the hierarchy. */
+/* Multigrid hierarchy over an index grid: level k+1 has cells twice the size of level k, a cell belongs to the domain iff all 8 of its
+ * children do, leaves of level k+1 are 2x2x2 leaves of level k; coarsening stops at a single leaf, when no cell is fully covered any
+ * more, or after max_levels (<= 0: no cap). The grid must outlive the hierarchy. */
 typedef struct hns_mg hns_mg;
 int hns_mg_create(const hns_grid* g, int max_levels, hns_mg** out);
 void hns_mg_destroy(hns_mg* mg);
@@ -357,6 +357,25 @@ int hns_dist_time_sweeps(hns_dist* d, hns_state* s, int mode, int n, void* strea
 int hns_dist_allreduce_sum(hns_dist* d, double* inout_host, int n, void* stream);
 uint64_t hns_dist_bytes_sent(const hns_dist* d);
 uint64_t hns_dist_exchanges(const hns_dist* d);
+/* Sharded multigrid pressure solve: hns_dist_frame / _cook / _frame_timed then run `cycles` V(nu_pre, nu_post) cycles instead of the
+ * red-black solve (`iterations` is then unused). Level 0 is the shard (sweeps on the owned leaves with their ghost exchanges), levels >= 1
+ * are replicated: the ranks' restricted residuals are gathered into every rank's level-1 right-hand side through peer memory, and
+ * every rank runs the coarse levels itself. The owned voxels equal those of hns_state_set_pressure_solver's single-GPU frame bit for
+ * bit. `mg` is an hns_mg over the GLOBAL grid (its levels >= 1 are the single-GPU hierarchy; its coarse arrays are used by this
+ * solver, so do not solve with it elsewhere at the same time; it must outlive the setting); local_to_global[i] = the global leaf id
+ * of local leaf i (every leaf of the bound state, owned and ghost). mg = NULL switches back to red-black (other arguments ignored);
+ * so does a refused call (bad cycles / nu / omega, ids out of range or not matching the hierarchy's level-0 leaves).
+ * Setup, collective: every rank calls _set_pressure_solver (64 opaque bytes out: the IPC handle of its level-1 block; may be NULL with
+ * one rank), the caller all-gathers them, calls _mg_connect with the handle of every OTHER rank, then _mg_finish; the solver takes
+ * effect at _mg_finish. HNS_ERR_UNSUPPORTED with more than one rank and no peer-memory exchange (the NCCL fallback). A gather that
+ * waits for a rank longer than ~4 s sets the error word (hns_dist_error: low byte 11). */
+int hns_dist_set_pressure_solver(hns_dist* d, hns_state* s, hns_mg* mg, const int32_t* local_to_global, int cycles, int nu_pre, int nu_post,
+                                 float omega_smooth, uint8_t* handle_out64);
+int hns_dist_mg_connect(hns_dist* d, int rank, const uint8_t* handle64);
+int hns_dist_mg_finish(hns_dist* d);
+/* V-cycles that gathered a level-1 right-hand side, and the bytes this rank stored into the other ranks' copies, since hns_dist_create */
+uint64_t hns_dist_mg_gathers(const hns_dist* d);
+uint64_t hns_dist_mg_gather_bytes(const hns_dist* d);
 
 #ifdef __cplusplus
 }
