@@ -30,7 +30,6 @@ SIGNATURES = {
     "hns_launch_count": (C.c_uint64, []),
     "hns_launch_count_reset": (None, []),
     "hns_set_device": (C.c_int, [C.c_int]),
-    "hns_set_l2_persist_mb": (C.c_int, [C.c_int]),
     "hns_set_packed_advection": (C.c_int, [C.c_int]),
     "hns_packed_advection_launches": (C.c_uint64, []),
     "hns_nvdb_write": (C.c_int, [C.c_char_p, C.c_void_p, C.c_uint64]),
@@ -95,8 +94,6 @@ SIGNATURES = {
     "hns_state_advect_scalars": (C.c_int, [C.c_void_p, C.c_float, C.c_int, C.c_void_p]),
     "hns_state_sync": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hns_state_time_frames": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_uint, C.c_void_p, c_f32p, c_f32p]),
-    "hns_state_gather_element0": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
-    "hns_state_set_element0": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hns_state_pack_leaves": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "hns_state_unpack_leaves": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "hns_state_field_device_ptr": (C.c_void_p, [C.c_void_p, C.c_int]),
@@ -115,8 +112,6 @@ SIGNATURES = {
     "hns_dist_frame": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p]),
     "hns_dist_cook": (C.c_int, [C.c_void_p, C.c_void_p, c_f32p, C.c_int, C.POINTER(c_f32p), C.c_int, C.c_float, C.c_void_p]),
     "hns_dist_frame_timed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p, c_f32p]),
-    "hns_dist_debug_step": (C.c_int, [C.c_void_p, c_f32p]),
-    "hns_dist_time_sweeps": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, c_f32p]),
     "hns_dist_allreduce_sum": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.c_int, C.c_void_p]),
     "hns_state_residual_sums": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.c_void_p]),
     "hns_state_divergence_sum_squares": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_double), C.c_void_p]),

@@ -361,8 +361,7 @@ __device__ __forceinline__ void scalar_fields(const float* __restrict__ base, co
 template <int kSem, bool kCollision>
 __global__ void __launch_bounds__(512, 2) k_advect_scalars2(GridView g, const float* __restrict__ u, const float* __restrict__ v,
                                                             const float* __restrict__ w, const __grid_constant__ ScalarPtrs sp, int S, float sdt,
-                                                            const float* __restrict__ elem0, const float* __restrict__ sdf,
-                                                            uint8_t* __restrict__ cold) {
+                                                            const float* __restrict__ sdf, uint8_t* __restrict__ cold) {
 	extern __shared__ __align__(16) float region[];
 	__shared__ int meta[3][kMeta];
 	__shared__ float fill[3 + 16];
@@ -372,10 +371,10 @@ __global__ void __launch_bounds__(512, 2) k_advect_scalars2(GridView g, const fl
 	const int x = tid >> 6, y = (tid >> 3) & 7, z = tid & 7;
 	const Own own = make_own(x, y, z);
 	const Stager stg = make_stager();
-	// what inactive cells hold: advect_scalars reads array element 0 (of the GLOBAL arrays: elem0 when given), advect_scalar reads 0
+	// what inactive cells hold: advect_scalars reads array element 0, advect_scalar reads 0
 	if (tid < 3 + S) {
 		float f = 0.f;
-		if (kSem == 0) f = elem0 ? __ldg(elem0 + tid) : (tid == 0 ? __ldg(u) : tid == 1 ? __ldg(v) : tid == 2 ? __ldg(w) : __ldg(sp.in[tid - 3]));
+		if (kSem == 0) f = tid == 0 ? __ldg(u) : tid == 1 ? __ldg(v) : tid == 2 ? __ldg(w) : __ldg(sp.in[tid - 3]);
 		fill[tid] = f;
 	}
 	const int jobs_per_leaf = 1 + (S - 1 + 3) / 4;
@@ -482,7 +481,7 @@ __global__ void __launch_bounds__(512, 2) k_advect_scalars2(GridView g, const fl
 template <int kSem, bool kCollision>
 __global__ void __launch_bounds__(512) k_advect_scalars_cold(GridView g, const float* __restrict__ u, const float* __restrict__ v,
                                                              const float* __restrict__ w, const __grid_constant__ ScalarPtrs sp, int S, float sdt,
-                                                             const float* __restrict__ elem0, const float* __restrict__ sdf, uint8_t* cold) {
+                                                             const float* __restrict__ sdf, uint8_t* cold) {
 	const int tid = threadIdx.x;
 	const int x = tid >> 6, y = (tid >> 3) & 7, z = tid & 7;
 	__shared__ uint32_t todo[512], n_todo;
@@ -494,16 +493,15 @@ __global__ void __launch_bounds__(512) k_advect_scalars_cold(GridView g, const f
 		const LeafFrame f{o.x, o.y, o.z, g.nbr + uint64_t(leaf) * 27u};
 		const uint64_t self = uint64_t(leaf) * 512u + uint32_t(tid);
 		const int ci = o.x + x, cj = o.y + y, ck = o.z + z;
-		const float *eu = elem0 ? elem0 : u, *ev = elem0 ? elem0 + 1 : v, *ew = elem0 ? elem0 + 2 : w;
 		float bx = fmaf(-sdt, __ldg(u + self), float(ci)), by = fmaf(-sdt, __ldg(v + self), float(cj)), bz = fmaf(-sdt, __ldg(w + self), float(ck));
 		if (kCollision && trilinear_f(g, f, sdf, bx, by, bz) < 0.0f) bx = float(ci), by = float(cj), bz = float(ck);
 		const int bi = __float2int_rd(bx), bj = __float2int_rd(by), bk = __float2int_rd(bz);
 		const float btx = bx - float(bi), bty = by - float(bj), btz = bz - float(bk);
 		float uf, vf, wf;
 		if (kSem == 0) {
-			uf = far_weighted(g, f, u, eu, bi, bj, bk, btx, bty, btz);
-			vf = far_weighted(g, f, v, ev, bi, bj, bk, btx, bty, btz);
-			wf = far_weighted(g, f, w, ew, bi, bj, bk, btx, bty, btz);
+			uf = far_weighted(g, f, u, bi, bj, bk, btx, bty, btz);
+			vf = far_weighted(g, f, v, bi, bj, bk, btx, bty, btz);
+			wf = far_weighted(g, f, w, bi, bj, bk, btx, bty, btz);
 		} else {
 			trilinear_vec(g, f, u, v, w, bx, by, bz, uf, vf, wf);
 		}
@@ -520,12 +518,11 @@ __global__ void __launch_bounds__(512) k_advect_scalars_cold(GridView g, const f
 #pragma unroll 1
 		for (int k = 0; k < S; ++k) {
 			const float* __restrict__ a = sp.in[k];
-			const float* e0 = elem0 ? elem0 + 3 + k : a;
 			const float phi0 = __ldg(a + self);
 			float phiF, phiB;
 			if (kSem == 0) {
-				phiF = far_weighted(g, f, a, e0, bi, bj, bk, btx, bty, btz);
-				phiB = far_weighted(g, f, a, e0, fi, fj, fk, ftx, fty, ftz);
+				phiF = far_weighted(g, f, a, bi, bj, bk, btx, bty, btz);
+				phiB = far_weighted(g, f, a, fi, fj, fk, ftx, fty, ftz);
 			} else {
 				phiF = trilinear_f(g, f, a, bx, by, bz);
 				phiB = trilinear_f(g, f, a, fx, fy, fz);
@@ -534,7 +531,7 @@ __global__ void __launch_bounds__(512) k_advect_scalars_cold(GridView g, const f
 			float mn = phi0, mx = phi0;
 #pragma unroll
 			for (int q = 0; q < 6; ++q) {
-				const float val = nb[q] < 0 ? (kSem == 0 ? __ldg(e0) : 0.f) : __ldg(a + nb[q]);
+				const float val = nb[q] < 0 ? (kSem == 0 ? __ldg(a) : 0.f) : __ldg(a + nb[q]);
 				mn = fminf(mn, val), mx = fmaxf(mx, val);
 			}
 			sp.out[k][self] = fmaxf(fminf(mn, phiF), fminf(corr, fmaxf(mx, phiF)));
@@ -764,8 +761,7 @@ struct Trace4 {
 };
 template <int kSem, bool kCollision>
 __global__ void __launch_bounds__(512, 2) k_advect_scalars4(GridView g, const __grid_constant__ GroupPtrs gp, const __grid_constant__ ScalarPtrs sp, int S,
-                                                            float sdt, const float* __restrict__ elem0, const float* __restrict__ sdf,
-                                                            uint8_t* __restrict__ cold) {
+                                                            float sdt, const float* __restrict__ sdf, uint8_t* __restrict__ cold) {
 	extern __shared__ __align__(128) float4 region4[];
 	int(*meta)[kMeta] = reinterpret_cast<int(*)[kMeta]>(region4 + 2 * kCells);
 	float4* fill = reinterpret_cast<float4*>(meta + 3);
@@ -776,10 +772,10 @@ __global__ void __launch_bounds__(512, 2) k_advect_scalars4(GridView g, const __
 	const int oc = (x + kHaloXY) * kCX + (y + kHaloXY) * kCY + (z + kHaloZ);
 	const Stager4 stg = make_stager4();
 	const int jobs_per_leaf = 1 + (S - 1 + 3) / 4;
-	// what inactive cells hold: advect_scalars reads array element 0 (of the GLOBAL arrays: elem0 when given), advect_scalar reads 0
+	// what inactive cells hold: advect_scalars reads array element 0, advect_scalar reads 0
 	if (tid < 4 * jobs_per_leaf) {
 		float f = 0.f;
-		if (kSem == 0 && tid < 3 + S) f = elem0 ? __ldg(elem0 + tid) : __ldg(reinterpret_cast<const float*>(gp.g[tid >> 2]) + (tid & 3));
+		if (kSem == 0 && tid < 3 + S) f = __ldg(reinterpret_cast<const float*>(gp.g[tid >> 2]) + (tid & 3));
 		reinterpret_cast<float*>(fill)[tid] = f;
 	}
 	const uint32_t n_jobs = items.count * uint32_t(jobs_per_leaf);
@@ -992,7 +988,7 @@ void launch_advect_vector(const GridView& g, const float* const vel[3], float* c
 }
 
 void launch_advect_scalars(const GridView& g, const float* const vel[3], const ScalarPtrs& sp, int S, float dt, float inv_dx, int sampler_semantics,
-                           const float* elem0, cudaStream_t st, const float* sdf, uint8_t* cold, const AdvectGroups* grp) {
+                           cudaStream_t st, const float* sdf, uint8_t* cold, const AdvectGroups* grp) {
 	if (!g.count() || S <= 0) return;
 	DeviceInfo& d = device_info();
 	ensure_attrs(d);
@@ -1012,16 +1008,16 @@ void launch_advect_scalars(const GridView& g, const float* const vel[3], const S
 		                                   : (sdf ? k_advect_scalars4<1, true> : k_advect_scalars4<1, false>);
 		auto cold4 = sampler_semantics == 0 ? (sdf ? k_advect_scalars_cold<0, true> : k_advect_scalars_cold<0, false>)
 		                                    : (sdf ? k_advect_scalars_cold<1, true> : k_advect_scalars_cold<1, false>);
-		HNS_LAUNCH(hot4, grid, 512, kAdvect4Smem, st, g, gp, sp, S, sdt, elem0, sdf, cold);
-		HNS_LAUNCH(cold4, cold_grid, 512, 0, st, g, vel[0], vel[1], vel[2], sp, S, sdt, elem0, sdf, cold);
+		HNS_LAUNCH(hot4, grid, 512, kAdvect4Smem, st, g, gp, sp, S, sdt, sdf, cold);
+		HNS_LAUNCH(cold4, cold_grid, 512, 0, st, g, vel[0], vel[1], vel[2], sp, S, sdt, sdf, cold);
 		return;
 	}
 	auto hot = sampler_semantics == 0 ? (sdf ? k_advect_scalars2<0, true> : k_advect_scalars2<0, false>)
 	                                  : (sdf ? k_advect_scalars2<1, true> : k_advect_scalars2<1, false>);
 	auto cold_k = sampler_semantics == 0 ? (sdf ? k_advect_scalars_cold<0, true> : k_advect_scalars_cold<0, false>)
 	                                     : (sdf ? k_advect_scalars_cold<1, true> : k_advect_scalars_cold<1, false>);
-	HNS_LAUNCH(hot, grid, 512, kAdvectSmem, st, g, vel[0], vel[1], vel[2], sp, S, sdt, elem0, sdf, cold);
-	HNS_LAUNCH(cold_k, cold_grid, 512, 0, st, g, vel[0], vel[1], vel[2], sp, S, sdt, elem0, sdf, cold);
+	HNS_LAUNCH(hot, grid, 512, kAdvectSmem, st, g, vel[0], vel[1], vel[2], sp, S, sdt, sdf, cold);
+	HNS_LAUNCH(cold_k, cold_grid, 512, 0, st, g, vel[0], vel[1], vel[2], sp, S, sdt, sdf, cold);
 }
 
 }  // namespace hns

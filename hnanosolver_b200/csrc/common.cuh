@@ -69,68 +69,6 @@ struct GridView {
 #endif
 };
 
-// ---- L2 residency of the pressure field during the solve ----------------------------------------------------------------------
-// The two pressure halves (one allocation) are read by every one of the 2 x iterations half-sweeps; everything else a sweep touches
-// streams. An access-policy window marks a fraction of the pressure lines "persisting" in the L2 set-aside for the launches
-// enqueued while it is set, so those lines are served from L2 in every sweep instead of from HBM. Scoped: the previous window of
-// the caller's stream is put back when the object dies (attributes are captured per launch at enqueue time).
-// MEASURED ON B200 AND SWITCHED OFF BY DEFAULT: on the 512^3 workload (161 MB of pressure) the 40-iteration solve takes 4.59 ms
-// without a window, 4.77 / 4.80 / 6.50 / 7.54 ms with 32 / 48 / 64 / 80 MB set aside, and a large set-aside also slows the
-// streaming kernels around it (the normal L2 shrinks). The knob stays for experiments (DESIGN.md 4).
-struct L2PressureWindow {
-	cudaStream_t st = nullptr;
-	bool active = false;
-	cudaStreamAttrValue saved{};
-	static long long& requested_mb() {  // HNS_L2_PERSIST_MB (default 0 = off, see below); hns_set_l2_persist_mb() overrides it
-		static long long mb = [] {
-			const char* e = std::getenv("HNS_L2_PERSIST_MB");
-			return e ? std::atoll(e) : 0ll;
-		}();
-		return mb;
-	}
-	static long long& applied() {
-		static long long bytes = -1;  // -1: device limit not set yet
-		return bytes;
-	}
-	static size_t persist_bytes() {  // set-aside size, clamped to the device limit
-		long long& cached = applied();
-		if (cached < 0) {
-			int dev = 0, max_persist = 0;
-			cudaGetDevice(&dev);
-			cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev);
-			cached = std::max(0ll, std::min<long long>(requested_mb() << 20, max_persist));
-			if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, size_t(cached)) != cudaSuccess) cached = 0;
-			cudaGetLastError();
-		}
-		return size_t(cached);
-	}
-	L2PressureWindow(cudaStream_t stream, const void* base, size_t bytes) : st(stream) {
-		const size_t persist = persist_bytes();
-		if (!persist || !bytes || bytes <= persist / 2) return;  // small fields live in the L2 anyway
-		int dev = 0, max_window = 0;
-		cudaGetDevice(&dev);
-		cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-		if (max_window <= 0) return;
-		if (cudaStreamGetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &saved) != cudaSuccess) {
-			cudaGetLastError();
-			return;
-		}
-		cudaStreamAttrValue v{};
-		v.accessPolicyWindow.base_ptr = const_cast<void*>(base);
-		v.accessPolicyWindow.num_bytes = std::min(bytes, size_t(max_window));
-		v.accessPolicyWindow.hitRatio = float(std::min(1.0, double(persist) / double(v.accessPolicyWindow.num_bytes)));
-		v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-		v.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
-		if (cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &v) == cudaSuccess) active = true;
-		else cudaGetLastError();
-	}
-	~L2PressureWindow() {
-		if (active) cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &saved);
-	}
-	L2PressureWindow(const L2PressureWindow&) = delete;
-	L2PressureWindow& operator=(const L2PressureWindow&) = delete;
-};
-
 // packed field groups of the advection kernels (kernels.cuh, advect.cu)
 struct AdvectGroups {
 	float4* g[5] = {};
@@ -263,7 +201,6 @@ struct hns_state {
 	int skip_scalar = -1;  // scalar that is carried but not advected ("collision_sdf")
 	bool collision = false;  // hasCollision with collision data: scalar `skip_scalar` is the SDF the kernels collide against
 	const float* collision_sdf() const { return collision && skip_scalar >= 0 ? sc[skip_scalar] : nullptr; }
-	const float* elem0 = nullptr;  // device float[3 + n_scalars]: element 0 of the global arrays (sharded runs), else null
 	uint64_t vel_version = 1;  // bumped by every entry point that (may) overwrite the velocity planes; lets a sharded run skip a ghost exchange of unchanged data
 	const int32_t* active = nullptr;  // device list of the leaves the kernels process (sharded runs: the owned leaves), null = all
 	uint32_t n_active = 0;

@@ -10,7 +10,6 @@
 // NCCL instance torch has already loaded in the same process.
 #include <dlfcn.h>
 
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -34,7 +33,6 @@ struct Nccl {
 	int (*CommDestroy)(ncclComm_t) = nullptr;
 	int (*Send)(const void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
 	int (*Recv)(void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
-	int (*Broadcast)(const void*, void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
 	int (*AllReduce)(const void*, void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
 	int (*GroupStart)() = nullptr;
 	int (*GroupEnd)() = nullptr;
@@ -54,7 +52,6 @@ static int load_nccl() {
 	HNS_SYM(CommDestroy, "ncclCommDestroy")
 	HNS_SYM(Send, "ncclSend")
 	HNS_SYM(Recv, "ncclRecv")
-	HNS_SYM(Broadcast, "ncclBroadcast")
 	HNS_SYM(AllReduce, "ncclAllReduce")
 	HNS_SYM(GroupStart, "ncclGroupStart")
 	HNS_SYM(GroupEnd, "ncclGroupEnd")
@@ -91,7 +88,6 @@ struct hns_dist {
 	};
 	std::vector<Peer> peers;
 	int max_fields = 0;
-	float* d_elem0 = nullptr;
 	double* d_reduce = nullptr;  // staging of hns_dist_allreduce_sum
 	uint64_t bytes_sent = 0, exchanges = 0;
 	// work lists (local leaf ids, device): owned = boundary (sent to some peer) + interior
@@ -114,26 +110,16 @@ struct hns_dist {
 	uint32_t seq[16] = {};  // per flag channel (kCh* below)
 	uint32_t* d_err = nullptr;
 	int n_scalars = 0;
-	// timed mode: events inside one pressure half-sweep (k = 20): bs: before B, after B, after push, after signal+wait, after unpack; st: before I, after I
-	cudaEvent_t dbg[7] = {};
-	bool dbg_valid = false;
 	// fused boundary sweep + push: CSR over the boundary work list -> (peer index, leaf id on that peer)
 	uint32_t* d_push_off = nullptr;
 	int32_t *d_push_peer = nullptr, *d_push_leaf = nullptr;
 	float** d_remote_p[2] = {nullptr, nullptr};  // [n_peers] per colour
-	uint32_t* d_counter = nullptr;
-	uint32_t seq_p[2] = {0, 0}, frame_id = 0;
 	std::vector<int32_t> h_boundary;             // host copy of the boundary work list
 	const hns_state* bound_state = nullptr;
-	int aux_blocks = 148;           // HNS_AUX_BLOCKS: CTA cap of the background scalar exchange (it must not starve the sweeps)
-	bool push_whole_leaves = false; // HNS_PUSH_WHOLE_LEAVES=1: push every row of every ghost copy (A/B switch)
 	uint64_t push_bytes_per_sweep = 0;
-	bool fused_push = true;         // HNS_FUSED_PUSH=0: pack / push / signal / wait / unpack kernels instead (A/B switch)
-	bool signal_in_kernel = false;  // HNS_SIGNAL_IN_KERNEL=1: the boundary sweep raises the arrival flags itself (A/B switch)
-	uint32_t* d_seq_base = nullptr;  // device [3]: sequence bases of the red pushes, black pushes, frames -- mirror seq_p[0], seq_p[1], frame_id
+	uint32_t* d_seq_base = nullptr;  // device [3]: sequence bases of the red pushes, black pushes, frames
 	cudaStream_t copy_stream = nullptr;  // hns_dist_cook: host <-> device transfers overlapping the frame
 	cudaEvent_t ev_copy[6] = {};
-	bool cook_overlap = true;       // HNS_COOK_OVERLAP=0: transfers and frame one after the other on the caller's stream (A/B switch)
 	// Sharded multigrid pressure solve (hns_dist_set_pressure_solver): level 0 is this rank's shard, levels >= 1 of `mg` (a hierarchy
 	// over the GLOBAL grid) are replicated -- every rank runs the coarse part of every cycle itself on the gathered level-1 rhs.
 	struct ShardedMg {
@@ -155,6 +141,9 @@ struct hns_dist {
 		int graph_coarsest[2] = {0, 0};
 	} smg;
 };
+
+// CTA cap of the background scalar exchange: it must not starve the pressure sweeps it runs beside
+constexpr int kAuxBlocks = 148;
 
 // flag channels: 0..7 of the ghost exchanges (see dist_frame), 8 / 9 the red / black pressure exchanges of the sharded multigrid solve
 // (landing in the regions of channels 2 / 3), 10 the level-1 gather. k_wait reports a time-out as 1 + channel in the error word.
@@ -278,14 +267,13 @@ void hns_dist_destroy(hns_dist* d) {
 	mg_release(d);
 	for (auto& p : d->peers) cudaFree(p.d_send), cudaFree(p.d_recv), cudaFree(p.buf_send), cudaFree(p.buf_recv);
 	cudaFree(d->d_reduce);
-	cudaFree(d->d_elem0), cudaFree(d->d_owned), cudaFree(d->d_boundary), cudaFree(d->d_interior);
+	cudaFree(d->d_owned), cudaFree(d->d_boundary), cudaFree(d->d_interior);
 	cudaFree(d->d_boundary_nbr), cudaFree(d->d_interior_nbr);
 	for (auto& p : d->peers) {
 		if (p.ipc_base) cudaIpcCloseMemHandle(p.ipc_base);
 		if (p.ipc_pbase) cudaIpcCloseMemHandle(p.ipc_pbase);
 	}
-	cudaFree(d->d_push_off), cudaFree(d->d_push_peer), cudaFree(d->d_push_leaf), cudaFree(d->d_remote_p[0]), cudaFree(d->d_remote_p[1]),
-	    cudaFree(d->d_counter);
+	cudaFree(d->d_push_off), cudaFree(d->d_push_peer), cudaFree(d->d_push_leaf), cudaFree(d->d_remote_p[0]), cudaFree(d->d_remote_p[1]);
 	cudaFree(d->block), cudaFree(d->d_remote_flags), cudaFree(d->d_local_flags), cudaFree(d->d_err);
 	for (auto& e : d->ev_I)
 		if (e) cudaEventDestroy(e);
@@ -329,14 +317,11 @@ int hns_dist_set_plan(hns_dist* d, hns_state* s, int n_peers, const int* peer_ra
 		HNS_CUDA(up(inter, &d->d_interior));
 		cudaFree(d->d_boundary_nbr), cudaFree(d->d_interior_nbr);
 		d->d_boundary_nbr = d->d_interior_nbr = nullptr;
-		const char* e = std::getenv("HNS_LIST_NBR");  // A/B switch, default on
-		if (!e || std::atoi(e) != 0) {
-			HNS_CUDA(cudaMalloc(&d->d_boundary_nbr, std::max<size_t>(bnd.size(), 1) * 27 * sizeof(int32_t)));
-			HNS_CUDA(cudaMalloc(&d->d_interior_nbr, std::max<size_t>(inter.size(), 1) * 27 * sizeof(int32_t)));
-			launch_gather_nbr_rows(s->grid->view.nbr, d->d_boundary, d->n_boundary, d->d_boundary_nbr, nullptr);
-			launch_gather_nbr_rows(s->grid->view.nbr, d->d_interior, d->n_interior, d->d_interior_nbr, nullptr);
-			HNS_CUDA(cudaDeviceSynchronize());
-		}
+		HNS_CUDA(cudaMalloc(&d->d_boundary_nbr, std::max<size_t>(bnd.size(), 1) * 27 * sizeof(int32_t)));
+		HNS_CUDA(cudaMalloc(&d->d_interior_nbr, std::max<size_t>(inter.size(), 1) * 27 * sizeof(int32_t)));
+		launch_gather_nbr_rows(s->grid->view.nbr, d->d_boundary, d->n_boundary, d->d_boundary_nbr, nullptr);
+		launch_gather_nbr_rows(s->grid->view.nbr, d->d_interior, d->n_interior, d->d_interior_nbr, nullptr);
+		HNS_CUDA(cudaDeviceSynchronize());
 		s->active = d->d_owned, s->n_active = d->n_owned;
 		if (!d->comm_stream) {
 			int prio_lo = 0, prio_hi = 0;  // the exchange kernels are tiny and latency-critical: let their CTAs overtake the queued interior sweep
@@ -369,8 +354,7 @@ int hns_dist_set_plan(hns_dist* d, hns_state* s, int n_peers, const int* peer_ra
 		d->peers.push_back(p);
 	}
 	// advect_scalars' "inactive -> element 0": the plan keeps global leaf 0 on every rank as LOCAL leaf 0 (a ghost fed by rank 0 in the
-	// exchange before advect_scalars), so element 0 of the local arrays is the global one: no override
-	s->elem0 = nullptr;
+	// exchange before advect_scalars), so element 0 of the local arrays is the global one
 	if (!d->d_err) {
 		HNS_CUDA(cudaMalloc(&d->d_err, sizeof(uint32_t)));
 		HNS_CUDA(cudaMemset(d->d_err, 0, sizeof(uint32_t)));
@@ -379,15 +363,10 @@ int hns_dist_set_plan(hns_dist* d, hns_state* s, int n_peers, const int* peer_ra
 	d->n_scalars = s->n_scalars;
 	d->bound_state = s;
 	d->vel_exchanged_version = ~uint64_t(0);
-	if (const char* e = std::getenv("HNS_SIGNAL_IN_KERNEL")) d->signal_in_kernel = std::atoi(e) != 0;
-	if (const char* e = std::getenv("HNS_FUSED_PUSH")) d->fused_push = std::atoi(e) != 0;
-	if (const char* e = std::getenv("HNS_COOK_OVERLAP")) d->cook_overlap = std::atoi(e) != 0;
 	if (!d->d_seq_base) {
 		HNS_CUDA(cudaMalloc(&d->d_seq_base, 3 * sizeof(uint32_t)));
 		HNS_CUDA(cudaMemset(d->d_seq_base, 0, 3 * sizeof(uint32_t)));
 	}
-	if (const char* e = std::getenv("HNS_AUX_BLOCKS")) d->aux_blocks = std::atoi(e);
-	if (const char* e = std::getenv("HNS_PUSH_WHOLE_LEAVES")) d->push_whole_leaves = std::atoi(e) != 0;
 	return HNS_OK;
 }
 
@@ -488,7 +467,6 @@ int hns_dist_ipc_finish(hns_dist* d) {
 					const int32_t nb = nbr[uint64_t(leaf) * 27 + face_slot[f]];
 					if (nb >= 0 && owner[nb] == int32_t(i)) mask |= 1 << f;
 				}
-				if (d->push_whole_leaves) mask = 0x30;
 				if (!mask) continue;
 				per_leaf[leaf].push_back({int32_t(i) | (mask << 8), p.peer_leaf[k]});
 				int rows = 64;
@@ -523,10 +501,6 @@ int hns_dist_ipc_finish(hns_dist* d) {
 			HNS_CUDA(cudaMalloc(&d->d_remote_p[c], rp.size() * sizeof(float*)));
 			HNS_CUDA(cudaMemcpy(d->d_remote_p[c], rp.data(), rp.size() * sizeof(float*), cudaMemcpyHostToDevice));
 		}
-		if (!d->d_counter) {
-			HNS_CUDA(cudaMalloc(&d->d_counter, sizeof(uint32_t)));
-			HNS_CUDA(cudaMemset(d->d_counter, 0, sizeof(uint32_t)));
-		}
 	}
 	d->p2p = true;
 	return HNS_OK;
@@ -560,8 +534,8 @@ static int check_device_error(hns_dist* d) {
 // scattered into the ghost leaves. Four small launches, no library call, NVLink bandwidth instead of NCCL's p2p channel bandwidth.
 // `channel` selects the arrival flag; the bricks land in region `region_ch` starting `skip_fields` whole fields in, so two exchanges
 // with different flags can share one region (velocity and scalars of channel 4).
-static int exchange_p2p(hns_dist* d, hns_state* s, int channel, int n_fields, const int* fields, cudaStream_t st, cudaEvent_t* dbg = nullptr,
-                        int region_ch = -1, int skip_fields = 0, int max_blocks = 0) {
+static int exchange_p2p(hns_dist* d, hns_state* s, int channel, int n_fields, const int* fields, cudaStream_t st, int region_ch = -1,
+                        int skip_fields = 0, int max_blocks = 0) {
 	const int S = d->n_scalars;
 	if (region_ch < 0) region_ch = channel;
 	for (auto& p : d->peers) {
@@ -578,10 +552,8 @@ static int exchange_p2p(hns_dist* d, hns_state* s, int channel, int n_fields, co
 	}
 	const uint32_t seq = ++d->seq[channel];
 	const int np = int(d->peers.size());
-	if (dbg) cudaEventRecord(dbg[2], st);
 	HNS_LAUNCH(k_signal, 1, 32, 0, st, d->d_remote_flags, np, channel, seq);
 	HNS_LAUNCH(k_wait, 1, 32, 0, st, d->d_local_flags, np, channel, seq, d->d_err);
-	if (dbg) cudaEventRecord(dbg[3], st);
 	for (auto& p : d->peers) {
 		if (!p.n_recv) continue;
 		const float* src = reinterpret_cast<const float*>(d->block + p.region_off + channel_offset(region_ch, p.n_recv, S)) + uint64_t(skip_fields) * 512u * p.n_recv;
@@ -592,13 +564,12 @@ static int exchange_p2p(hns_dist* d, hns_state* s, int channel, int n_fields, co
 			src += p.n_recv * fpl;
 		}
 	}
-	if (dbg) cudaEventRecord(dbg[4], st);
 	++d->exchanges;
 	HNS_CUDA(cudaGetLastError());
 	return HNS_OK;
 }
-static int exchange_channel(hns_dist* d, hns_state* s, int channel, int n_fields, const int* fields, cudaStream_t st, cudaEvent_t* dbg = nullptr) {
-	return d->p2p ? exchange_p2p(d, s, channel, n_fields, fields, st, dbg) : hns_dist_exchange(d, s, n_fields, fields, st);
+static int exchange_channel(hns_dist* d, hns_state* s, int channel, int n_fields, const int* fields, cudaStream_t st) {
+	return d->p2p ? exchange_p2p(d, s, channel, n_fields, fields, st) : hns_dist_exchange(d, s, n_fields, fields, st);
 }
 
 // pack -> grouped send/recv -> unpack of the given fields' ghost bricks, all on `stream`
@@ -671,8 +642,8 @@ int hns_dist_cook(hns_dist* d, hns_state* s, float* velocity, int n_float, float
 	// Like hns_compute_sim (api.cu): the shard crosses PCIe on a copy stream while the kernels run. Velocity (and the collision SDF) first
 	// -- advect_vector and the divergence start as soon as they have landed --, the four combustion inputs next, the remaining scalars
 	// behind them (they are needed by the scalars' ghost exchange behind the pressure solve); the projected velocity goes back while
-	// advect_scalars runs, the scalars when it is done. HNS_COOK_OVERLAP=0: everything on the caller's stream, one after the other.
-	cudaStream_t cs = d->cook_overlap ? d->copy_stream : st;
+	// advect_scalars runs, the scalars when it is done.
+	cudaStream_t cs = d->copy_stream;
 	cudaEvent_t e_start = d->ev_copy[0], e_vel_in = d->ev_copy[1], e_comb_in = d->ev_copy[2], e_all_in = d->ev_copy[3], e_vel_out = d->ev_copy[4],
 	            e_done = d->ev_copy[5];
 	HNS_CUDA(cudaEventRecord(e_start, st));
@@ -707,7 +678,7 @@ int hns_dist_cook(hns_dist* d, hns_state* s, float* velocity, int n_float, float
 }
 
 // Same frame with CUDA events between the phases; ms_out[8] = exchange velocity, advect_vector, exchange advected, divergence(+combustion),
-// pressure solve incl. its exchanges, gradient, final exchange (+element-0 broadcast), advect_scalars. Synchronises the stream.
+// pressure solve incl. its exchanges, gradient, final exchange, advect_scalars. Synchronises the stream.
 int hns_dist_frame_timed(hns_dist* d, hns_state* s, int iterations, float dt, void* stream, float* ms_out) {
 	if (!ms_out) return fail(HNS_ERR_INVALID_ARGUMENT, "null argument");
 	cudaEvent_t ev[9];
@@ -721,14 +692,18 @@ int hns_dist_frame_timed(hns_dist* d, hns_state* s, int iterations, float dt, vo
 }
 
 // The pressure solve of the peer-memory mode: interior sweeps on `st`, boundary sweeps (which store every swept quad into the peers'
-// ghost copies) + flag signal / wait on `bs`; with `dbg_mode` the events of half-sweep 20 are recorded (timed frames).
-static int record_fused_pressure(hns_dist* d, hns_state* s, int iterations, float omega, cudaStream_t st, cudaStream_t bs, bool dbg_mode) {
+// ghost copies) + flag signal / wait on the comm stream.
+// (Replaying this pipeline as a CUDA graph -- two captured streams, which is why the sequence numbers live in device memory -- was
+// measured at 2 GPUs: 8.75 ms per frame against 8.54 ms launched directly; the graph's two branches do not overlap the way the
+// high-priority comm stream does. Removed; profiles/r2d_tune2_dist_graph.txt.)
+static int fused_pressure(hns_dist* d, hns_state* s, int iterations, float omega, cudaStream_t st) {
 	GridView vb = s->grid->view, vi = s->grid->view;
 	vb.list = d->d_boundary, vb.num_list = d->n_boundary, vb.list_nbr = d->d_boundary_nbr;
 	vi.list = d->d_interior, vi.num_list = d->n_interior, vi.list_nbr = d->d_interior_nbr;
 	const float dx = s->grid->voxel_size;
 	const int np = int(d->peers.size());
 	const uint32_t* base = d->d_seq_base;
+	cudaStream_t bs = d->comm_stream;
 	// "my pressure arrays are zeroed and nobody reads last frame's ghosts any more": peers may start pushing into them
 	HNS_LAUNCH(k_signal_rel, 1, 32, 0, st, d->d_remote_flags, np, 5, base + 2, 1u);
 	HNS_CUDA(cudaEventRecord(d->ev_I[1], st));  // "I_0": everything before the solve
@@ -736,47 +711,24 @@ static int record_fused_pressure(hns_dist* d, hns_state* s, int iterations, floa
 	for (int it = 0; it < iterations; ++it)
 		for (int color = 0; color < 2; ++color, ++k) {
 			const int cur = k & 1, prev = cur ^ 1;
-			cudaEvent_t* dbg = nullptr;
-			if (dbg_mode && k == 20) {
-				if (!d->dbg[0])
-					for (auto& e : d->dbg) cudaEventCreate(&e);
-				dbg = d->dbg, d->dbg_valid = true;
-			}
 			HNS_CUDA(cudaStreamWaitEvent(bs, d->ev_I[prev], 0));
-			if (dbg) cudaEventRecord(dbg[0], bs);
 			// ghosts of the colour this sweep reads: pushed by the peers' previous boundary sweep (first sweep: their "zeroed" signal).
 			// Red sweep of iteration `it` reads black pushes up to number `it`; black reads red pushes up to `it + 1`.
 			if (k == 0) HNS_LAUNCH(k_wait_rel, 1, 32, 0, bs, d->d_local_flags, np, 5, base + 2, 1u, d->d_err);
 			else HNS_LAUNCH(k_wait_rel, 1, 32, 0, bs, d->d_local_flags, np, 2 + (color ^ 1), base + (color ^ 1), uint32_t(it + color), d->d_err);
-			if (dbg) cudaEventRecord(dbg[2], bs);
 			RbgsPush push;
-			push.dst_off = d->d_push_off, push.dst_peer = d->d_push_peer, push.dst_leaf = d->d_push_leaf;
-			push.remote_pc = d->d_remote_p[color], push.signal_flags = d->d_remote_flags, push.n_peers = np;
-			push.signal_ch = 2 + color, push.signal_seq = d->seq_p[color] + uint32_t(it) + 1u, push.counter = d->signal_in_kernel ? d->d_counter : nullptr;
+			push.dst_off = d->d_push_off, push.dst_peer = d->d_push_peer, push.dst_leaf = d->d_push_leaf, push.remote_pc = d->d_remote_p[color];
 			launch_rbgs_color_push(vb, s->div, s->p, dx, color, omega, color, push, bs);
-			if (!d->signal_in_kernel) HNS_LAUNCH(k_signal_rel, 1, 32, 0, bs, d->d_remote_flags, np, 2 + color, base + color, uint32_t(it) + 1u);
+			HNS_LAUNCH(k_signal_rel, 1, 32, 0, bs, d->d_remote_flags, np, 2 + color, base + color, uint32_t(it) + 1u);
 			HNS_CUDA(cudaEventRecord(d->ev_B[cur], bs));
-			if (dbg) cudaEventRecord(dbg[1], bs), cudaEventRecord(dbg[3], bs), cudaEventRecord(dbg[4], bs);
 			if (k > 0) HNS_CUDA(cudaStreamWaitEvent(st, d->ev_B[prev], 0));
-			if (dbg) cudaEventRecord(dbg[5], st);
 			if (d->n_interior) launch_rbgs_color(vi, s->div, s->p, dx, color, omega, color, st);
 			HNS_CUDA(cudaEventRecord(d->ev_I[cur], st));
-			if (dbg) cudaEventRecord(dbg[6], st);
 		}
 	HNS_LAUNCH(k_wait_rel, 1, 32, 0, bs, d->d_local_flags, np, 3, base + 1, uint32_t(iterations), d->d_err);  // the peers' last black push
 	HNS_CUDA(cudaEventRecord(d->ev_exchanged, bs));
 	HNS_CUDA(cudaStreamWaitEvent(st, d->ev_exchanged, 0));
 	HNS_LAUNCH(k_advance_bases, 1, 32, 0, st, d->d_seq_base, uint32_t(iterations));
-	return HNS_OK;
-}
-
-// (Replaying this pipeline as a CUDA graph -- two captured streams, which is why the sequence numbers live in device memory -- was
-// measured at 2 GPUs: 8.75 ms per frame against 8.54 ms launched directly; the graph's two branches do not overlap the way the
-// high-priority comm stream does. Removed; profiles/r2d_tune2_dist_graph.txt.)
-static int fused_pressure(hns_dist* d, hns_state* s, int iterations, float omega, cudaStream_t st, bool timed) {
-	const int rc = record_fused_pressure(d, s, iterations, omega, st, d->comm_stream, timed);
-	if (rc) return rc;
-	d->seq_p[0] += uint32_t(iterations), d->seq_p[1] += uint32_t(iterations), ++d->frame_id;  // host mirrors of the device bases
 	d->bytes_sent += d->push_bytes_per_sweep * 2u * uint64_t(iterations);
 	d->exchanges += 2u * uint64_t(iterations);
 	return HNS_OK;
@@ -790,6 +742,7 @@ static int fused_pressure(hns_dist* d, hns_state* s, int iterations, float omega
 // Half-sweep k reads colour c_{k-1} and writes colour c_k, so I_k and B_k/x_k never touch the same colour of the same leaf at the same
 // time, and the exchange latency disappears behind the interior sweep as long as B + x is the shorter chain. On return the caller's
 // stream has joined the exchanges: the ghosts of both colours are current. mg_flags: the multigrid solve's flag channels (peer memory).
+// The red-black solve of the NCCL fallback and of a rank without boundary leaves, and the smoother of the sharded multigrid solve.
 static int pipelined_sweeps(hns_dist* d, hns_state* s, int iterations, float omega, bool mg_flags, cudaStream_t st) {
 	GridView vb = s->grid->view, vi = s->grid->view;
 	vb.list = d->d_boundary, vb.num_list = d->n_boundary, vb.list_nbr = d->d_boundary_nbr;
@@ -811,7 +764,7 @@ static int pipelined_sweeps(hns_dist* d, hns_state* s, int iterations, float ome
 			if (d->n_interior) launch_rbgs_color(vi, s->div, s->p, dx, color, omega, color, st);
 			HNS_CUDA(cudaEventRecord(d->ev_I[cur], st));
 			if (!mg_flags) rc = exchange_channel(d, s, 2 + color, 1, color ? fblk : fred, bs);
-			else rc = d->peers.empty() ? HNS_OK : exchange_p2p(d, s, kChMgPressure + color, 1, color ? fblk : fred, bs, nullptr, 2 + color, 0);
+			else rc = d->peers.empty() ? HNS_OK : exchange_p2p(d, s, kChMgPressure + color, 1, color ? fblk : fred, bs, 2 + color, 0);
 			if (rc) return rc;
 		}
 	HNS_CUDA(cudaEventRecord(d->ev_exchanged, bs));
@@ -880,7 +833,7 @@ static int sharded_mg_pressure(hns_dist* d, hns_state* s, cudaStream_t st) {
 		}
 		launch_mg_prolong(g, s->p, nullptr, m.d_parent, mg->lv[1].grid->view, mg->lv[1].p, st);
 		for (int color = 0; color < 2 && !d->peers.empty(); ++color)
-			if ((rc = exchange_p2p(d, s, kChMgPressure + color, 1, fp + color, st, nullptr, 2 + color, 0))) return rc;
+			if ((rc = exchange_p2p(d, s, kChMgPressure + color, 1, fp + color, st, 2 + color, 0))) return rc;
 		if ((rc = pipelined_sweeps(d, s, m.nu_post, m.omega, true, st))) return rc;
 		++m.gathers;
 		m.gather_bytes += uint64_t(d->n_owned) * 256u * uint64_t(np);
@@ -910,7 +863,7 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 	if (hns_state_collision_active(s)) {
 		const int fsdf[1] = {10 + s->skip_scalar};
 		if (d->p2p) {
-			if ((rc = exchange_p2p(d, s, 7, 1, fsdf, st, nullptr, 5, 0))) return rc;
+			if ((rc = exchange_p2p(d, s, 7, 1, fsdf, st, 5, 0))) return rc;
 		} else if ((rc = hns_dist_exchange(d, s, 1, fsdf, st))) {
 			return rc;
 		}
@@ -932,7 +885,7 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 		const int fmag[1] = {26};
 		if ((rc = hns_state_vorticity_mag(s, stream))) return rc;
 		if (d->p2p) {
-			if ((rc = exchange_p2p(d, s, 7, 1, fmag, st, nullptr, 5, 0))) return rc;
+			if ((rc = exchange_p2p(d, s, 7, 1, fmag, st, 5, 0))) return rc;
 		} else if ((rc = hns_dist_exchange(d, s, 1, fmag, st))) {
 			return rc;
 		}
@@ -956,7 +909,7 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 		for (int i = 0; i < s->n_scalars; ++i) fsc.push_back(10 + i);
 		HNS_CUDA(cudaEventRecord(d->ev_scalars_final, st));
 		HNS_CUDA(cudaStreamWaitEvent(d->aux_stream, d->ev_scalars_final, 0));
-		if ((rc = exchange_p2p(d, s, 6, int(fsc.size()), fsc.data(), d->aux_stream, nullptr, 4, 3, d->aux_blocks))) return rc;
+		if ((rc = exchange_p2p(d, s, 6, int(fsc.size()), fsc.data(), d->aux_stream, 4, 3, kAuxBlocks))) return rc;
 		HNS_CUDA(cudaEventRecord(d->ev_scalars_exchanged, d->aux_stream));
 	}
 	mark();
@@ -965,9 +918,8 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 		if ((rc = sharded_mg_pressure(d, s, st))) return rc;
 	} else {
 		const float omega = hns_omega_compute(s->grid->voxel_size);
-		const bool fused = d->p2p && d->fused_push && d->n_boundary > 0;
-		if (fused) {
-			if ((rc = fused_pressure(d, s, iterations, omega, st, marks != nullptr))) return rc;
+		if (d->p2p && d->n_boundary > 0) {
+			if ((rc = fused_pressure(d, s, iterations, omega, st))) return rc;
 		} else if ((rc = pipelined_sweeps(d, s, iterations, omega, false, st))) {
 			return rc;
 		}
@@ -1135,62 +1087,6 @@ int hns_dist_mg_finish(hns_dist* d) {
 	return HNS_OK;
 }
 
-// after hns_dist_frame_timed: microseconds inside pressure half-sweep 20, all relative to the start of its boundary sweep:
-// out[0..4] = end of boundary sweep, end of push, end of signal+wait, end of unpack, (unused); out[5], out[6] = start / end of the interior sweep
-int hns_dist_debug_step(hns_dist* d, float* out7) {
-	if (!d || !out7 || !d->dbg_valid) return fail(HNS_ERR_RUNTIME, "no timed frame recorded");
-	for (int i = 1; i < 7; ++i) {
-		float ms = 0.f;
-		cudaEventElapsedTime(&ms, d->dbg[0], d->dbg[i]);
-		out7[i - 1] = ms * 1e3f;
-	}
-	out7[6] = 0.f;
-	return HNS_OK;
-}
-// Diagnostic: n pressure half-sweeps WITHOUT any exchange, timed with events (ms for all n). mode 0: every local leaf, no work list;
-// 1: owned list; 2: interior list only; 3: boundary list only; 4: interior on `stream` + boundary on the comm stream, pipelined like
-// the real solve. Ghost values go stale, so only the timing is meaningful.
-int hns_dist_time_sweeps(hns_dist* d, hns_state* s, int mode, int n, void* stream, float* ms_out) {
-	if (!d || !s || !ms_out || n <= 0 || mode < 0 || mode > 4) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument");
-	cudaStream_t st = static_cast<cudaStream_t>(stream), bs = d->comm_stream;
-	GridView vb = s->grid->view, vi = s->grid->view, vo = s->grid->view, va = s->grid->view;
-	vb.list = d->d_boundary, vb.num_list = d->n_boundary, vb.list_nbr = d->d_boundary_nbr;
-	vi.list = d->d_interior, vi.num_list = d->n_interior, vi.list_nbr = d->d_interior_nbr;
-	vo.list = d->d_owned, vo.num_list = d->n_owned;
-	const float dx = s->grid->voxel_size, omega = hns_omega_compute(dx);
-	cudaEvent_t e0, e1;
-	cudaEventCreate(&e0), cudaEventCreate(&e1);
-	cudaStreamSynchronize(st), cudaStreamSynchronize(bs);
-	cudaEventRecord(e0, st);
-	HNS_CUDA(cudaEventRecord(d->ev_I[1], st));
-	HNS_CUDA(cudaEventRecord(d->ev_B[1], bs));
-	for (int k = 0; k < n; ++k) {
-		const int color = k & 1, cur = k & 1, prev = cur ^ 1;
-		switch (mode) {
-			case 0: launch_rbgs_color(va, s->div, s->p, dx, color, omega, color, st); break;
-			case 1: launch_rbgs_color(vo, s->div, s->p, dx, color, omega, color, st); break;
-			case 2: launch_rbgs_color(vi, s->div, s->p, dx, color, omega, color, st); break;
-			case 3: launch_rbgs_color(vb, s->div, s->p, dx, color, omega, color, st); break;
-			default:
-				HNS_CUDA(cudaStreamWaitEvent(bs, d->ev_I[prev], 0));
-				launch_rbgs_color(vb, s->div, s->p, dx, color, omega, color, bs);
-				HNS_CUDA(cudaEventRecord(d->ev_B[cur], bs));
-				HNS_CUDA(cudaStreamWaitEvent(st, d->ev_B[prev], 0));
-				launch_rbgs_color(vi, s->div, s->p, dx, color, omega, color, st);
-				HNS_CUDA(cudaEventRecord(d->ev_I[cur], st));
-		}
-	}
-	if (mode == 4) {
-		HNS_CUDA(cudaEventRecord(d->ev_exchanged, bs));
-		HNS_CUDA(cudaStreamWaitEvent(st, d->ev_exchanged, 0));
-	}
-	cudaEventRecord(e1, st);
-	cudaStreamSynchronize(st);
-	cudaEventElapsedTime(ms_out, e0, e1);
-	cudaEventDestroy(e0), cudaEventDestroy(e1);
-	HNS_CUDA(cudaGetLastError());
-	return HNS_OK;
-}
 // global sums of the ranks' fp64 partial sums (residual / divergence norms): ncclAllReduce(sum, fp64), SURVEY.md 8e
 int hns_dist_allreduce_sum(hns_dist* d, double* inout_host, int n, void* stream) {
 	if (!d || !inout_host || n <= 0 || n > 16) return fail(HNS_ERR_INVALID_ARGUMENT, "bad argument");

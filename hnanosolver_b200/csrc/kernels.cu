@@ -350,8 +350,8 @@ __device__ __forceinline__ float sor_update_diag(float pxp, float pxm, float pyp
 // `reverse` walks the leaves back to front: consecutive launches alternate direction so that each one starts on the bricks the
 // previous launch touched last, which are still resident in the 126 MB L2.
 // kPush: the sharded run's boundary sweep -- every freshly swept quad is also stored straight into the ghost copy of the leaf on
-// each peer GPU that holds one (NVLink peer memory, CUDA IPC), and the last block to finish raises the peers' arrival flags:
-// compute and ghost exchange are one kernel, nothing is packed, sent or unpacked afterwards.
+// each peer GPU that holds one (NVLink peer memory, CUDA IPC): nothing is packed, sent or unpacked afterwards; the caller raises the
+// peers' arrival flags from a follow-up kernel.
 // kMask: a coarse level of the multigrid solve -- `diag_c` holds the operator's diagonal of every cell of the swept colour: 6 plus a
 // boundary term per face neighbour outside the domain (multigrid.cu), 0 for a cell that is itself outside. Such cells keep the value 0
 // they were initialised with, which is the Dirichlet condition of the reference's solve (inactive -> 0); the update divides by the
@@ -361,82 +361,64 @@ __global__ void __launch_bounds__(256) k_rbgs_split(GridView g, const float* __r
                                                     float dx2, int color, float omega, int reverse, RbgsPush push,
                                                     const float* __restrict__ diag_c = nullptr) {
 	RowCtx c;
-	const bool flags_stream_div = (reverse & 2) == 0;  // bit 1 of `reverse`: A/B switch, plain read-only loads of the divergence
-	reverse &= 1;
 	uint32_t i = blockIdx.x * 4u + (threadIdx.x >> 6);
-	const bool active = i < g.count();
-	if (!active && !(kPush && push.counter)) return;
-	if (active) {
-		if (reverse) i = g.count() - 1u - i;
-		const int r = threadIdx.x & 63;
-		c.x = r >> 3, c.y = r & 7;
-		if (g.list_nbr) {
-			c.nbr = g.list_nbr + uint64_t(i) * 27u;
-			c.leaf = uint32_t(__ldg(c.nbr + kSlotSelf));
-		} else {
-			c.leaf = g.leaf_at(i);
-			c.nbr = g.nbr + uint64_t(c.leaf) * 27u;
-		}
-		const uint32_t q = c.self_q();
-		const int sc = (c.x + c.y + color) & 1;  // swept voxels of this row are z = 2j + sc
-		const float4 C = ld4(p_c, q);            // old values of the swept colour (only this thread writes them)
-		// other colour: plain (coherent) loads when peers write ghost values into this array, read-only path otherwise
-		auto ldo = [&](uint64_t idx) { return kPush ? ld4(p_o, idx) : ldg4(p_o, idx); };
-		const float4 O = ldo(q);                 // own row: the z neighbours
-		uint32_t t;
-		const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
-		const float4 Oxp = (t = c.row_q(1, 0)) != RowCtx::kNoRow ? ldo(t) : zero4;
-		const float4 Oxm = (t = c.row_q(-1, 0)) != RowCtx::kNoRow ? ldo(t) : zero4;
-		const float4 Oyp = (t = c.row_q(0, 1)) != RowCtx::kNoRow ? ldo(t) : zero4;
-		const float4 Oym = (t = c.row_q(0, -1)) != RowCtx::kNoRow ? ldo(t) : zero4;
-		// the divergence is read once per sweep and not again before 2 x 240 MB of pressure have passed through the L2: load it
-		// with the streaming (evict-first) policy so that it does not displace pressure lines the next, reversed sweep starts on
-		const float4 D = (flags_stream_div) ? __ldcs(reinterpret_cast<const float4*>(div_c + q)) : ldg4(div_c, q);
-		// z neighbours: sc == 0: voxel j (z = 2j) has below = O[j-1] (j = 0: last other-colour voxel of the -z leaf), above = O[j]
-		//               sc == 1: voxel j (z = 2j+1) has below = O[j], above = O[j+1] (j = 3: first other-colour voxel of the +z leaf)
-		float halo = 0.f;
-		if (sc == 0) {
-			if ((t = c.z_q(kSlotZm)) != RowCtx::kNoRow) halo = p_o[t + 3u];
-		} else {
-			if ((t = c.z_q(kSlotZp)) != RowCtx::kNoRow) halo = p_o[t];
-		}
-		const float b0 = sc ? O.x : halo, b1 = sc ? O.y : O.x, b2 = sc ? O.z : O.y, b3 = sc ? O.w : O.z;  // below (z-1)
-		const float a0 = sc ? O.y : O.x, a1 = sc ? O.z : O.y, a2 = sc ? O.w : O.z, a3 = sc ? halo : O.w;  // above (z+1)
-		float4 n;
-		n.x = sor_update(Oxp.x, Oxm.x, Oyp.x, Oym.x, a0, b0, D.x, C.x, dx2, omega);
-		n.y = sor_update(Oxp.y, Oxm.y, Oyp.y, Oym.y, a1, b1, D.y, C.y, dx2, omega);
-		n.z = sor_update(Oxp.z, Oxm.z, Oyp.z, Oym.z, a2, b2, D.z, C.z, dx2, omega);
-		n.w = sor_update(Oxp.w, Oxm.w, Oyp.w, Oym.w, a3, b3, D.w, C.w, dx2, omega);
-		if (kMask) {
-			const float4 W = ldg4(diag_c, q);
-			n.x = W.x != 0.f ? sor_update_diag(Oxp.x, Oxm.x, Oyp.x, Oym.x, a0, b0, D.x, C.x, dx2, omega, W.x) : 0.f;
-			n.y = W.y != 0.f ? sor_update_diag(Oxp.y, Oxm.y, Oyp.y, Oym.y, a1, b1, D.y, C.y, dx2, omega, W.y) : 0.f;
-			n.z = W.z != 0.f ? sor_update_diag(Oxp.z, Oxm.z, Oyp.z, Oym.z, a2, b2, D.z, C.z, dx2, omega, W.z) : 0.f;
-			n.w = W.w != 0.f ? sor_update_diag(Oxp.w, Oxm.w, Oyp.w, Oym.w, a3, b3, D.w, C.w, dx2, omega, W.w) : 0.f;
-		}
-		*reinterpret_cast<float4*>(p_c + q) = n;
-		if (kPush) {
-			const uint32_t row4 = q & 255u;  // quad offset inside the half-brick
-			// bit f of this row's face membership: 0 x==0, 1 x==7, 2 y==0, 3 y==7; a z face (bits 4, 5) involves every row
-			const int mine = (c.x == 0 ? 1 : 0) | (c.x == 7 ? 2 : 0) | (c.y == 0 ? 4 : 0) | (c.y == 7 ? 8 : 0) | 0x30;
-			for (uint32_t e = __ldg(push.dst_off + i), e1 = __ldg(push.dst_off + i + 1); e < e1; ++e) {
-				const int pm = __ldg(push.dst_peer + e);  // peer index | face mask << 8
-				if ((pm >> 8) & mine)
-					*reinterpret_cast<float4*>(push.remote_pc[pm & 255] + (uint64_t(__ldg(push.dst_leaf + e)) * 256u + row4)) = n;
-			}
-		}
+	if (i >= g.count()) return;
+	if (reverse) i = g.count() - 1u - i;
+	const int r = threadIdx.x & 63;
+	c.x = r >> 3, c.y = r & 7;
+	if (g.list_nbr) {
+		c.nbr = g.list_nbr + uint64_t(i) * 27u;
+		c.leaf = uint32_t(__ldg(c.nbr + kSlotSelf));
+	} else {
+		c.leaf = g.leaf_at(i);
+		c.nbr = g.nbr + uint64_t(c.leaf) * 27u;
 	}
-	if (kPush && push.counter) {  // in-kernel arrival signal (otherwise the caller launches a signal kernel behind this one)
-		__threadfence_system();  // this block's peer stores are performed before it counts itself done
-		__syncthreads();
-		if (threadIdx.x == 0) {
-			const uint32_t done = atomicAdd(push.counter, 1u);
-			if (done == gridDim.x - 1u) {
-				*push.counter = 0u;
-				__threadfence_system();
-				for (int pp = 0; pp < push.n_peers; ++pp)
-					if (push.signal_flags[pp]) asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(push.signal_flags[pp] + push.signal_ch), "r"(push.signal_seq) : "memory");
-			}
+	const uint32_t q = c.self_q();
+	const int sc = (c.x + c.y + color) & 1;  // swept voxels of this row are z = 2j + sc
+	const float4 C = ld4(p_c, q);            // old values of the swept colour (only this thread writes them)
+	// other colour: plain (coherent) loads when peers write ghost values into this array, read-only path otherwise
+	auto ldo = [&](uint64_t idx) { return kPush ? ld4(p_o, idx) : ldg4(p_o, idx); };
+	const float4 O = ldo(q);                 // own row: the z neighbours
+	uint32_t t;
+	const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
+	const float4 Oxp = (t = c.row_q(1, 0)) != RowCtx::kNoRow ? ldo(t) : zero4;
+	const float4 Oxm = (t = c.row_q(-1, 0)) != RowCtx::kNoRow ? ldo(t) : zero4;
+	const float4 Oyp = (t = c.row_q(0, 1)) != RowCtx::kNoRow ? ldo(t) : zero4;
+	const float4 Oym = (t = c.row_q(0, -1)) != RowCtx::kNoRow ? ldo(t) : zero4;
+	// the divergence is read once per sweep and not again before 2 x 240 MB of pressure have passed through the L2: load it
+	// with the streaming (evict-first) policy so that it does not displace pressure lines the next, reversed sweep starts on
+	const float4 D = __ldcs(reinterpret_cast<const float4*>(div_c + q));
+	// z neighbours: sc == 0: voxel j (z = 2j) has below = O[j-1] (j = 0: last other-colour voxel of the -z leaf), above = O[j]
+	//               sc == 1: voxel j (z = 2j+1) has below = O[j], above = O[j+1] (j = 3: first other-colour voxel of the +z leaf)
+	float halo = 0.f;
+	if (sc == 0) {
+		if ((t = c.z_q(kSlotZm)) != RowCtx::kNoRow) halo = p_o[t + 3u];
+	} else {
+		if ((t = c.z_q(kSlotZp)) != RowCtx::kNoRow) halo = p_o[t];
+	}
+	const float b0 = sc ? O.x : halo, b1 = sc ? O.y : O.x, b2 = sc ? O.z : O.y, b3 = sc ? O.w : O.z;  // below (z-1)
+	const float a0 = sc ? O.y : O.x, a1 = sc ? O.z : O.y, a2 = sc ? O.w : O.z, a3 = sc ? halo : O.w;  // above (z+1)
+	float4 n;
+	n.x = sor_update(Oxp.x, Oxm.x, Oyp.x, Oym.x, a0, b0, D.x, C.x, dx2, omega);
+	n.y = sor_update(Oxp.y, Oxm.y, Oyp.y, Oym.y, a1, b1, D.y, C.y, dx2, omega);
+	n.z = sor_update(Oxp.z, Oxm.z, Oyp.z, Oym.z, a2, b2, D.z, C.z, dx2, omega);
+	n.w = sor_update(Oxp.w, Oxm.w, Oyp.w, Oym.w, a3, b3, D.w, C.w, dx2, omega);
+	if (kMask) {
+		const float4 W = ldg4(diag_c, q);
+		n.x = W.x != 0.f ? sor_update_diag(Oxp.x, Oxm.x, Oyp.x, Oym.x, a0, b0, D.x, C.x, dx2, omega, W.x) : 0.f;
+		n.y = W.y != 0.f ? sor_update_diag(Oxp.y, Oxm.y, Oyp.y, Oym.y, a1, b1, D.y, C.y, dx2, omega, W.y) : 0.f;
+		n.z = W.z != 0.f ? sor_update_diag(Oxp.z, Oxm.z, Oyp.z, Oym.z, a2, b2, D.z, C.z, dx2, omega, W.z) : 0.f;
+		n.w = W.w != 0.f ? sor_update_diag(Oxp.w, Oxm.w, Oyp.w, Oym.w, a3, b3, D.w, C.w, dx2, omega, W.w) : 0.f;
+	}
+	*reinterpret_cast<float4*>(p_c + q) = n;
+	if (kPush) {
+		const uint32_t row4 = q & 255u;  // quad offset inside the half-brick
+		// bit f of this row's face membership: 0 x==0, 1 x==7, 2 y==0, 3 y==7; a z face (bits 4, 5) involves every row
+		const int mine = (c.x == 0 ? 1 : 0) | (c.x == 7 ? 2 : 0) | (c.y == 0 ? 4 : 0) | (c.y == 7 ? 8 : 0) | 0x30;
+		for (uint32_t e = __ldg(push.dst_off + i), e1 = __ldg(push.dst_off + i + 1); e < e1; ++e) {
+			const int pm = __ldg(push.dst_peer + e);  // peer index | face mask << 8
+			if ((pm >> 8) & mine)
+				*reinterpret_cast<float4*>(push.remote_pc[pm & 255] + (uint64_t(__ldg(push.dst_leaf + e)) * 256u + row4)) = n;
 		}
 	}
 }
@@ -471,18 +453,6 @@ void launch_gather_nbr_rows(const int32_t* nbr, const int32_t* list, uint32_t n,
 }
 
 // (the advection kernels live in advect.cu)
-
-// element 0 of velocity (x,y,z) and of each scalar field -> dst[3 + S]
-__global__ void k_gather_element0(const float* u, const float* v, const float* w, ScalarPtrs sp, int S, float* __restrict__ dst) {
-	const int t = threadIdx.x;
-	if (t == 0) dst[0] = u[0];
-	if (t == 1) dst[1] = v[0];
-	if (t == 2) dst[2] = w[0];
-	if (t >= 3 && t < 3 + S) dst[t] = sp.in[t - 3][0];
-}
-void launch_gather_element0(const float* const vel[3], const ScalarPtrs& sp, int S, float* dst, cudaStream_t st) {
-	HNS_LAUNCH(k_gather_element0, 1, 32, 0, st, vel[0], vel[1], vel[2], sp, S, dst);
-}
 
 // =============================================================================================================
 // combustion_oxygen / temperature_buoyancy  (reference Kernel.cu:923-966, 831-847) -- element-wise

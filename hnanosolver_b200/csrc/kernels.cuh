@@ -70,16 +70,13 @@ void launch_advect_vector(const GridView& g, const float* const vel[3], float* c
                           const CombustionJob* comb = nullptr);
 
 // advect_scalars (Kernel.cu:118-266) when sampler_semantics == 0; advect_scalar (Kernel.cu:269-352) per field when == 1
-// elem0 (device, float[3 + S], may be null): element 0 of the GLOBAL velocity / scalar arrays, the value advect_scalars reads for
-// inactive voxels; null = element 0 of the arrays passed in (single-GPU runs).
+// advect_scalars reads element 0 of the arrays passed in for inactive voxels (a shard's local leaf 0 is global leaf 0, dist.py::make_plan)
 void launch_advect_scalars(const GridView& g, const float* const vel[3], const ScalarPtrs& sp, int S, float dt, float inv_dx,
-                           int sampler_semantics, const float* elem0, cudaStream_t st, const float* sdf, uint8_t* cold,
-                           const AdvectGroups* grp = nullptr);
+                           int sampler_semantics, cudaStream_t st, const float* sdf, uint8_t* cold, const AdvectGroups* grp = nullptr);
 // enforceCollisionBoundaries (Kernel.cu:77-116; blend_divisor 0.1, mixed_sum 0) and the boundary tails of advect_vector (:432-450;
 // 1.5, 1) and subtractPressureGradient (:808-826; 0.1, 0): vel -> out (may alias), per voxel
 void launch_collision_boundary(const GridView& g, const float* const vel[3], float* const out[3], const float* sdf, float inv_dx,
                                float blend_divisor, int mixed_sum, cudaStream_t st);
-void launch_gather_element0(const float* const vel[3], const ScalarPtrs& sp, int S, float* dst, cudaStream_t st);
 // divergence (Kernel.cu:499-519); burn != null: plus combustion's expansion term, div = fma(burn, expansion, div) where burn != -1
 void launch_divergence(const GridView& g, const float* const vel[3], float* const div[2], float inv_dx, cudaStream_t st, const float* burn = nullptr,
                        float expansion = 0.f);
@@ -89,17 +86,13 @@ void launch_rbgs_color(const GridView& g, const float* const div[2], float* cons
 // Boundary sweep of a sharded run with the ghost exchange fused in: besides writing p[color] locally, every swept quad of work item i
 // is stored into the ghost copies listed in dst_peer/dst_leaf[dst_off[i] .. dst_off[i+1]) (peer index | face mask << 8 -- only rows on
 // a face the peer's stencil reads are stored: bits 0..3 = x==0, x==7, y==0, y==7, bits 4..5 = a z face = every row --, leaf id in that peer's local
-// numbering) through remote_pc[peer] = that peer's p[color] array mapped over NVLink. With a counter the last block to finish also
-// raises signal_flags[*][signal_ch] (every block then pays a system fence); without one the caller signals from a follow-up kernel.
+// numbering) through remote_pc[peer] = that peer's p[color] array mapped over NVLink. The caller raises the peers' arrival flags from
+// a follow-up kernel.
 struct RbgsPush {
 	const uint32_t* dst_off = nullptr;
 	const int32_t* dst_peer = nullptr;
 	const int32_t* dst_leaf = nullptr;
 	float* const* remote_pc = nullptr;
-	uint32_t* const* signal_flags = nullptr;
-	int n_peers = 0, signal_ch = 0;
-	uint32_t signal_seq = 0;
-	uint32_t* counter = nullptr;
 };
 void launch_rbgs_color_push(const GridView& g, const float* const div[2], float* const p[2], float dx, int color, float omega, int reverse,
                             const RbgsPush& push, cudaStream_t st);

@@ -64,16 +64,17 @@ __device__ __forceinline__ void corner_weights(float tx, float ty, float tz, flo
 	w[0] = w00 * itz, w[1] = w10 * itz, w[2] = w01 * itz, w[3] = w11 * itz;
 	w[4] = w00 * tz, w[5] = w10 * tz, w[6] = w01 * tz, w[7] = w11 * tz;
 }
-// cold path: weighted 8-corner sums through the leaf table / tree walk, for samples outside the staged region
-static __device__ __noinline__ float far_weighted(const GridView& g, const LeafFrame& f, const float* __restrict__ a, const float* __restrict__ e0, int i0,
-                                           int j0, int k0, float tx, float ty, float tz) {
+// cold path: weighted 8-corner sums through the leaf table / tree walk, for samples outside the staged region; inactive corners read
+// array element 0
+static __device__ __noinline__ float far_weighted(const GridView& g, const LeafFrame& f, const float* __restrict__ a, int i0, int j0, int k0, float tx,
+                                           float ty, float tz) {
 	float wt[8];
 	corner_weights(tx, ty, tz, wt);
 	float acc = 0.f;
 #pragma unroll 1
 	for (int q = 0; q < 8; ++q) {
 		const int64_t t = voxel_index(g, f, i0 + (q & 1), j0 + ((q >> 1) & 1), k0 + (q >> 2));
-		acc = fmaf(t < 0 ? __ldg(e0) : __ldg(a + t), wt[q], acc);
+		acc = fmaf(t < 0 ? __ldg(a) : __ldg(a + t), wt[q], acc);
 	}
 	return acc;
 }

@@ -407,21 +407,7 @@ class ShardedSimulation:
 
         ms = (C.c_float * 8)()
         _lib.check(_lib.lib().hns_dist_frame_timed(self._dist, self.sim._h, iterations, dt, C.c_void_p(self._stream()), ms))
-        out = dict(zip(self.PHASES, [float(x) for x in ms]))
-        step = (C.c_float * 7)()
-        if _lib.lib().hns_dist_debug_step(self._dist, step) == 0:
-            out["step20_us(B_end,push_end,wait_end,unpack_end,I_start,I_end)"] = [round(float(x), 1) for x in step[:6]]
-        return out
-
-    def time_sweeps(self, mode: int, n: int) -> float:
-        """microseconds per exchange-free pressure half-sweep (diagnostic; see hns_dist_time_sweeps for the modes)"""
-        import ctypes as C
-
-        from . import _lib
-
-        ms = C.c_float()
-        _lib.check(_lib.lib().hns_dist_time_sweeps(self._dist, self.sim._h, mode, n, C.c_void_p(self._stream()), C.byref(ms)))
-        return float(ms.value) * 1e3 / n
+        return dict(zip(self.PHASES, [float(x) for x in ms]))
 
     def owned(self, arr: np.ndarray) -> np.ndarray:
         """Rows of a per-voxel local array that belong to owned leaves."""

@@ -382,12 +382,6 @@ class Simulation:
     def field_ptr(self, field: int) -> int:
         return _lib.lib().hns_state_field_device_ptr(self._h, field) or 0
 
-    def gather_element0(self, dst_dev_ptr: int, stream=None):
-        check(_lib.lib().hns_state_gather_element0(self._h, C.c_void_p(dst_dev_ptr), _stream(stream)))
-
-    def set_element0(self, values_dev_ptr: int | None):
-        check(_lib.lib().hns_state_set_element0(self._h, C.c_void_p(values_dev_ptr) if values_dev_ptr else None))
-
     def pack_leaves(self, field: int, ids_dev_ptr: int, n_ids: int, dst_dev_ptr: int, stream=None):
         check(_lib.lib().hns_state_pack_leaves(self._h, field, C.c_void_p(ids_dev_ptr), n_ids, C.c_void_p(dst_dev_ptr), _stream(stream)))
 

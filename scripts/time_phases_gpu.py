@@ -25,21 +25,13 @@ stages = [("advect_vector", lambda: sim.advect_velocity(w.dt, st)),
           ("divergence", lambda: sim.divergence(True, st)),
           ("combustion+buoyancy", lambda: sim.combustion_buoyancy(w.dt, st)),
           ("pressure_solve(40)", lambda: sim.pressure_solve(40, omega, 0, st)),
-          ("pressure_solve(40) plain div loads", lambda: sim.pressure_solve(40, omega, 4, st)),
           ("pressure_solve(40) forward only", lambda: sim.pressure_solve(40, omega, 2, st)),
           ("pressure_solve(40) again", lambda: sim.pressure_solve(40, omega, 0, st)),
           ("subtract_gradient", lambda: sim.subtract_gradient(True, st)),
           ("advect_scalars(5)", lambda: sim.advect_scalars(w.dt, 0, st))]
-from hnanosolver_b200 import _lib
-pre = {}
-for mb in (() if not os.environ.get("L2_SWEEP") else (0, 32, 48, 64, 80, 96, 0)):
-    pre[f"pressure_solve(40) L2 persist {mb} MB"] = (lambda mb=mb: (_lib.lib().hns_set_l2_persist_mb(mb), sim.pressure_solve(2, omega, 0, st)))
-    stages.append((f"pressure_solve(40) L2 persist {mb} MB", lambda: sim.pressure_solve(40, omega, 0, st)))
 acc = {k: [] for k, _ in stages}
 for r in range(reps + 2):
     for k, fn in stages:
-        if k in pre:
-            pre[k](); torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); fn(); e1.record(); torch.cuda.synchronize()
         if r >= 2:

@@ -46,6 +46,15 @@ def test_no_cpu_fallback_when_library_missing(monkeypatch):
         _lib.lib()
 
 
+def test_native_environment_switches():
+    """The library reads only the switches whose two sides both stay in the product (each side is compared bit for bit by the tests)."""
+    names = set()
+    for dp, _, files in os.walk(os.path.join(ROOT, "hnanosolver_b200", "csrc")):
+        for f in files:
+            names |= set(re.findall(r"getenv\(\s*\"(HNS_[A-Z0-9_]+)\"", open(os.path.join(dp, f), errors="replace").read()))
+    assert names == {"HNS_ADVECT4", "HNS_FUSED_COMBUSTION", "HNS_MG_GRAPH"}
+
+
 def test_product_does_not_touch_the_oracle():
     pkg = os.path.join(ROOT, "hnanosolver_b200")
     for dp, _, files in os.walk(pkg):

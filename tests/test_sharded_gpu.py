@@ -17,8 +17,6 @@ pytestmark = pytest.mark.gpu
 
 P2P_MODES = [
     dict(),                                                       # fused boundary sweep + push, two frames (velocity-ghost reuse)
-    dict(env=dict(HNS_FUSED_PUSH=0)),                             # pack / push / signal / wait / unpack kernels
-    dict(env=dict(HNS_SIGNAL_IN_KERNEL=1)),                       # the boundary sweep raises the arrival flags itself
     dict(vorticity=[0.8, 2.0]),                                   # vorticity confinement with the |curl| ghost exchange
     dict(collision=True),                                         # SDF collision path
     dict(cook=True),                                              # host-buffer entry point (hns_dist_cook), garbage in the ghost entries
@@ -66,7 +64,7 @@ def test_sharded_frame_is_bitwise_the_single_gpu_frame_peer_memory(world):
     assert reports[0]["exchanges_per_frame"] >= 2 * 12       # the pressure ghosts travel after every half-sweep
     # the sharded frame runs the packed (third-generation) advection kernels too: advect_scalars in both frames, advect_vector in the
     # second one (velocity ghosts and group 0 carried over); none with collision data
-    assert reports[0]["packed_advection_launches"] == 3 and reports[4]["packed_advection_launches"] == 0
+    assert reports[0]["packed_advection_launches"] == 3 and reports[2]["packed_advection_launches"] == 0
 
 
 def test_sharded_frame_is_bitwise_the_single_gpu_frame_nccl():
@@ -79,4 +77,4 @@ def test_sharded_frame_is_bitwise_the_single_gpu_frame_nccl():
 def test_sharded_frame_four_ranks():
     if _gpus() < 4:
         pytest.skip("needs 4 GPUs")
-    _run(4, P2P_MODES[:1] + P2P_MODES[3:6] + NCCL_MODES[:1], False)
+    _run(4, P2P_MODES[:1] + P2P_MODES[1:4] + NCCL_MODES[:1], False)

@@ -27,7 +27,6 @@ MG_MODES = [
     dict(multigrid=dict(cycles=3, nu_pre=1, nu_post=0)),                 # no post-smoothing: the exchange after the prolongation feeds the
     dict(multigrid=dict(cycles=3, nu_pre=0, nu_post=1)),                 # next residual / gradient; no pre-smoothing: it feeds the red sweep
     dict(multigrid=dict(max_levels=2)),                                  # level 1 is the last level (smoothed, not solved in one CTA)
-    dict(multigrid=dict(), env=dict(HNS_FUSED_PUSH=0)),
     dict(multigrid=dict(), env=dict(HNS_MG_GRAPH=0)),                     # coarse levels launched directly instead of a CUDA graph
     dict(multigrid=dict(), cook=True),                                   # host-buffer entry point (hns_dist_cook)
     dict(multigrid=dict(), collision=True, vorticity=[0.8, 2.0]),
