@@ -66,21 +66,20 @@ static int pressure_solve(hns_state* s, int iterations, float dx, float omega, u
 // ---- packed groups of the advection kernels (advect.cu, third generation) ------------------------------------------------------------
 // The kernels that write the velocity and the scalars right before an advection pass also write them as float4 groups:
 // subtractPressureGradient -> group 0 {u, v, w, first advected scalar}, combustion -> group 1 {fuel, waste, temperature, flame}.
-// A group is current while the version counters it was written at still match (hns_state::vel_version / sc_version, bumped by every
-// entry point that may overwrite the brick fields) and it was built from the very buffers the advection pass is about to read; otherwise
-// the advection launchers fall back to the second-generation kernels on the brick fields. Not used with collision data (the boundary
-// pass rewrites the velocity after the gradient), nor with a work list unless it is a sharded frame's: the kernels then write the groups
-// of the owned leaves and dist.cu re-packs the ghost leaves after the exchange in front of the advection pass (groups_refresh_leaves).
-static bool groups_allowed(const hns_state* s) {
-	return s->n && (!s->active || s->grp_dist) && !s->collision_sdf() && packed_advection_enabled();
-}
+// Every producer records what it wrote with group_written: the brick field behind each lane and the version counters
+// (hns_state::vel_version / sc_version, bumped by every entry point that may overwrite the brick fields). A consumer asks
+// group_if_current for the fields it is about to read and gets the group only while those lanes mirror exactly those buffers and the
+// counters the lanes depend on have not moved since; otherwise it runs the second-generation kernels on the brick fields. Not used
+// with collision data (the boundary pass rewrites the velocity after the gradient). In a sharded frame the kernels write the groups of
+// the owned leaves only; dist.cu re-packs the ghost leaves after the exchange in front of the advection pass and records them again.
+static bool groups_allowed(const hns_state* s) { return s->n && !s->collision_sdf() && packed_advection_enabled(); }
 static bool ensure_group(hns_state* s, int j) {
-	if (!s->grp.g[j] && cudaMalloc(&s->grp.g[j], s->n * sizeof(float4)) != cudaSuccess) {
+	float4*& buf = s->grp[j].buf;
+	if (!buf && cudaMalloc(&buf, s->n * sizeof(float4)) != cudaSuccess) {
 		cudaGetLastError();
-		s->grp.g[j] = nullptr;
+		buf = nullptr;
 	}
-	s->grp.n = s->n;
-	return s->grp.g[j] != nullptr;
+	return buf != nullptr;
 }
 // The scalars an advection pass moves, in the order it moves them: every scalar except the one marked as not advected
 // ("collision_sdf", HNanoSolver.cu:327). When the state carries exactly one scalar besides the four combustion fields -- the
@@ -113,38 +112,50 @@ static bool combustion_packs(const hns_state* s) {  // will advect_scalars find 
 	return true;
 }
 
-GroupsCurrent groups_current(const hns_state* s) {
-	GroupsCurrent c;
-	if (!groups_allowed(s)) return c;
-	c.g0 = s->grp.g[0] && s->grp0_vel_version == s->vel_version && s->grp0_sc_version == s->sc_version;
-	c.g1 = s->grp.g[1] && s->grp1_sc_version == s->sc_version;
-	return c;
+// The fields the advection passes read from group j, which are also what its producers pack: {u, v, w, first advected scalar} and
+// {advected scalars 1..4}; a lane past the end of the list is null.
+void group_wants(const hns_state* s, int j, const float* want[4]) {
+	int idx[16];
+	const int S = advect_list(s, idx);
+	for (int k = 0; k < 4; ++k) {
+		const int i = j == 0 ? k - 3 : k + 1;  // position in the list; lanes 0..2 of group 0 are the velocity
+		want[k] = i < 0 ? s->vel[k] : i < S ? s->sc[idx[i]] : nullptr;
+	}
 }
-int groups_refresh_leaves(hns_state* s, const int32_t* ids, uint64_t n_ids, GroupsCurrent which, cudaStream_t st) {
-	if (which.g0) launch_pack4_leaves(ids, n_ids, s->vel[0], s->vel[1], s->vel[2], s->grp0_s0, s->grp.g[0], st);
-	if (which.g1) launch_pack4_leaves(ids, n_ids, s->grp1_src[0], s->grp1_src[1], s->grp1_src[2], s->grp1_src[3], s->grp.g[1], st);
-	HNS_CUDA(cudaGetLastError());
-	return HNS_OK;
+// Group j if every non-null lane of `want` is the field the group mirrors and that field's counter has not moved since the group was
+// written: vel_version for lanes 0..2 of group 0, sc_version for every other lane. Null otherwise.
+const float4* group_if_current(const hns_state* s, int j, const float* const want[4]) {
+	const PackedGroup& g = s->grp[j];
+	if (!groups_allowed(s) || !g.buf) return nullptr;
+	for (int k = 0; k < 4; ++k) {
+		const bool velocity = j == 0 && k < 3;
+		if (want[k] && (g.src[k] != want[k] || (velocity ? g.vel_version != s->vel_version : g.sc_version != s->sc_version))) return nullptr;
+	}
+	return g.buf;
 }
-void groups_stamp(hns_state* s, GroupsCurrent which) {
-	if (which.g0) s->grp0_vel_version = s->vel_version, s->grp0_sc_version = s->sc_version;
-	if (which.g1) s->grp1_sc_version = s->sc_version;
+// after a producer has written group j from `src` and bumped the counters of the fields it wrote
+void group_written(hns_state* s, int j, const float* const src[4]) {
+	PackedGroup& g = s->grp[j];
+	std::copy(src, src + 4, g.src);
+	g.vel_version = s->vel_version, g.sc_version = s->sc_version;
 }
 
-static bool group0_current(const hns_state* s) { return groups_allowed(s) && s->grp.g[0] && s->grp0_vel_version == s->vel_version; }
+static const float4* velocity_group(const hns_state* s) {  // group 0 as advect_vector reads it: the velocity lanes only
+	const float* const want[4] = {s->vel[0], s->vel[1], s->vel[2], nullptr};
+	return group_if_current(s, 0, want);
+}
 static int stage_advect_velocity(hns_state* s, float dt, float inv, cudaStream_t st, const CombustionJob* comb = nullptr) {
-	const bool packed = group0_current(s);
-	s->grp.valid = packed ? 1u : 0u;
-	launch_advect_vector(s->view(), s->vel, s->adv, dt, inv, st, s->collision_sdf(), s->cold, packed ? &s->grp : nullptr, comb);
+	launch_advect_vector(s->view(), s->vel, s->adv, dt, inv, st, s->collision_sdf(), s->cold, velocity_group(s), comb);
 	return HNS_OK;
 }
 // the combustion fields' outputs become the current fields (HNanoSolver.cu:239-246); `packed`: group 1 was written along with them
 static void combustion_swap(hns_state* s, bool packed) {
-	for (int c = 0; c < 4; ++c) std::swap(s->sc[s->comb_idx[c]], s->sc_out[s->comb_idx[c]]);
+	const int* ci = s->comb_idx;
+	for (int c = 0; c < 4; ++c) std::swap(s->sc[ci[c]], s->sc_out[ci[c]]);
 	++s->sc_version;
 	if (packed) {
-		s->grp1_sc_version = s->sc_version;
-		for (int c = 0; c < 4; ++c) s->grp1_src[c] = s->sc[s->comb_idx[c]];
+		const float* const src[4] = {s->sc[ci[0]], s->sc[ci[1]], s->sc[ci[2]], s->sc[ci[3]]};
+		group_written(s, 1, src);
 	}
 }
 // update_div / buoyancy = false: the expansion term is already in the divergence (launch_combustion_divergence), the buoyancy force
@@ -154,7 +165,7 @@ static int stage_combustion_buoyancy(hns_state* s, float dt, cudaStream_t st, bo
 	const bool packed = combustion_packs(s) && ensure_group(s, 1);
 	if (packed) {
 		launch_combustion_buoyancy_packed(s->sc[iF], s->sc[iW], s->sc[iT], s->div, s->sc[iL], s->sc_out[iF], s->sc_out[iW], s->sc_out[iT], s->sc_out[iL],
-		                                  s->grp.g[1], s->adv, s->comb.temperatureRelease, s->comb.expansionRate, dt, s->comb.ambientTemp,
+		                                  s->grp[1].buf, s->adv, s->comb.temperatureRelease, s->comb.expansionRate, dt, s->comb.ambientTemp,
 		                                  s->comb.buoyancyStrength, s->n, st, update_div, buoyancy);
 	} else {
 		launch_combustion_oxygen(s->sc[iF], s->sc[iW], s->sc[iT], s->div, s->sc[iL], s->sc_out[iF], s->sc_out[iW], s->sc_out[iT], s->sc_out[iL],
@@ -167,13 +178,13 @@ static int stage_combustion_buoyancy(hns_state* s, float dt, cudaStream_t st, bo
 // adv - grad p -> vel (from_advected), or in place on vel (the stand-alone projection; every thread reads only its own velocity row)
 // buoy: the buoyancy force goes onto the advected velocity in the same pass (frame() with the fused combustion pass)
 static int stage_subtract_gradient(hns_state* s, bool from_advected, float inv, cudaStream_t st, bool allow_group = true, const Buoyancy* buoy = nullptr) {
-	int idx[16];
-	const int S = advect_list(s, idx);
 	const bool packed = allow_group && from_advected && groups_allowed(s) && ensure_group(s, 0);
-	const float* s0 = packed && S > 0 ? s->sc[idx[0]] : nullptr;
-	launch_subtract_gradient(s->view(), from_advected ? s->adv : s->vel, s->p, s->vel, inv, st, packed ? s->grp.g[0] : nullptr, s0, buoy);
+	const float* src[4];
+	group_wants(s, 0, src);
+	launch_subtract_gradient(s->view(), from_advected ? s->adv : s->vel, s->p, s->vel, inv, st, packed ? s->grp[0].buf : nullptr,
+	                         packed ? src[3] : nullptr, buoy);
 	++s->vel_version;
-	if (packed) s->grp0_vel_version = s->vel_version, s->grp0_sc_version = s->sc_version, s->grp0_s0 = s0;
+	if (packed) group_written(s, 0, src);
 	return HNS_OK;
 }
 static int stage_advect_scalars(hns_state* s, float dt, float inv, int sampler_semantics, cudaStream_t st) {
@@ -182,15 +193,16 @@ static int stage_advect_scalars(hns_state* s, float dt, float inv, int sampler_s
 	if (!S || !s->n) return HNS_OK;
 	ScalarPtrs sp{};
 	for (int k = 0; k < S; ++k) sp.in[k] = s->sc[idx[k]], sp.out[k] = s->sc_out[idx[k]];
-	unsigned valid = 0;
-	if (groups_allowed(s)) {
-		if (s->grp.g[0] && s->grp0_vel_version == s->vel_version && s->grp0_sc_version == s->sc_version && s->grp0_s0 == sp.in[0]) valid |= 1u;
-		bool g1 = S > 1 && S <= 5 && s->grp.g[1] && s->grp1_sc_version == s->sc_version;
-		for (int c = 0; g1 && c < 4; ++c) g1 = s->grp1_src[c] == sp.in[1 + c];
-		if (g1) valid |= 2u;
+	// the packed kernels move one scalar (group 0) or five (groups 0 and 1)
+	const int n_groups = S == 1 ? 1 : S == 5 ? 2 : 0;
+	const float4* grp[2] = {};
+	bool packed = n_groups > 0;
+	for (int j = 0; j < n_groups; ++j) {
+		const float* want[4];
+		group_wants(s, j, want);
+		packed &= (grp[j] = group_if_current(s, j, want)) != nullptr;
 	}
-	s->grp.valid = valid;
-	launch_advect_scalars(s->view(), s->vel, sp, S, dt, inv, sampler_semantics, st, s->collision_sdf(), s->cold, valid ? &s->grp : nullptr);
+	launch_advect_scalars(s->view(), s->vel, sp, S, dt, inv, sampler_semantics, st, s->collision_sdf(), s->cold, packed ? grp : nullptr);
 	for (int k = 0; k < S; ++k) std::swap(s->sc[idx[k]], s->sc_out[idx[k]]);
 	++s->sc_version;
 	return HNS_OK;
@@ -255,7 +267,7 @@ static bool fused_combustion_enabled() {
 // buoyancy force into the gradient pass. Same arithmetic on the same values. Only for the frame on resident fields (no collision data,
 // no work list) whose advect_vector takes the packed path and whose advect_scalars finds the combustion fields as group 1.
 static bool fused_combustion(hns_state* s, const FrameDeps* deps) {
-	if (deps || !s->comb_enabled || s->active || !fused_combustion_enabled() || !combustion_packs(s) || !group0_current(s) || !ensure_group(s, 1))
+	if (deps || !s->comb_enabled || s->active || !fused_combustion_enabled() || !combustion_packs(s) || !velocity_group(s) || !ensure_group(s, 1))
 		return false;
 	if (!s->burn && cudaMalloc(&s->burn, s->n * sizeof(float)) != cudaSuccess) {
 		cudaGetLastError();
@@ -273,7 +285,7 @@ static int frame(hns_state* s, int iterations, float dt, float voxel_size, unsig
 	if (fused) {
 		const int* ci = s->comb_idx;
 		const CombustionJob job{{s->sc[ci[0]], s->sc[ci[1]], s->sc[ci[2]], s->sc[ci[3]]},
-		                        {s->sc_out[ci[0]], s->sc_out[ci[1]], s->sc_out[ci[2]], s->sc_out[ci[3]]}, s->grp.g[1], s->burn,
+		                        {s->sc_out[ci[0]], s->sc_out[ci[1]], s->sc_out[ci[2]], s->sc_out[ci[3]]}, s->grp[1].buf, s->burn,
 		                        s->comb.temperatureRelease};
 		stage_advect_velocity(s, dt, inv, st, &job);
 		combustion_swap(s, true);
@@ -330,14 +342,31 @@ static int frame(hns_state* s, int iterations, float dt, float voxel_size, unsig
 	}
 	if (deps && deps->scalar_inputs) HNS_CUDA(cudaStreamWaitEvent(st, deps->scalar_inputs, 0));
 	if (split_combustion && !sdf && groups_allowed(s) && ensure_group(s, 0)) {
-		int idx[16];
-		const float* s0 = advect_list(s, idx) > 0 ? s->sc[idx[0]] : nullptr;
-		launch_pack4(s->vel[0], s->vel[1], s->vel[2], s0, s->grp.g[0], s->n, st);  // 0.2 ms behind 40 ms of transfers
-		s->grp0_vel_version = s->vel_version, s->grp0_sc_version = s->sc_version, s->grp0_s0 = s0;
+		const float* src[4];
+		group_wants(s, 0, src);
+		launch_pack4(src[0], src[1], src[2], src[3], s->grp[0].buf, s->n, st);  // 0.2 ms behind 40 ms of transfers
+		group_written(s, 0, src);
 	}
 	stage_advect_scalars(s, dt, inv, 0, st);
 	HNS_CUDA(cudaGetLastError());
 	return HNS_OK;
+}
+
+// field ids of the ghost-exchange interface: 0..2 velocity, 3..5 advected velocity, 6/7 pressure red/black, 8/9 divergence red/black,
+// 10+i scalar i. Pressure and divergence halves hold 256 floats per leaf, everything else 512.
+float* field_ptr(hns_state* s, int field, int* floats_per_leaf) {
+	*floats_per_leaf = (field >= 6 && field <= 9) ? 256 : 512;
+	if (field >= 0 && field < 3) return s->vel[field];
+	if (field >= 3 && field < 6) return s->adv[field - 3];
+	if (field == 6 || field == 7) return s->p[field - 6];
+	if (field == 8 || field == 9) return s->div[field - 8];
+	if (field >= 10 && field < 10 + s->n_scalars) return s->sc[field - 10];
+	if (field == 26) return s->vort[3];  // |curl| plane of the vorticity confinement (null until first used)
+	return nullptr;
+}
+void field_written(hns_state* s, int field) {
+	if (field >= 0 && field < 3) ++s->vel_version;
+	if (field >= 10) ++s->sc_version;
 }
 
 }  // namespace hns
@@ -415,7 +444,7 @@ void hns_state_destroy(hns_state* s) {
 	for (int i = 0; i < 16; ++i) cudaFree(s->sc[i]), cudaFree(s->sc_out[i]);
 	cudaFree(s->aos);
 	cudaFree(s->cold);
-	for (float4* q : s->grp.g) cudaFree(q);
+	for (const PackedGroup& g : s->grp) cudaFree(g.buf);
 	cudaFree(s->burn);
 	cudaFree(s->d_sums);
 	if (s->solve_graph.exec) cudaGraphExecDestroy(s->solve_graph.exec);
@@ -631,8 +660,9 @@ int hns_state_time_frames(hns_state* s, int frames, int iterations, float dt, un
 		// alike (every timed frame pays for that second copy in its own gradient pass). The restored input stands in for that velocity,
 		// so it is packed here, outside the events, like the restore copies themselves.
 		if (groups_allowed(s) && ensure_group(s, 0)) {
-			launch_pack4(s->vel[0], s->vel[1], s->vel[2], nullptr, s->grp.g[0], s->n, st);
-			s->grp0_vel_version = s->vel_version, s->grp0_sc_version = 0, s->grp0_s0 = nullptr;
+			const float* const src[4] = {s->vel[0], s->vel[1], s->vel[2], nullptr};
+			launch_pack4(src[0], src[1], src[2], src[3], s->grp[0].buf, s->n, st);
+			group_written(s, 0, src);
 		}
 		cudaEventRecord(ev[4 * f + 0], st);
 		rc = frame(s, iterations, dt, s->grid->voxel_size, flags, st, ev[4 * f + 1], ev[4 * f + 2]);
@@ -656,23 +686,11 @@ int hns_state_time_frames(hns_state* s, int frames, int iterations, float dt, un
 	return HNS_OK;
 }
 
-// field ids of the ghost-exchange interface: 0..2 velocity, 3..5 advected velocity, 6/7 pressure red/black, 8/9 divergence red/black,
-// 10+i scalar i. Pressure and divergence halves hold 256 floats per leaf, everything else 512.
-static float* field_ptr(hns_state* s, int field, int* floats_per_leaf) {
-	*floats_per_leaf = (field >= 6 && field <= 9) ? 256 : 512;
-	if (field >= 0 && field < 3) return s->vel[field];
-	if (field >= 3 && field < 6) return s->adv[field - 3];
-	if (field == 6 || field == 7) return s->p[field - 6];
-	if (field == 8 || field == 9) return s->div[field - 8];
-	if (field >= 10 && field < 10 + s->n_scalars) return s->sc[field - 10];
-	if (field == 26) return s->vort[3];  // |curl| plane of the vorticity confinement (null until first used)
-	return nullptr;
-}
 void* hns_state_field_device_ptr(hns_state* s, int field) {
+	if (!s) return nullptr;
+	field_written(s, field);  // the caller may write through the pointer
 	int fpl;
-	if (s && field >= 0 && field < 3) ++s->vel_version;  // the caller may write through the pointer
-	if (s && field >= 10) ++s->sc_version;
-	return s ? field_ptr(s, field, &fpl) : nullptr;
+	return field_ptr(s, field, &fpl);
 }
 int hns_state_field_floats_per_leaf(int field) { return (field >= 6 && field <= 9) ? 256 : 512; }
 int hns_state_pack_leaves(hns_state* s, int field, const int32_t* ids, uint64_t n_ids, float* dst, void* stream) {
@@ -689,8 +707,7 @@ int hns_state_unpack_leaves(hns_state* s, int field, const int32_t* ids, uint64_
 	int fpl;
 	float* f = field_ptr(s, field, &fpl);
 	HNS_REQUIRE(f, "bad field id");
-	if (field < 3) ++s->vel_version;
-	if (field >= 10) ++s->sc_version;
+	field_written(s, field);
 	launch_unpack_leaves(f, ids, n_ids, src, fpl, static_cast<cudaStream_t>(stream));
 	HNS_CUDA(cudaGetLastError());
 	return HNS_OK;

@@ -69,11 +69,12 @@ struct GridView {
 #endif
 };
 
-// packed field groups of the advection kernels (kernels.cuh, advect.cu)
-struct AdvectGroups {
-	float4* g[5] = {};
-	unsigned valid = 0;
-	uint64_t n = 0;  // voxels per group
+// A packed float4 group of the advection kernels (kernels.cuh, advect.cu; api.cu, "packed groups"): lane k mirrors the brick field
+// src[k] (null: the lane holds 0) as it was when the state's version counters stood at vel_version / sc_version.
+struct PackedGroup {
+	float4* buf = nullptr;  // float4[n], allocated on first use
+	const float* src[4] = {};
+	uint64_t vel_version = 0, sc_version = 0;
 };
 
 // slot ids of the six face neighbours
@@ -108,14 +109,13 @@ __device__ __forceinline__ int probe_leaf(const GridView& g, int x, int y, int z
 struct hns_mg;
 struct hns_state;
 namespace hns {
-// packed advection groups in a sharded frame (api.cu): which groups the kernels of this frame have written for the owned leaves, and
-// -- after the ghost exchange that precedes the advection pass -- the same for the listed (ghost) leaves, from the brick fields
-struct GroupsCurrent {
-	bool g0 = false, g1 = false;
-};
-GroupsCurrent groups_current(const hns_state* s);
-int groups_refresh_leaves(hns_state* s, const int32_t* ids, uint64_t n_ids, GroupsCurrent which, cudaStream_t st);
-void groups_stamp(hns_state* s, GroupsCurrent which);
+// ghost-exchange fields of a state (api.cu; ids as for hns_state_pack_leaves): the device pointer, or null for a bad id
+float* field_ptr(hns_state* s, int field, int* floats_per_leaf);
+void field_written(hns_state* s, int field);  // bumps the version counter a write into `field` invalidates
+// packed advection groups (api.cu, "packed groups")
+void group_wants(const hns_state* s, int j, const float* want[4]);
+const float4* group_if_current(const hns_state* s, int j, const float* const want[4]);
+void group_written(hns_state* s, int j, const float* const src[4]);
 int mg_pressure_solve(hns_state* s, hns_mg* mg, int max_cycles, double rel_tol, int nu_pre, int nu_post, float omega, cudaStream_t st);  // multigrid.cu
 void mg_coarse_cycle(hns_mg* mg, float* const rhs1[2], int nu_pre, int nu_post, float omega, cudaStream_t st);
 cudaGraphExec_t mg_capture_coarse(hns_mg* mg, float* const rhs1[2], int nu_pre, int nu_post, float omega, uint64_t* launches);
@@ -185,13 +185,9 @@ struct hns_state {
 	float* sc_out[16] = {};
 	float* aos = nullptr; // staging float[N][3] for host <-> device velocity transfers
 	uint8_t* cold = nullptr;  // [L] leaf flags of the advection kernels (advect.cu), zero between launches
-	// packed groups the advection kernels stage from, allocated on first use, and what they were built from (api.cu, "packed groups")
-	hns::AdvectGroups grp;
+	// the packed groups the advection kernels stage from: {u, v, w, first advected scalar} and {fuel, waste, temperature, flame}
+	hns::PackedGroup grp[2];
 	uint64_t sc_version = 1;  // bumped by every entry point that (may) overwrite a scalar field, like vel_version for the velocity
-	uint64_t grp0_vel_version = 0, grp0_sc_version = 0, grp1_sc_version = 0;  // 0 never matches: the counters start at 1
-	const float* grp0_s0 = nullptr;                                          // the scalar buffer in group 0's fourth lane
-	const float* grp1_src[4] = {nullptr, nullptr, nullptr, nullptr};         // the buffers group 1 mirrors
-	bool grp_dist = false;  // a sharded frame (dist.cu) re-packs the ghost leaves of the groups after its exchanges
 	float* burn = nullptr;  // float[n], allocated on first use: combustion's burn per voxel from advect_vector to the divergence (api.cu, frame)
 	float* vort[4] = {nullptr, nullptr, nullptr, nullptr};  // vorticity confinement scratch, allocated on first use: output planes u, v, w and |curl|
 	// optional combustion + buoyancy stage of the all-in-one frame

@@ -223,8 +223,6 @@ __global__ void k_advance_bases(uint32_t* base, uint32_t iterations) {
 }
 }  // namespace hns
 
-static int floats_per_leaf(int field) { return (field >= 6 && field <= 9) ? 256 : 512; }
-
 extern "C" {
 
 int hns_dist_unique_id(uint8_t* out128) {
@@ -542,8 +540,8 @@ static int exchange_p2p(hns_dist* d, hns_state* s, int channel, int n_fields, co
 		if (!p.n_send) continue;
 		float* dst = reinterpret_cast<float*>(p.remote_region + channel_offset(region_ch, p.n_send, S)) + uint64_t(skip_fields) * 512u * p.n_send;
 		for (int k = 0; k < n_fields; ++k) {
-			const int fpl = floats_per_leaf(fields[k]);
-			float* f = static_cast<float*>(hns_state_field_device_ptr(s, fields[k]));
+			int fpl;
+			const float* f = field_ptr(s, fields[k], &fpl);
 			if (!f) return fail(HNS_ERR_INVALID_ARGUMENT, "bad field id");
 			launch_pack_leaves(f, p.d_send, p.n_send, dst, fpl, st, max_blocks);
 			dst += p.n_send * fpl;
@@ -558,8 +556,9 @@ static int exchange_p2p(hns_dist* d, hns_state* s, int channel, int n_fields, co
 		if (!p.n_recv) continue;
 		const float* src = reinterpret_cast<const float*>(d->block + p.region_off + channel_offset(region_ch, p.n_recv, S)) + uint64_t(skip_fields) * 512u * p.n_recv;
 		for (int k = 0; k < n_fields; ++k) {
-			const int fpl = floats_per_leaf(fields[k]);
-			float* f = static_cast<float*>(hns_state_field_device_ptr(s, fields[k]));
+			int fpl;
+			float* f = field_ptr(s, fields[k], &fpl);
+			field_written(s, fields[k]);
 			launch_unpack_leaves(f, p.d_recv, p.n_recv, src, fpl, st, max_blocks);
 			src += p.n_recv * fpl;
 		}
@@ -578,20 +577,23 @@ int hns_dist_exchange(hns_dist* d, hns_state* s, int n_fields, const int* fields
 	if (!d->comm && d->world > 1) return fail(HNS_ERR_RUNTIME, "no NCCL communicator (hns_dist_create without an id) and the peer-memory exchange is not connected");
 	if (d->peers.empty()) return HNS_OK;  // a single rank (or one that shares no leaf): nothing to send or receive
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
+	float* f[3 + 16];  // n_fields <= max_fields = 3 + n_scalars
+	int fpl[3 + 16];
+	uint64_t leaf_floats = 0;  // of all the fields
+	for (int k = 0; k < n_fields; ++k) {
+		if (!(f[k] = field_ptr(s, fields[k], &fpl[k]))) return fail(HNS_ERR_INVALID_ARGUMENT, "bad field id");
+		leaf_floats += fpl[k];
+	}
 	for (auto& p : d->peers) {
 		uint64_t off = 0;
 		for (int k = 0; k < n_fields && p.n_send; ++k) {
-			const int fpl = floats_per_leaf(fields[k]);
-			float* f = static_cast<float*>(hns_state_field_device_ptr(s, fields[k]));
-			if (!f) return fail(HNS_ERR_INVALID_ARGUMENT, "bad field id");
-			launch_pack_leaves(f, p.d_send, p.n_send, p.buf_send + off, fpl, st);
-			off += p.n_send * fpl;
+			launch_pack_leaves(f[k], p.d_send, p.n_send, p.buf_send + off, fpl[k], st);
+			off += p.n_send * fpl[k];
 		}
 	}
 	HNS_NCCL(g_nccl.GroupStart());
 	for (auto& p : d->peers) {
-		uint64_t cs = 0, cr = 0;
-		for (int k = 0; k < n_fields; ++k) cs += p.n_send * floats_per_leaf(fields[k]), cr += p.n_recv * floats_per_leaf(fields[k]);
+		const uint64_t cs = p.n_send * leaf_floats, cr = p.n_recv * leaf_floats;
 		if (cs) HNS_NCCL(g_nccl.Send(p.buf_send, cs, ncclFloat, p.rank, d->comm, st));
 		if (cr) HNS_NCCL(g_nccl.Recv(p.buf_recv, cr, ncclFloat, p.rank, d->comm, st));
 		d->bytes_sent += cs * 4;
@@ -600,10 +602,9 @@ int hns_dist_exchange(hns_dist* d, hns_state* s, int n_fields, const int* fields
 	for (auto& p : d->peers) {
 		uint64_t off = 0;
 		for (int k = 0; k < n_fields && p.n_recv; ++k) {
-			const int fpl = floats_per_leaf(fields[k]);
-			float* f = static_cast<float*>(hns_state_field_device_ptr(s, fields[k]));
-			launch_unpack_leaves(f, p.d_recv, p.n_recv, p.buf_recv + off, fpl, st);
-			off += p.n_recv * fpl;
+			field_written(s, fields[k]);
+			launch_unpack_leaves(f[k], p.d_recv, p.n_recv, p.buf_recv + off, fpl[k], st);
+			off += p.n_recv * fpl[k];
 		}
 	}
 	++d->exchanges;
@@ -852,7 +853,6 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 	mark();
 	const int fvel[3] = {0, 1, 2}, fadv[3] = {3, 4, 5};
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	s->grp_dist = true;  // this frame re-packs the ghost leaves of the packed advection groups itself (below)
 	if (s->skip_scalar >= 0 && s->skip_scalar != s->n_scalars - 1)
 		return fail(HNS_ERR_UNSUPPORTED, "sharded frames need the non-advected scalar (collision_sdf) to be the last scalar field");
 	// collision path: enforceCollisionBoundaries and the collision tests of advect_vector read the SDF in ghost leaves (neighbour rows
@@ -899,8 +899,10 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 	// Packed advection groups (api.cu): the combustion pass has just written group 1 for every voxel, the gradient pass below writes
 	// group 0 for the owned leaves; the exchanges that follow refresh the ghost leaves of the brick fields only (and bump the version
 	// counters), so what is current now is noted here and the groups' ghost leaves are re-packed in front of advect_scalars.
-	GroupsCurrent packed;
-	packed.g1 = groups_current(s).g1;
+	const float* want[2][4];
+	bool packed[2];
+	group_wants(s, 1, want[1]);
+	packed[1] = group_if_current(s, 1, want[1]) != nullptr;
 	if (deps && deps->scalar_inputs) HNS_CUDA(cudaStreamWaitEvent(st, deps->scalar_inputs, 0));
 	// The scalars are final until advect_scalars: exchange their ghosts now, on a third stream, behind the pressure solve.
 	const bool scalars_early = d->p2p && s->n_scalars > 0;
@@ -927,7 +929,8 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 	mark();
 	if ((rc = hns_state_subtract_gradient(s, 1, stream))) return rc;
 	if (hns_state_collision_active(s) && (rc = hns_state_enforce_collision(s, stream))) return rc;  // HNanoSolver.cu:292-296
-	packed.g0 = groups_current(s).g0;
+	group_wants(s, 0, want[0]);
+	packed[0] = group_if_current(s, 0, want[0]) != nullptr;
 	mark();
 	std::vector<int> last = {0, 1, 2};
 	if (!scalars_early)
@@ -938,11 +941,11 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 		HNS_CUDA(cudaEventRecord(deps->velocity_done, st));
 	}
 	if (scalars_early) HNS_CUDA(cudaStreamWaitEvent(st, d->ev_scalars_exchanged, 0));
-	if (packed.g0 || packed.g1) {
-		for (auto& p : d->peers)
-			if (p.n_recv && (rc = groups_refresh_leaves(s, p.d_recv, p.n_recv, packed, st))) return rc;
-		groups_stamp(s, packed);
-	}
+	for (auto& p : d->peers)
+		for (int j = 0; j < 2; ++j)
+			if (packed[j]) launch_pack4_leaves(p.d_recv, p.n_recv, want[j][0], want[j][1], want[j][2], want[j][3], s->grp[j].buf, st);
+	for (int j = 0; j < 2; ++j)
+		if (packed[j]) group_written(s, j, want[j]);
 	// advect_scalars' "inactive -> element 0" value (reference Kernel.cu:192,225) is global voxel 0's = local voxel 0's: that exchange
 	// has just refreshed it on every rank
 	mark();

@@ -16,9 +16,9 @@ void launch_aos_to_soa(const float* aos, float* u, float* v, float* w, uint64_t 
 void launch_soa_to_aos(const float* u, const float* v, const float* w, float* aos, uint64_t n, cudaStream_t st);
 
 // Packed groups of the advection kernels (advect.cu, third generation): float4[n] per group in brick voxel order, group 0 =
-// {u, v, w, first advected scalar}, group j >= 1 = {scalar 4j-3 .. 4j} of the list handed to launch_advect_scalars. Scratch owned by the
-// caller; bit j of `valid` says the producer of those fields already wrote the group, otherwise the launcher packs it first
-// (struct AdvectGroups, common.cuh).
+// {u, v, w, first advected scalar}, group 1 = {scalars 1..4} of the list handed to launch_advect_scalars. Owned and kept current by
+// the caller (struct PackedGroup, common.cuh; api.cu, "packed groups"): the launchers run the packed kernels exactly when they are
+// handed groups, and never pack one themselves.
 void launch_pack4(const float* a, const float* b, const float* c, const float* d, float4* out, uint64_t n, cudaStream_t st);
 void launch_pack4_leaves(const int32_t* ids, uint64_t n_ids, const float* a, const float* b, const float* c, const float* d, float4* out,
                          cudaStream_t st);
@@ -63,16 +63,17 @@ __device__ __forceinline__ float combustion_voxel(const float4 in, float temp_ga
 // advect_vector (reference src/Cuda/Kernel.cu:354-453)
 // cold: device uint8[num_leaves of the grid], zero between launches -- scratch in which the staged kernel flags the leaves whose samples
 // left its shared-memory region; a follow-up kernel redoes those leaves through the neighbour table and clears the flags (advect.cu)
-// comb: the staged kernel also runs combustion_oxygen on every voxel of the grid; honoured on the packed path without sdf only (group 0
-// current, packed advection on), which the caller checks (api.cu, frame)
+// sdf != null: the hasCollision variant incl. its boundary tail; second generation only
+// grp0 != null: the third generation, staging from packed group 0 (it holds this velocity; needs sdf == null)
+// comb: the staged kernel also runs combustion_oxygen on every voxel of the grid (needs grp0)
 void launch_advect_vector(const GridView& g, const float* const vel[3], float* const out[3], float dt, float inv_dx, cudaStream_t st,
-                          const float* sdf, uint8_t* cold, const AdvectGroups* grp = nullptr,  // sdf != null: the hasCollision variant incl. its boundary tail
-                          const CombustionJob* comb = nullptr);
+                          const float* sdf, uint8_t* cold, const float4* grp0 = nullptr, const CombustionJob* comb = nullptr);
 
 // advect_scalars (Kernel.cu:118-266) when sampler_semantics == 0; advect_scalar (Kernel.cu:269-352) per field when == 1
 // advect_scalars reads element 0 of the arrays passed in for inactive voxels (a shard's local leaf 0 is global leaf 0, dist.py::make_plan)
+// grp != null: the third generation, staging from packed groups 0 (S == 1) or 0 and 1 (S == 5) of these fields; needs sdf == null
 void launch_advect_scalars(const GridView& g, const float* const vel[3], const ScalarPtrs& sp, int S, float dt, float inv_dx,
-                           int sampler_semantics, cudaStream_t st, const float* sdf, uint8_t* cold, const AdvectGroups* grp = nullptr);
+                           int sampler_semantics, cudaStream_t st, const float* sdf, uint8_t* cold, const float4* const grp[2] = nullptr);
 // enforceCollisionBoundaries (Kernel.cu:77-116; blend_divisor 0.1, mixed_sum 0) and the boundary tails of advect_vector (:432-450;
 // 1.5, 1) and subtractPressureGradient (:808-826; 0.1, 0): vel -> out (may alias), per voxel
 void launch_collision_boundary(const GridView& g, const float* const vel[3], float* const out[3], const float* sdf, float inv_dx,
