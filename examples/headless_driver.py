@@ -6,6 +6,9 @@ build the sidecar, CreateIndexGrid once per topology, then one Compute_Sim per f
 Two ways to run a frame are shown side by side and must agree bit for bit:
   * the drop-in launchers on HOST buffers (CreateIndexGrid + Compute_Sim), every frame crossing PCIe like the reference does, and
   * the resident state (Simulation.step), which keeps the fields in HBM between frames.
+An emitter at the plume's base (density, temperature and fuel sources and an upward velocity source, as NanoVDB grids) is added in
+front of every frame, as the SOP does with compSum (SOP_HNanoSolver.cpp:159-181): on the host blocks with io.comp_sum, on the
+resident state with Simulation.add_source. The domain stays fixed: the emitter's leaves outside it are dropped.
 With an output directory the last frame is written as a NanoVDB file + sidecar blocks (hnanosolver_b200.io) and read back.
 """
 import os
@@ -48,13 +51,23 @@ sim.upload(w.velocity, list(fields.values()))
 sim.set_combustion(True, names.index("fuel"), names.index("waste"), names.index("temperature"), names.index("flame"), params)
 sim.set_collision(names.index("collision_sdf"))
 
+# ---- emitter: 2 % of the leaves at the plume's base and four leaves outside the domain ----
+src_origins, src_values = synth.emitter(w.origins, fraction=0.02, speed=0.2 * float(np.abs(w.velocity).max()))
+emitter = {k: hio.grid_from_sidecar(src_origins, v, w.voxel_size, k) for k, v in src_values.items()}
+host_sources = [("vel" if k == "velocity" else k, buf) for k, buf in emitter.items()]
+device_sources = [("velocity" if k == "velocity" else names.index(k), H.Source(buf)) for k, buf in emitter.items()]
+print(f"emitter: {len(src_origins)} leaves, {device_sources[0][1].leaves_outside(grid)} of them outside the domain (dropped)")
+
 t_host = t_dev = 0.0
 for f in range(frames):
     sdf = fields["collision_sdf"]
     data.pValues(H.FLOAT, "collision_sdf")[:] = sdf            # the launcher hands the SDF block back zeroed, like the reference
     t0 = time.perf_counter()
+    hio.comp_sum(w.origins, data, host_sources)
     H.Compute_Sim(data, grid, iterations, w.dt, w.voxel_size, params, True)
     t1 = time.perf_counter()
+    for target, src in device_sources:
+        sim.add_source(target, src)
     sim.step(iterations, w.dt)
     sim.sync()
     t2 = time.perf_counter()
@@ -66,7 +79,7 @@ for f in range(frames):
           f"max temperature {data.pValues(H.FLOAT, 'temperature').max():.4f}  host-buffer path == resident path: {same}", flush=True)
     assert same
 print(f"{w.num_leaves} leaves, {w.num_voxels} voxels, {iterations} pressure iterations: {t_host / frames * 1e3:.2f} ms per frame through the "
-      f"launchers on host buffers, {t_dev / frames * 1e3:.2f} ms per frame on resident state")
+      f"launchers on host buffers (sourcing on the host included), {t_dev / frames * 1e3:.2f} ms per frame on resident state")
 
 if out_dir:
     hio.save_cache(out_dir, grid.nanovdb_buffer(), data)

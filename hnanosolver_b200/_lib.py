@@ -73,6 +73,13 @@ SIGNATURES = {
     "hns_state_upload_scalar": (C.c_int, [C.c_void_p, C.c_int, c_f32p]),
     "hns_state_download_scalar": (C.c_int, [C.c_void_p, C.c_int, c_f32p]),
     "hns_state_download_aux": (C.c_int, [C.c_void_p, C.c_int, c_f32p]),
+    "hns_source_create": (C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]),
+    "hns_source_destroy": (None, [C.c_void_p]),
+    "hns_source_components": (C.c_int, [C.c_void_p]),
+    "hns_source_num_leaves": (C.c_uint64, [C.c_void_p]),
+    "hns_source_leaves_outside": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]),
+    "hns_state_add_source_velocity": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "hns_state_add_source_scalar": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "hns_state_set_combustion": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(CombustionParams)]),
     "hns_state_step": (C.c_int, [C.c_void_p, C.c_int, C.c_float, C.c_uint, C.c_void_p]),
     "hns_state_advect_velocity": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p]),

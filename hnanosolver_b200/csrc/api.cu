@@ -487,6 +487,78 @@ int hns_state_download_scalar(hns_state* s, int i, float* host) {
 	HNS_CUDA(cudaMemcpy(host, s->sc[i], s->n * 4, cudaMemcpyDeviceToHost));
 	return HNS_OK;
 }
+// ---- sources (compSum into resident fields) -----------------------------------------------------------------------
+int hns_source_create(const void* buffer, uint64_t bytes, hns_source** out) {
+	HNS_REQUIRE(out, "null argument");
+	*out = nullptr;
+	SourceTables t;
+	int rc = source_tables(buffer, bytes, t);  // every refusal of a malformed buffer happens here, before any CUDA call
+	if (rc) return rc;
+	auto* src = new hns_source();
+	src->components = t.components;
+	src->num_leaves = t.keys.size();
+	const uint64_t L = src->num_leaves;
+	cudaError_t e = cudaGetDevice(&src->device);
+	if (e == cudaSuccess && L) {
+		if ((e = cudaMalloc(&src->keys, L * sizeof(ulonglong2))) == cudaSuccess && (e = cudaMalloc(&src->origins, L * sizeof(int4))) == cudaSuccess &&
+		    (e = cudaMalloc(&src->values, t.values.size() * sizeof(float))) == cudaSuccess &&
+		    (e = cudaMemcpy(src->keys, t.keys.data(), L * sizeof(ulonglong2), cudaMemcpyHostToDevice)) == cudaSuccess &&
+		    (e = cudaMemcpy(src->origins, t.origins.data(), L * sizeof(int4), cudaMemcpyHostToDevice)) == cudaSuccess)
+			e = cudaMemcpy(src->values, t.values.data(), t.values.size() * sizeof(float), cudaMemcpyHostToDevice);
+	}
+	if (e != cudaSuccess) {
+		hns_source_destroy(src);
+		return fail(HNS_ERR_CUDA, std::string("hns_source_create: ") + cudaGetErrorString(e));
+	}
+	*out = src;
+	return HNS_OK;
+}
+void hns_source_destroy(hns_source* src) {
+	if (!src) return;
+	cudaFree(src->keys), cudaFree(src->origins), cudaFree(src->values);
+	delete src;
+}
+int hns_source_components(const hns_source* src) { return src ? src->components : 0; }
+uint64_t hns_source_num_leaves(const hns_source* src) { return src ? src->num_leaves : 0; }
+int hns_source_leaves_outside(const hns_source* src, const hns_grid* g, uint64_t* out) {
+	HNS_REQUIRE(src && g && out, "null argument");
+	HNS_REQUIRE(src->device == g->device, "the source and the grid live on different devices");
+	*out = 0;
+	if (!src->num_leaves) return HNS_OK;
+	unsigned long long* d_count = nullptr;
+	HNS_CUDA(cudaMalloc(&d_count, sizeof(*d_count)));
+	cudaMemset(d_count, 0, sizeof(*d_count));
+	launch_count_leaves_outside(g->view, *src, d_count, 0);
+	unsigned long long n = 0;
+	const cudaError_t e = cudaMemcpy(&n, d_count, sizeof(n), cudaMemcpyDeviceToHost);
+	cudaFree(d_count);
+	HNS_CUDA(e);
+	*out = n;
+	return HNS_OK;
+}
+// The add covers every leaf of the state's grid, ghost leaves of a shard included (the work list is ignored): a rank computes the same
+// bits for a ghost leaf as its owner, without an exchange. The version counters move as for any other write, so the packed advection
+// groups ("packed groups" above) stop mirroring what was sourced.
+static int add_source(hns_state* s, const hns_source* src, float* const field[3], int field_id, void* stream) {
+	HNS_REQUIRE(src->device == s->grid->device, "the source lives on another device than the state");
+	launch_add_source(s->grid->view, *src, field, static_cast<cudaStream_t>(stream));
+	field_written(s, field_id);
+	HNS_CUDA(cudaGetLastError());
+	return HNS_OK;
+}
+int hns_state_add_source_velocity(hns_state* s, const hns_source* src, void* stream) {
+	HNS_REQUIRE(s && src, "null argument");
+	HNS_REQUIRE(src->components == 3, "the velocity takes a Vec3f source");
+	return add_source(s, src, s->vel, 0, stream);
+}
+int hns_state_add_source_scalar(hns_state* s, int index, const hns_source* src, void* stream) {
+	HNS_REQUIRE(s && src, "null argument");
+	HNS_REQUIRE(index >= 0 && index < s->n_scalars, "scalar index out of range");
+	HNS_REQUIRE(src->components == 1, "a scalar field takes a float source");
+	float* const field[3] = {s->sc[index], nullptr, nullptr};
+	return add_source(s, src, field, 10 + index, stream);
+}
+
 int hns_state_download_aux(hns_state* s, int which, float* host) {
 	HNS_REQUIRE(s && host, "null argument");
 	if (which == 0 || which == 1) {

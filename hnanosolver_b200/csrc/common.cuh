@@ -80,6 +80,27 @@ struct PackedGroup {
 // slot ids of the six face neighbours
 constexpr int kSlotXm = 4, kSlotXp = 22, kSlotYm = 10, kSlotYp = 16, kSlotZm = 12, kSlotZp = 14, kSlotSelf = 13;
 
+// Position of leaf origin (x, y, z) in NanoVDB's leaf order as a pair compared lexicographically: x = the root tile key with the sign
+// bias that makes it increase with signed coordinates, y = upper-node offset << 12 | lower-node offset.
+__host__ __device__ inline ulonglong2 nvdb_leaf_key(int32_t x, int32_t y, int32_t z) {
+	const uint64_t bx = uint32_t(x) ^ 0x80000000u, by = uint32_t(y) ^ 0x80000000u, bz = uint32_t(z) ^ 0x80000000u;
+	const uint64_t tile = (bz >> 12) | (by >> 12) << 21 | (bx >> 12) << 42;
+	const uint64_t node = uint64_t(((x & 4095) >> 7) << 10 | ((y & 4095) >> 7) << 5 | ((z & 4095) >> 7)) << 12 |
+	                      uint64_t(((x & 127) >> 3) << 8 | ((y & 127) >> 3) << 4 | ((z & 127) >> 3));
+	return make_ulonglong2(tile, node);
+}
+__host__ __device__ inline bool key_less(const ulonglong2& a, const ulonglong2& b) { return a.x < b.x || (a.x == b.x && a.y < b.y); }
+
+// A source grid's leaves on the host, validated and sorted by nvdb_leaf_key (nvdb_io.cu, source_tables): what hns_source_create copies
+// to the device. values: float[L][512 * components], each leaf's 512 values as the grid stores them (Vec3f: AoS).
+struct SourceTables {
+	int components = 0;
+	std::vector<ulonglong2> keys;
+	std::vector<int4> origins;  // (x, y, z, 0)
+	std::vector<float> values;
+};
+int source_tables(const void* buffer, uint64_t bytes, SourceTables& out);
+
 #ifdef __CUDACC__
 // Leaf ordinal containing voxel (x,y,z), or -1: the ReadAccessor walk (root tile scan -> upper -> lower) on the emitted buffer.
 __device__ __forceinline__ int probe_leaf(const GridView& g, int x, int y, int z) {
@@ -223,4 +244,14 @@ struct hns_state {
 		v.list = active, v.num_list = n_active, v.far_flag = far_flag;
 		return v;
 	}
+};
+
+// a source grid on the device (hns_source_create): the host tables of source_tables, copied
+struct hns_source {
+	int device = 0;
+	int components = 0;
+	uint64_t num_leaves = 0;
+	ulonglong2* keys = nullptr;  // [L], ascending
+	int4* origins = nullptr;     // [L]
+	float* values = nullptr;     // [L][512 * components]
 };

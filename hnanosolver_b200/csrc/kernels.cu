@@ -1032,4 +1032,85 @@ void launch_unpack_leaves(float* field, const int32_t* ids, uint64_t n_ids, cons
 	HNS_LAUNCH(k_unpack_leaves, copy_grid(total, max_blocks), 256, 0, st, field, ids, src, total, qshift);
 }
 
+// =============================================================================================================
+// sourcing: openvdb::tools::compSum of a source grid into resident fields (reference SOP_HNanoSolver.cpp:159-181, io.comp_sum)
+// =============================================================================================================
+// Index of key t in keys[0..n) (ascending), or -1. The warp searches together, 32 probes per round: a million leaves take four rounds
+// of one dependent load each.
+__device__ __forceinline__ int find_key_warp(const ulonglong2* __restrict__ keys, uint32_t n, const ulonglong2 t, uint32_t lane) {
+	uint32_t lo = 0;
+	while (n > 32) {
+		const uint32_t step = (n + 31) / 32, i = lane * step;
+		const bool le = i < n && !key_less(t, __ldg(keys + lo + i));
+		const uint32_t c = __popc(__ballot_sync(0xffffffffu, le));  // the probes <= t are a prefix of the lanes
+		if (!c) return -1;
+		lo += (c - 1) * step;
+		n = min(step, n - (c - 1) * step);
+	}
+	bool hit = false;
+	if (lane < n) {
+		const ulonglong2 k = __ldg(keys + lo + lane);
+		hit = k.x == t.x && k.y == t.y;
+	}
+	const uint32_t b = __ballot_sync(0xffffffffu, hit);
+	return b ? int(lo + __ffs(b) - 1) : -1;
+}
+// One warp per leaf, eight leaves per CTA; lane t owns the voxel quads k * 32 + t (k = 0..3) of the leaf's 512 voxels. The field's loads
+// go out before the search, whose result only selects the source's quads: 8 B per voxel and plane, plus 4 B per voxel and component
+// where the source has the leaf. C = 3: the source is AoS, three float4 per quad of voxels, split into the three planes.
+template <int C>
+__global__ void __launch_bounds__(256) k_add_source(const int4* __restrict__ origin, uint32_t num_leaves, const ulonglong2* __restrict__ keys,
+                                                    uint32_t n_keys, const float* __restrict__ values, float* f0, float* f1, float* f2) {
+	const uint32_t leaf = blockIdx.x * 8u + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
+	if (leaf >= num_leaves) return;  // the whole warp
+	float4* const plane[3] = {reinterpret_cast<float4*>(f0) + uint64_t(leaf) * 128u, reinterpret_cast<float4*>(f1) + uint64_t(leaf) * 128u,
+	                          reinterpret_cast<float4*>(f2) + uint64_t(leaf) * 128u};
+	float4 v[C][4], s[C][4];
+#pragma unroll
+	for (int c = 0; c < C; ++c)
+#pragma unroll
+		for (int k = 0; k < 4; ++k) v[c][k] = plane[c][k * 32 + lane], s[c][k] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+	const int4 o = __ldg(origin + leaf);
+	const int j = find_key_warp(keys, n_keys, nvdb_leaf_key(o.x, o.y, o.z), lane);
+	if (j >= 0) {
+		const float4* src = reinterpret_cast<const float4*>(values) + uint64_t(j) * (128u * C);
+#pragma unroll
+		for (int k = 0; k < 4; ++k) {
+			const uint32_t q = k * 32 + lane;
+			if constexpr (C == 1) {
+				s[0][k] = __ldg(src + q);
+			} else {  // voxels 4q .. 4q+3: (x0 y0 z0 x1) (y1 z1 x2 y2) (z2 x3 y3 z3)
+				const float4 a = __ldg(src + 3 * q), b = __ldg(src + 3 * q + 1), d = __ldg(src + 3 * q + 2);
+				s[0][k] = make_float4(a.x, a.w, b.z, d.y);
+				s[1][k] = make_float4(a.y, b.x, b.w, d.z);
+				s[2][k] = make_float4(a.z, b.y, d.x, d.w);
+			}
+		}
+	}
+#pragma unroll
+	for (int c = 0; c < C; ++c)
+#pragma unroll
+		for (int k = 0; k < 4; ++k)
+			plane[c][k * 32 + lane] = make_float4(v[c][k].x + s[c][k].x, v[c][k].y + s[c][k].y, v[c][k].z + s[c][k].z, v[c][k].w + s[c][k].w);
+}
+void launch_add_source(const GridView& g, const hns_source& src, float* const field[3], cudaStream_t st) {
+	if (!g.num_leaves) return;
+	const unsigned blocks = (g.num_leaves + 7u) / 8u;
+	if (src.components == 3)
+		HNS_LAUNCH(k_add_source<3>, blocks, 256, 0, st, g.origin, g.num_leaves, src.keys, uint32_t(src.num_leaves), src.values, field[0], field[1], field[2]);
+	else
+		HNS_LAUNCH(k_add_source<1>, blocks, 256, 0, st, g.origin, g.num_leaves, src.keys, uint32_t(src.num_leaves), src.values, field[0], field[0], field[0]);
+}
+
+__global__ void __launch_bounds__(256) k_count_leaves_outside(GridView g, const int4* __restrict__ origins, uint32_t n, unsigned long long* count) {
+	const uint32_t i = blockIdx.x * 256u + threadIdx.x;
+	if (i >= n) return;
+	const int4 o = __ldg(origins + i);
+	if (probe_leaf(g, o.x, o.y, o.z) < 0) atomicAdd(count, 1ull);
+}
+void launch_count_leaves_outside(const GridView& g, const hns_source& src, unsigned long long* count, cudaStream_t st) {
+	if (src.num_leaves)
+		HNS_LAUNCH(k_count_leaves_outside, unsigned((src.num_leaves + 255) / 256), 256, 0, st, g, src.origins, uint32_t(src.num_leaves), count);
+}
+
 }  // namespace hns

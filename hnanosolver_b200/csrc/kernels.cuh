@@ -148,5 +148,11 @@ void launch_pack_leaves(const float* field, const int32_t* ids, uint64_t n_ids, 
 void launch_unpack_leaves(float* field, const int32_t* ids, uint64_t n_ids, const float* src, int floats_per_leaf, cudaStream_t st, int max_blocks = 0);
 // colour-split (red, black) -> brick order
 void launch_split_to_brick(const float* const f[2], float* out, uint64_t n, cudaStream_t st);
+// compSum of a source grid (struct hns_source: keys, values, components) into brick fields, field[0..components): every voxel of every
+// leaf of g -- its work list is ignored -- becomes value + s, s = the source's value where it has a leaf at that origin and +0.0f
+// elsewhere (which turns -0.0 into +0.0, as compSum against a background tile does)
+void launch_add_source(const GridView& g, const hns_source& src, float* const field[3], cudaStream_t st);
+// adds to *count the source leaves whose origin is not a leaf of g
+void launch_count_leaves_outside(const GridView& g, const hns_source& src, unsigned long long* count, cudaStream_t st);
 
 }  // namespace hns

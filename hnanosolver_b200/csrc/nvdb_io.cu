@@ -58,7 +58,8 @@ T rd(const uint8_t* p) {
 // a buffer that can be a single ValueOnIndex grid: long enough, known magic, sizes consistent
 int check_grid(const uint8_t* g, uint64_t bytes, bool need_index_grid) {
 	using namespace hns;
-	if (!g || bytes < nvdb::kGrid + nvdb::kTree + nvdb::kRoot) return fail(HNS_ERR_INVALID_ARGUMENT, "buffer is too small for a NanoVDB grid");
+	// 64: the RootData of a float grid, the smallest there is -- an empty float grid is nothing else (open_grid checks the grid's own)
+	if (!g || bytes < nvdb::kGrid + nvdb::kTree + 64) return fail(HNS_ERR_INVALID_ARGUMENT, "buffer is too small for a NanoVDB grid");
 	const uint64_t magic = rd<uint64_t>(g);
 	if (magic != kMagicNumb && magic != kMagicGrid) return fail(HNS_ERR_INVALID_ARGUMENT, "buffer does not start with a NanoVDB grid magic number");
 	if (rd<uint64_t>(g + kOffGridSize) > bytes) return fail(HNS_ERR_INVALID_ARGUMENT, "grid size in the header exceeds the buffer");
@@ -357,16 +358,9 @@ int hns_sidecar_to_nanovdb(const int32_t* domain_origins, uint64_t n_leaves, con
 	const uint64_t bytes = hns_sidecar_nanovdb_bytes(domain_origins, n_leaves, components);
 	if (!out_buf || capacity < bytes) return fail(HNS_ERR_INVALID_ARGUMENT, "output buffer is too small");
 	for (uint64_t l = 1; l < n_leaves; ++l) {  // strictly increasing NanoVDB order: (tile, upper offset, lower offset)
-		auto key = [&](const int32_t* o, uint64_t& tile, uint32_t& node) {
-			const int64_t bias = int64_t(1) << 31;
-			tile = (uint64_t(uint32_t(int64_t(o[2]) + bias) >> 12)) | (uint64_t(uint32_t(int64_t(o[1]) + bias) >> 12) << 21) | (uint64_t(uint32_t(int64_t(o[0]) + bias) >> 12) << 42);
-			node = uint32_t(((o[0] & 4095) >> 7) << 10 | ((o[1] & 4095) >> 7) << 5 | ((o[2] & 4095) >> 7)) << 12 |
-			       uint32_t(((o[0] & 127) >> 3) << 8 | ((o[1] & 127) >> 3) << 4 | ((o[2] & 127) >> 3));
-		};
-		uint64_t ta, tb;
-		uint32_t na, nb;
-		key(domain_origins + 3 * (l - 1), ta, na), key(domain_origins + 3 * l, tb, nb);
-		if (!(ta < tb || (ta == tb && na < nb))) return fail(HNS_ERR_TOPOLOGY, "leaves are not in strictly increasing NanoVDB order at leaf " + std::to_string(l));
+		const int32_t *a = domain_origins + 3 * (l - 1), *b = domain_origins + 3 * l;
+		if (!key_less(nvdb_leaf_key(a[0], a[1], a[2]), nvdb_leaf_key(b[0], b[1], b[2])))
+			return fail(HNS_ERR_TOPOLOGY, "leaves are not in strictly increasing NanoVDB order at leaf " + std::to_string(l));
 	}
 	uint8_t* buf = static_cast<uint8_t*>(out_buf);
 	std::memset(buf, 0, bytes);
@@ -477,3 +471,49 @@ int hns_sidecar_to_nanovdb(const int32_t* domain_origins, uint64_t n_leaves, con
 }
 
 }  // extern "C"
+
+namespace hns {
+
+// The source of compSum (SOP_HNanoSolver.cpp:159-181) as flat tables: the float / Vec3f grid's leaf records -- all inside the buffer,
+// their origins (bboxMin & ~7, as hns_nvdb_leaf_topology reads them) distinct -- sorted by nvdb_leaf_key, with the 512 values of each.
+// Host only and before any CUDA call: a malformed buffer is refused here, and the device indexes these tables, never an offset read
+// from the buffer.
+int source_tables(const void* buffer, uint64_t bytes, SourceTables& out) {
+	GridWalk w{};
+	int rc = open_grid(buffer, bytes, w);
+	if (rc) return rc;
+	if (!w.lay->leaf_values) return fail(HNS_ERR_UNSUPPORTED, "an index grid holds no values to add");
+	const uint8_t* tree = w.g + kTree;
+	const uint64_t leaf_off = rd<uint64_t>(tree + kOffNodeOffset), L = rd<uint32_t>(tree + kOffNodeCount);
+	if (L && (leaf_off > bytes - kTree || L * w.lay->leaf > bytes - kTree - leaf_off))
+		return fail(HNS_ERR_INVALID_ARGUMENT, "leaf nodes lie outside the buffer");
+	std::vector<int4> origins(L);
+	std::vector<ulonglong2> keys(L);
+	std::vector<uint32_t> order(L);
+	for (uint64_t l = 0; l < L; ++l) {
+		int32_t o[3];
+		std::memcpy(o, tree + leaf_off + l * w.lay->leaf, 12);
+		origins[l] = make_int4(o[0] & ~7, o[1] & ~7, o[2] & ~7, 0);
+		keys[l] = nvdb_leaf_key(origins[l].x, origins[l].y, origins[l].z);
+		order[l] = uint32_t(l);
+	}
+	std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return key_less(keys[a], keys[b]); });
+	for (uint64_t i = 1; i < L; ++i)
+		if (!key_less(keys[order[i - 1]], keys[order[i]])) {
+			const int4 o = origins[order[i]];
+			return fail(HNS_ERR_INVALID_ARGUMENT, "two leaves of the source have the origin (" + std::to_string(o.x) + ", " + std::to_string(o.y) + ", " +
+			                                          std::to_string(o.z) + ")");
+		}
+	const int C = w.lay->components;
+	const size_t leaf_floats = size_t(512) * C;
+	out.components = C;
+	out.keys.resize(L), out.origins.resize(L), out.values.resize(L * leaf_floats);
+	for (uint64_t i = 0; i < L; ++i) {
+		const uint32_t l = order[i];
+		out.keys[i] = keys[l], out.origins[i] = origins[l];
+		std::memcpy(out.values.data() + i * leaf_floats, tree + leaf_off + l * w.lay->leaf + w.lay->leaf_values, leaf_floats * sizeof(float));
+	}
+	return HNS_OK;
+}
+
+}  // namespace hns

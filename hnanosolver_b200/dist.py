@@ -352,6 +352,11 @@ class ShardedSimulation:
     def upload(self, velocity, scalars):
         self.sim.upload(velocity, scalars)
 
+    def add_source(self, target, source, stream=None):
+        """Simulation.add_source on this rank's state (owned and ghost leaves alike: no exchange needed), by default on the frame's
+        stream. Collective where it writes the velocity: every rank adds the same sources (include/hns_b200.h, sources)."""
+        self.sim.add_source(target, source, self._stream() if stream is None else stream)
+
     def frame(self, iterations: int, dt: float) -> None:
         if self.native:
             import ctypes as C
@@ -420,13 +425,15 @@ class ShardedSimulation:
 # ------------------------------------------------------------------------------------------------------------------
 def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), fill: float = 0.35, seed: int = 7, iterations: int = 12,
                          frames: int = 2, collision: bool = False, vorticity=(0.0, 1.0), cook: bool = False, combustion: bool = True,
-                         native: bool = True, multigrid: dict | None = None):
+                         native: bool = True, multigrid: dict | None = None, source=False):
     """Collective. Runs `frames` sharded frames of a small sparse box and, on rank 0, the same frames on ONE GPU over the whole
     domain; compares the owned voxels of every rank (velocity, every scalar, pressure) with np.array_equal.
     Returns (ok, report) on rank 0 and (None, None) elsewhere. Two frames exercise the reuse of the velocity ghosts across frames.
     multigrid = dict(cycles, nu_pre, nu_post, omega, max_levels, red_black_frames): both sides solve the pressure with that many V-cycles
     (ShardedSimulation.set_pressure_solver against Simulation.set_pressure_solver over the whole domain); red_black_frames > 0 then
-    switches both back to red-black for that many more frames."""
+    switches both back to red-black for that many more frames.
+    source = True or a dict of synth.emitter arguments: both sides add the same emitter (density, fuel, temperature, velocity; a few
+    leaves outside the domain) with add_source before every frame. Needs the resident frame (cook=False)."""
     import torch
     import torch.distributed as tdist
 
@@ -454,6 +461,22 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
     if multigrid is not None:
         mgc = dict(cycles=2, nu_pre=2, nu_post=2, omega=1.15, max_levels=0, red_black_frames=0)
         mgc.update(multigrid)
+    sources = []
+    if source:
+        if cook:
+            raise ValueError("source= needs the resident frame (cook=False): a cook overwrites the state from the host arrays")
+        from . import io as hio
+
+        kw = dict(speed=0.1 * float(np.abs(wg.velocity).max()))
+        kw.update(source if isinstance(source, dict) else {})
+        so, values = synth.emitter(go, **kw)
+        sources = [("velocity" if k == "velocity" else names.index(k), H.Source(hio.grid_from_sidecar(so, v, wg.voxel_size, k)))
+                   for k, v in values.items()]
+
+    def feed(sim):
+        for target, src in sources:
+            sim.add_source(target, src)
+
     sh = ShardedSimulation(plan, np.ascontiguousarray(go[plan.local_ids]), wg.voxel_size, NS, device, native=native)
     try:
         if collision:
@@ -482,12 +505,14 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
         else:
             sh.upload(lv, lf)
             for _ in range(frames):
+                feed(sh)
                 sh.frame(iterations, wg.dt)
             if rb_frames:
                 torch.cuda.synchronize()
                 sh.check_errors()
                 sh.set_pressure_solver(None)
                 for _ in range(rb_frames):
+                    feed(sh)
                     sh.frame(iterations, wg.dt)
             torch.cuda.synchronize()
             sh.check_errors()
@@ -510,10 +535,12 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
                 ref_mg = H.Multigrid(g, mgc["max_levels"])
                 sim.set_pressure_solver(ref_mg, mgc["cycles"], mgc["nu_pre"], mgc["nu_post"], mgc["omega"])
             for _ in range(frames):
+                feed(sim)
                 sim.step(iterations, wg.dt)
             if rb_frames:
                 sim.set_pressure_solver(None)
                 for _ in range(rb_frames):
+                    feed(sim)
                     sim.step(iterations, wg.dt)
             sim.sync()
             ref = [sim.velocity()] + [sim.scalar(i) for i in range(NS)] + [sim.aux(1)]
@@ -530,7 +557,7 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
             report = dict(ok=ok, leaves=int(go.shape[0]), world=world, frames=frames, iterations=iterations, p2p=bool(getattr(sh, "p2p", False)),
                           native=native, collision=collision, vorticity=list(vorticity), cook=cook, exchanges_per_frame=sh.exchanges // max(frames, 1),
                           packed_advection_launches=packed_launches, multigrid=mgc, mg_gathers=gathers[0], mg_gather_bytes=gathers[1],
-                          mg_levels=ref_mg.num_levels if ref_mg is not None else 0, fields=lines)
+                          mg_levels=ref_mg.num_levels if ref_mg is not None else 0, sources=len(sources), fields=lines)
             del sim
         tdist.barrier()
         return ok, report

@@ -25,7 +25,7 @@ from ._lib import CombustionParams, HnsError, check, c_f32p, c_i32p, c_u64p
 from .grid_data import FLOAT, VEC3F, GridIndexedData
 
 __all__ = ["CreateIndexGrid", "Compute_Sim", "AdvectIndexGrid", "AdvectIndexGridVelocity", "ProjectNonDivergent", "Divergence",
-           "CombustionKernel", "IndexGridHandle", "Simulation", "Multigrid", "build_domain", "CombustionParams"]
+           "CombustionKernel", "IndexGridHandle", "Simulation", "Multigrid", "Source", "build_domain", "CombustionParams"]
 
 
 def _fp(a: np.ndarray):
@@ -248,6 +248,44 @@ class Multigrid:
         check(_lib.lib().hns_mg_set_coarsest_iterations(self._h, iterations))
 
 
+class Source:
+    """A NanoVDB float or Vec3f grid (uint8 host buffer: io.read_nvdb, io.grid_from_sidecar) on the current device, to be added to
+    resident fields with Simulation.add_source: openvdb::tools::compSum as the SOP does every cook (SOP_HNanoSolver.cpp:159-181),
+    bit for bit io.comp_sum. The buffer is validated on the host; a malformed one raises before anything reaches the GPU."""
+
+    def __init__(self, buffer: np.ndarray):
+        buf = np.ascontiguousarray(buffer, np.uint8)
+        h = C.c_void_p()
+        check(_lib.lib().hns_source_create(buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(h)))
+        self._h = h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            _lib.lib().hns_source_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def components(self) -> int:
+        """1 (float grid) or 3 (Vec3f grid)"""
+        return int(_lib.lib().hns_source_components(self._h))
+
+    @property
+    def num_leaves(self) -> int:
+        return int(_lib.lib().hns_source_num_leaves(self._h))
+
+    def leaves_outside(self, grid: IndexGridHandle) -> int:
+        """source leaves whose origin is not a leaf of `grid`: their values reach no field (the domain stays fixed)"""
+        n = C.c_uint64()
+        check(_lib.lib().hns_source_leaves_outside(self._h, grid._h, C.byref(n)))
+        return int(n.value)
+
+
 class Simulation:
     """Device-resident state of one simulation: velocity + n_scalars float fields on an index grid."""
 
@@ -282,6 +320,16 @@ class Simulation:
             a = np.ascontiguousarray(a, np.float32).reshape(-1)
             assert a.shape[0] == self.n
             check(_lib.lib().hns_state_upload_scalar(self._h, i, _fp(a)))
+
+    def add_source(self, target, source: Source, stream=None):
+        """compSum of `source` into the velocity (target "velocity", a Vec3f source) or into scalar `target` (an int, a float source):
+        every voxel of the grid gets value + the source's value there, +0.0 where the source has no leaf. Asynchronous on `stream`."""
+        if isinstance(target, str):
+            if target != "velocity":
+                raise ValueError(f'target must be "velocity" or a scalar index, not {target!r}')
+            check(_lib.lib().hns_state_add_source_velocity(self._h, source._h, _stream(stream)))
+        else:
+            check(_lib.lib().hns_state_add_source_scalar(self._h, int(target), source._h, _stream(stream)))
 
     def velocity(self) -> np.ndarray:
         out = np.empty((self.n, 3), np.float32)

@@ -321,3 +321,23 @@ def combustion_fields(w: Workload, seed: int = 123, chunk_leaves: int = 8192) ->
         if N:
             a[0] = 0.0
     return out
+
+
+def emitter(origins: np.ndarray, fraction: float = 0.05, n_outside: int = 4, speed: float = 1.0, seed: int = 11):
+    """A smoke emitter for sourcing (SOP_HNanoSolver.cpp:159-181): the `fraction` of the domain's leaves lowest in y -- the base of a
+    plume rising in +y -- plus `n_outside` leaves in another root tile beside the domain, which a fixed domain drops.
+    -> (source leaf origins (NanoVDB order), {"density", "temperature", "fuel": float32 (n * 512,), "velocity": float32 (n * 512, 3)});
+    the velocity pushes upward at up to `speed`. io.grid_from_sidecar turns each into a NanoVDB grid."""
+    o = np.asarray(origins, np.int32).reshape(-1, 3)
+    k = min(len(o), max(1, int(round(fraction * len(o))))) if len(o) else 0
+    base = o[np.argsort(o[:, 1], kind="stable")[:k]]
+    lo = o.min(0) if len(o) else np.zeros(3, np.int32)
+    outside = np.array([[lo[0] - 4096 - 8 * i, lo[1], lo[2]] for i in range(n_outside)], np.int32).reshape(-1, 3)
+    so = np.concatenate([base, outside])
+    so = np.ascontiguousarray(so[nanovdb_order(so)])
+    c = dense_coords(so)
+    values = {"density": 0.5 * hash_noise(seed, c, 30), "temperature": hash_noise(seed, c, 31), "fuel": 0.8 * hash_noise(seed, c, 32)}
+    vel = np.zeros((len(c), 3), np.float32)
+    vel[:, 1] = speed * hash_noise(seed, c, 33)
+    values["velocity"] = vel
+    return so, {name: np.ascontiguousarray(v, np.float32) for name, v in values.items()}

@@ -190,6 +190,33 @@ int hns_state_download_scalar(hns_state* s, int index, float* host);
 /* intermediate fields of the last step, for parity checks: which = 0 divergence, 1 pressure, 2 advected velocity (float[N][3]) */
 int hns_state_download_aux(hns_state* s, int which, float* host);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * Sources on resident state: openvdb::tools::compSum of source grids into the fed-back fields, as SOP_HNanoSolverVerb::cook does every
+ * cook (src/SOP/HNanoSolver/SOP_HNanoSolver.cpp:159-181), on the device instead of download / add on the host / upload.
+ * Semantics (bit for bit those of hnanosolver_b200.io.comp_sum): every voxel of every leaf of the state's grid becomes value + s, where
+ * s is the source's value at that voxel when the source has a leaf at that origin (all 512 values, active or not) and +0.0f otherwise
+ * -- so a -0.0 becomes +0.0 everywhere, as compSum against a background tile makes it. Plain IEEE single-precision adds; subnormals are
+ * kept. Index space only: the source's voxel size and transform are ignored. The domain stays fixed: a source leaf whose origin is not
+ * a leaf of the state's grid reaches no field (hns_source_leaves_outside counts them). Every leaf of the grid is written, ghost leaves
+ * of a shard included (the work list of hns_dist_set_plan is ignored), so each rank computes the same bits for a ghost as its owner.
+ * Sharded runs: a call that writes the velocity must be made on all ranks alike, like hns_state_upload_velocity (see hns_dist_frame).
+ * ------------------------------------------------------------------------------------------------------- */
+typedef struct hns_source hns_source;
+/* A NanoVDB float (GridType 1) or Vec3f (GridType 6) grid, given as a HOST copy of one grid (hns_nvdb_read,
+ * hns_sidecar_to_nanovdb), validated on the host and copied to the current device as a flat table of leaves.
+ * HNS_ERR_UNSUPPORTED: an index grid or any other grid type; HNS_ERR_INVALID_ARGUMENT: a buffer that is truncated, whose leaf
+ * records reach past its end or that holds two leaves with the same origin (all refused before any CUDA call). */
+int hns_source_create(const void* buffer, uint64_t bytes, hns_source** out);
+void hns_source_destroy(hns_source* src);
+int hns_source_components(const hns_source* src);        /* 1 or 3 */
+uint64_t hns_source_num_leaves(const hns_source* src);
+/* source leaves whose origin is not a leaf of g (their values reach no field); synchronous */
+int hns_source_leaves_outside(const hns_source* src, const hns_grid* g, uint64_t* out);
+/* compSum (SOP_HNanoSolver.cpp:159-181) on resident fields; asynchronous on `stream`. One kernel launch each. HNS_ERR_INVALID_ARGUMENT:
+ * a source of the wrong component count, a scalar index out of range, a source created on another device than the state's grid. */
+int hns_state_add_source_velocity(hns_state* s, const hns_source* src, void* stream);          /* Vec3f source */
+int hns_state_add_source_scalar(hns_state* s, int index, const hns_source* src, void* stream); /* float source */
+
 /* Enables the combustion_oxygen + temperature_buoyancy stage of the all-in-one frame (src/Cuda/HNanoSolver.cu:190-250) on the
  * scalar fields with the given indices, and the vorticityConfinement pass (Kernel.cu:969-1025) between advect_vector and the
  * divergence when params->vorticityScale != 0 and (int)params->factorScale != 0. The reference runs that kernel in place
