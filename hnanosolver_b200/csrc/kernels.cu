@@ -759,7 +759,9 @@ void launch_vorticity_force(const GridView& g, const float* const vel[3], const 
 //   restrict   parent rhs = mean of the 8 children's residuals           (summed z pair, then y pair, then x pair)
 //   prolong    p += trilinear interpolation of the parents' correction   (weights 3/4, 1/4 per axis; z, then y, then x)
 // =============================================================================================================
-// kNorm: also accumulates sum r^2 and sum rhs^2 in fp64 (per-thread partial sums, warp shuffles, one atomic per warp).
+// kNorm: also accumulates sum r^2 and sum rhs^2 in fp64 (per-thread partial sums, warp shuffles, one atomic per warp). That r is
+// recomputed in fp64 from the fp32 fields, scaled by the fp64 1 / dx^2 (`inv_dx2_f64`): the fp32 r of the transfer loses a converged
+// solve's residual to cancellation, and a norm taken from it comes out percents too small at relative residuals of 1e-7 to 1e-6.
 // kGather (with kRestrict, sharded runs): the restricted octant goes to n_gather colour-split arrays, gather[2 t] / gather[2 t + 1] = red /
 // black of target t -- every rank's copy of the level-1 right-hand side, peers' ones mapped over NVLink -- instead of crhs. Plain stores:
 // the flag that publishes them is raised by a later kernel in the same stream.
@@ -769,7 +771,7 @@ __global__ void __launch_bounds__(256) k_mg_residual(GridView g, const float* __
                                                      const float* __restrict__ diag_red, const float* __restrict__ diag_blk,
                                                      const int32_t* __restrict__ parent,
                                                      float* __restrict__ crhs_red, float* __restrict__ crhs_blk, double* __restrict__ sums,
-                                                     float* const* __restrict__ gather, int n_gather) {
+                                                     double inv_dx2_f64, float* const* __restrict__ gather, int n_gather) {
 	RowCtx c;
 	if (!make_row_ctx(g, c)) return;
 	const uint64_t self = c.self();
@@ -795,7 +797,11 @@ __global__ void __launch_bounds__(256) k_mg_residual(GridView g, const float* __
 		const float lap = fmaf(kMask ? -dg.v[z] : -6.0f, cp.v[z], sum);
 		r[z] = fmaf(-lap, inv_dx2, f.v[z]);
 		if (kMask && dg.v[z] == 0.f) r[z] = 0.f;
-		if (kNorm) a = fma(double(r[z]), double(r[z]), a), b = fma(double(f.v[z]), double(f.v[z]), b);
+		if (kNorm) {
+			const double sum64 = ((((double(pxp.v[z]) + double(pxm.v[z])) + double(pyp.v[z])) + double(pym.v[z])) + double(zp)) + double(zm);
+			const double r64 = kMask && dg.v[z] == 0.f ? 0.0 : double(f.v[z]) - (sum64 - (kMask ? double(dg.v[z]) : 6.0) * double(cp.v[z])) * inv_dx2_f64;
+			a = fma(r64, r64, a), b = fma(double(f.v[z]), double(f.v[z]), b);
+		}
 	}
 	if (kNorm) {
 #pragma unroll
@@ -834,12 +840,14 @@ void launch_mg_residual(const GridView& g, const float* const p[2], const float*
                         float* const coarse_rhs[2], double* sums, cudaStream_t st) {
 	if (!g.count()) return;
 	const float inv_dx2 = 1.0f / (dx * dx);
+	const double inv_dx2_f64 = 1.0 / (double(dx) * double(dx));
 	const unsigned grid = (g.count() + 3) / 4;
 	float* cr = coarse_rhs ? coarse_rhs[0] : nullptr;
 	float* cb = coarse_rhs ? coarse_rhs[1] : nullptr;
 	const float* dr = diag ? diag[0] : nullptr;
 	const float* db = diag ? diag[1] : nullptr;
-#define HNS_MG_RES(M, R, N) HNS_LAUNCH((k_mg_residual<M, R, N>), grid, 256, 0, st, g, p[0], p[1], rhs[0], rhs[1], inv_dx2, dr, db, parent, cr, cb, sums, nullptr, 0)
+#define HNS_MG_RES(M, R, N) \
+	HNS_LAUNCH((k_mg_residual<M, R, N>), grid, 256, 0, st, g, p[0], p[1], rhs[0], rhs[1], inv_dx2, dr, db, parent, cr, cb, sums, inv_dx2_f64, nullptr, 0)
 	const bool R = coarse_rhs != nullptr, N = sums != nullptr;
 	if (diag) {
 		if (R && N) HNS_MG_RES(true, true, true);
@@ -856,7 +864,7 @@ void launch_mg_restrict_gather(const GridView& g, const float* const p[2], const
                                float* const* gather, int n_gather, cudaStream_t st) {
 	if (!g.count() || n_gather <= 0) return;
 	HNS_LAUNCH((k_mg_residual<false, true, false, true>), (g.count() + 3) / 4, 256, 0, st, g, p[0], p[1], rhs[0], rhs[1], 1.0f / (dx * dx), nullptr,
-	           nullptr, parent, nullptr, nullptr, nullptr, gather, n_gather);
+	           nullptr, parent, nullptr, nullptr, nullptr, 0.0, gather, n_gather);
 }
 
 // sum of squares of a colour-split field over the listed leaves (fp64)
