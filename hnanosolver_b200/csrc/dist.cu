@@ -425,8 +425,11 @@ int hns_dist_ipc_finish(hns_dist* d) {
 	std::vector<uint32_t*> rem(std::max<size_t>(n, 1), nullptr), loc(std::max<size_t>(n, 1), nullptr);
 	for (size_t i = 0; i < n; ++i) {
 		if (!d->peers[i].remote_region) return fail(HNS_ERR_RUNTIME, "peer " + std::to_string(d->peers[i].rank) + " is not connected");
-		rem[i] = d->peers[i].n_send ? reinterpret_cast<uint32_t*>(d->peers[i].remote_region) : nullptr;
-		loc[i] = d->peers[i].n_recv ? reinterpret_cast<uint32_t*>(d->block + d->peers[i].region_off) : nullptr;
+		// Every exchange is a handshake with every peer, also with one this rank only sends to or only receives from: a region is
+		// written again only after a later flag of the rank that unpacks it, so a rank that only sends cannot run a frame ahead and
+		// overwrite ghost bricks its receivers have not unpacked yet (a region without bricks still has its flag words).
+		rem[i] = reinterpret_cast<uint32_t*>(d->peers[i].remote_region);
+		loc[i] = reinterpret_cast<uint32_t*>(d->block + d->peers[i].region_off);
 	}
 	if (n > 32) return fail(HNS_ERR_UNSUPPORTED, "more than 32 peers");
 	cudaFree(d->d_remote_flags), cudaFree(d->d_local_flags);
@@ -922,8 +925,10 @@ static int dist_frame(hns_dist* d, hns_state* s, int iterations, float dt, void*
 		const float omega = hns_omega_compute(s->grid->voxel_size);
 		if (d->p2p && d->n_boundary > 0) {
 			if ((rc = fused_pressure(d, s, iterations, omega, st))) return rc;
-		} else if ((rc = pipelined_sweeps(d, s, iterations, omega, false, st))) {
-			return rc;
+		} else {
+			// a rank without boundary leaves: its fused peers wait for its "pressure zeroed" flag of this frame as for each other's
+			if (d->p2p) HNS_LAUNCH(k_signal, 1, 32, 0, st, d->d_remote_flags, int(d->peers.size()), 5, ++d->seq[5]);
+			if ((rc = pipelined_sweeps(d, s, iterations, omega, false, st))) return rc;
 		}
 	}
 	mark();

@@ -66,8 +66,12 @@ def make_plan(global_origins: np.ndarray, world: int, rank: int) -> ShardPlan:
     """Contiguous, count-balanced ranges of the sorted leaf list; ghosts = 26-neighbours owned by another rank, plus global leaf 0
     on every rank: advect_scalars reads "array element 0" for inactive voxels (reference src/Cuda/Kernel.cu:192,225), and with
     leaf 0 held as a ghost (it sorts first, so it is LOCAL leaf 0 too) the local element 0 IS the global one after the exchange
-    that precedes advect_scalars -- no broadcast, no special case in the kernels."""
+    that precedes advect_scalars -- no broadcast, no special case in the kernels.
+    Every rank owns at least one leaf: fewer leaves than ranks is refused (ValueError) identically on every rank. An empty domain
+    gives every rank an empty plan."""
     L = global_origins.shape[0]
+    if 0 < L < world:
+        raise ValueError(f"make_plan: {L} leaves cannot be split over {world} ranks (every rank must own at least one leaf)")
     ranges = np.array([(L * r) // world for r in range(world + 1)], np.int64)
     owner = np.searchsorted(ranges, np.arange(L), side="right") - 1
     keys = _coord_keys(global_origins)
@@ -98,9 +102,8 @@ def make_plan(global_origins: np.ndarray, world: int, rank: int) -> ShardPlan:
     if L and world > 1:
         if rank == 0:
             for peer in range(1, world):
-                if ranges[peer + 1] > ranges[peer]:      # a rank without leaves holds nothing
-                    send.setdefault(peer, set()).add(0)
-        elif hi > lo:
+                send.setdefault(peer, set()).add(0)
+        else:
             recv.setdefault(0, set()).add(0)
             ghost.add(0)
     local_ids = np.array(sorted(set(mine.tolist()) | ghost), np.int64)
@@ -425,10 +428,18 @@ class ShardedSimulation:
 # ------------------------------------------------------------------------------------------------------------------
 def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), fill: float = 0.35, seed: int = 7, iterations: int = 12,
                          frames: int = 2, collision: bool = False, vorticity=(0.0, 1.0), cook: bool = False, combustion: bool = True,
-                         native: bool = True, multigrid: dict | None = None, source=False):
+                         native: bool = True, multigrid: dict | None = None, source=False, origins=None, element0: float | None = None,
+                         scalars: int | None = None):
     """Collective. Runs `frames` sharded frames of a small sparse box and, on rank 0, the same frames on ONE GPU over the whole
-    domain; compares the owned voxels of every rank (velocity, every scalar, pressure) with np.array_equal.
-    Returns (ok, report) on rank 0 and (None, None) elsewhere. Two frames exercise the reuse of the velocity ghosts across frames.
+    domain; compares the owned voxels of every rank (velocity, every scalar, pressure) bit for bit (float32 bit patterns, so -0.0 and
+    +0.0 differ). Returns (ok, report) on rank 0 and (None, None) elsewhere. Two frames exercise the reuse of the velocity ghosts
+    across frames.
+    origins: the global leaf origins (sorted into NanoVDB order here) instead of the sparse box global_sparse_origins(box, fill, seed);
+    the fields are evaluated at their coordinates and the collider is centred in their bounding box.
+    element0: voxel 0 of every advected scalar starts at this value instead of 0.0 (advect_scalars' "inactive -> element 0" value).
+    scalars: the number of advected scalars (default 5). With combustion they are density, fuel, waste, temperature and flame
+    followed by swirl fields of distinct phases; without it the first `scalars` of that list. The collision SDF comes after them, at
+    most 16 fields in all.
     multigrid = dict(cycles, nu_pre, nu_post, omega, max_levels, red_black_frames): both sides solve the pressure with that many V-cycles
     (ShardedSimulation.set_pressure_solver against Simulation.set_pressure_solver over the whole domain); red_black_frames > 0 then
     switches both back to red-black for that many more frames.
@@ -440,19 +451,43 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
     from . import _lib
     from . import launchers as H
 
-    go = global_sparse_origins(box, fill, seed)
-    vel, den, tem = synth._swirl_fields(max(box))
-    wg = synth._finish("parity", go, vel, [den, tem], ["density", "temperature"], 40, seed, with_coords=False)
+    if origins is None:
+        go = global_sparse_origins(box, fill, seed)
+    else:
+        go = np.asarray(origins, np.int32).reshape(-1, 3)
+        go = np.ascontiguousarray(go[synth.nanovdb_order(go)])
+    n_adv = 5 if scalars is None else int(scalars)
+    if n_adv < 0 or (combustion and n_adv < 5) or n_adv + int(collision) > 16:
+        raise ValueError(f"scalars={scalars}: at least 5 with combustion (its four fields follow density), at most 16 fields with the SDF")
+    R = max(box)
+    vel, den, tem = synth._swirl_fields(R)
+
+    def swirl(k):  # extra scalar k: a swirl of its own phase
+        def fn(cd, seed):
+            p = cd.astype(np.float32) * np.float32(2 * np.pi / R)
+            return (0.5 + 0.5 * np.sin(p[:, 0] + np.float32(0.9 * k)) * np.cos(p[:, 1] - np.float32(0.6 * k))
+                    * np.sin(p[:, 2] + np.float32(0.5 + 0.4 * k))).astype(np.float32)
+        return fn
+
+    extra = max(0, n_adv - 5)
+    wg = synth._finish("parity", go, vel, [den, tem] + [swirl(k) for k in range(extra)], ["density", "temperature"] + [f"swirl{k}" for k in range(extra)],
+                       40, seed, with_coords=False)
     plan = make_plan(go, world, rank)
     lo = np.repeat(plan.local_ids, 512) * 512 + np.tile(np.arange(512), plan.n_local)
     comb = synth.combustion_fields(wg)
-    names = ["density", "fuel", "waste", "temperature", "flame"]
-    gfields = [wg.scalars[0]] + [comb[k] for k in names[1:]]
+    names = ["density", "fuel", "waste", "temperature", "flame"] + [f"swirl{k}" for k in range(extra)]
+    gfields = [wg.scalars[0]] + [comb[k] for k in names[1:5]] + wg.scalars[2:]
+    names, gfields = names[:n_adv], gfields[:n_adv]
+    if element0 is not None and go.shape[0]:
+        for f in gfields:
+            f[0] = np.float32(element0)
     if collision:  # a sphere collider as the last scalar, hasCollision path on
         off = np.stack(np.unravel_index(np.arange(512), (8, 8, 8)), 1)
         gc = (np.repeat(go, 512, axis=0) + off[np.tile(np.arange(512), go.shape[0])]).astype(np.float32)
-        centre = np.array([box[0] / 2, box[1] / 2, box[2] / 2], np.float32)
-        sdf = (0.05 * (np.sqrt(((gc - centre) ** 2).sum(1)) - 20.0)).astype(np.float32)
+        lo_c, hi_c = go.min(0).astype(np.float64), go.max(0).astype(np.float64) + 8.0
+        centre = ((lo_c + hi_c) / 2).astype(np.float32)
+        radius = min(20.0, float((hi_c - lo_c).min()) / 4)   # 20 voxels, less in a domain too thin to have voxels outside it
+        sdf = (0.05 * (np.sqrt(((gc - centre) ** 2).sum(1)) - radius)).astype(np.float32)
         sdf[0] = 0.0
         names, gfields = names + ["collision_sdf"], gfields + [sdf]
     NS = len(gfields)
@@ -471,7 +506,7 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
         kw.update(source if isinstance(source, dict) else {})
         so, values = synth.emitter(go, **kw)
         sources = [("velocity" if k == "velocity" else names.index(k), H.Source(hio.grid_from_sidecar(so, v, wg.voxel_size, k)))
-                   for k, v in values.items()]
+                   for k, v in values.items() if k == "velocity" or k in names]
 
     def feed(sim):
         for target, src in sources:
@@ -548,16 +583,19 @@ def sharded_parity_check(rank: int, world: int, device, *, box=(256, 128, 128), 
                 ref[NS] = gfields[-1]   # the resident state keeps the SDF; hns_dist_cook hands the caller's block back untouched
             ok, lines = True, []
             for k, nm in enumerate(["velocity"] + names + ["pressure"]):
-                got = np.concatenate([gathered[r][k] for r in range(world)])
-                same = bool(np.array_equal(got, ref[k]))
+                got = np.ascontiguousarray(np.concatenate([gathered[r][k] for r in range(world)]), np.float32)
+                want = np.ascontiguousarray(ref[k], np.float32)
+                differ = got.view(np.uint32) != want.view(np.uint32)   # bits: a -0.0 where +0.0 is due is a difference
+                same = got.shape == want.shape and not differ.any()
                 ok &= same
-                bad = np.nonzero((got != ref[k]).reshape(got.shape[0], -1).any(1))[0]
+                bad = np.nonzero(differ.reshape(got.shape[0], -1).any(1))[0]
                 lines.append(f"{nm}: bitwise {'ok' if same else 'MISMATCH'} ({bad.size}/{got.shape[0]} voxels differ"
-                             + (f", max|diff| {np.abs(got.astype(np.float64) - ref[k]).max():.3e}, first leaves {np.unique(bad // 512)[:6].tolist()}" if bad.size else "") + ")")
+                             + (f", max|diff| {np.abs(got.astype(np.float64) - want).max():.3e}, first leaves {np.unique(bad // 512)[:6].tolist()}" if bad.size else "") + ")")
             report = dict(ok=ok, leaves=int(go.shape[0]), world=world, frames=frames, iterations=iterations, p2p=bool(getattr(sh, "p2p", False)),
                           native=native, collision=collision, vorticity=list(vorticity), cook=cook, exchanges_per_frame=sh.exchanges // max(frames, 1),
                           packed_advection_launches=packed_launches, multigrid=mgc, mg_gathers=gathers[0], mg_gather_bytes=gathers[1],
-                          mg_levels=ref_mg.num_levels if ref_mg is not None else 0, sources=len(sources), fields=lines)
+                          mg_levels=ref_mg.num_levels if ref_mg is not None else 0, sources=len(sources), scalars=n_adv, element0=element0,
+                          fields=lines)
             del sim
         tdist.barrier()
         return ok, report

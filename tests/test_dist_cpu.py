@@ -3,6 +3,7 @@ frame's steps on its LOCAL leaves with the CPU oracle as the per-step kernel, an
 ShardPlan / HaloExchanger code the GPU path uses. The owned results, concatenated in rank order, must equal the single-domain
 frame bit for bit."""
 import os
+import socket
 import sys
 
 import numpy as np
@@ -14,23 +15,28 @@ import torch.multiprocessing as mp
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+
+from helpers import PARTITIONS, partition_origins  # noqa: E402
+
 from hnanosolver_b200 import dist as hdist  # noqa: E402
 from hnanosolver_b200 import synth  # noqa: E402
 
+CATALOGUE = [(name, world) for name, (_, worlds) in PARTITIONS.items() for world, reach in worlds.items() if reach is not None]
 
-def test_plan_partitions_and_ghosts_are_consistent():
-    w = synth.smoke_sphere(48, 3)
-    world = 3
-    plans = [hdist.make_plan(w.origins, world, r) for r in range(world)]
-    L = w.num_leaves
+
+def _check_plan(origins, world):
+    plans = [hdist.make_plan(origins, world, r) for r in range(world)]
+    L = origins.shape[0]
     owned = np.concatenate([p.local_ids[p.owned_local] for p in plans])
     assert np.array_equal(owned, np.arange(L))                                    # a partition, in order
-    lut = {tuple(o): i for i, o in enumerate(w.origins.tolist())}
+    assert all(p.n_owned > 0 for p in plans)
+    lut = {tuple(o): i for i, o in enumerate(origins.tolist())}
     for p in plans:
         mine = set(p.local_ids[p.owned_local].tolist())
         want = set()
         for l in mine:
-            o = w.origins[l]
+            o = origins[l]
             for dx in (-8, 0, 8):
                 for dy in (-8, 0, 8):
                     for dz in (-8, 0, 8):
@@ -44,14 +50,39 @@ def test_plan_partitions_and_ghosts_are_consistent():
         assert np.all(np.diff(p.local_ids) > 0)                                   # local order == global NanoVDB order
         for q, ids in p.send.items():                                             # my send list == the peer's recv list
             assert np.array_equal(p.local_ids[ids], plans[q].local_ids[plans[q].recv[p.rank]])
+        for q, ids in p.recv.items():                                             # and every recv list has its send list
+            assert p.rank in plans[q].send and len(plans[q].send[p.rank]) == len(ids)
+            assert not p.owned_local[ids].any()                                   # nothing owned is overwritten by a ghost
 
 
-def _worker(rank, world, port, tmp):
+def test_plan_partitions_and_ghosts_are_consistent():
+    _check_plan(synth.smoke_sphere(48, 3).origins, 3)
+
+
+@pytest.mark.parametrize("name, world", CATALOGUE, ids=[f"{n}@{w}" for n, w in CATALOGUE])
+def test_plan_partitions_and_ghosts_are_consistent_on_partitions(name, world):
+    _check_plan(partition_origins(name), world)
+
+
+def _frame_workload(case):
+    """the sphere, or a partition of the catalogue with the sparse-smoke swirl on it and 0.625 in every scalar's element 0 (the
+    "inactive" value of advect_scalars, which ranks other than 0 read from their ghost copy of global leaf 0)"""
+    if case == "sphere":
+        return synth.smoke_sphere(40, 5)
+    o = partition_origins(case)
+    vel, den, tem = synth._swirl_fields(64)
+    w = synth._finish(case, o, vel, [den, tem], ["density", "temperature"], 40, 5)
+    for a in w.scalars:
+        a[0] = np.float32(0.625)
+    return w
+
+
+def _worker(rank, world, port, tmp, case):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
     from oracle import oracle as O
 
-    w = synth.smoke_sphere(40, 5)
+    w = _frame_workload(case)
     I, dt, h = 5, w.dt, w.voxel_size
     plan = hdist.make_plan(w.origins, world, rank)
     lo = np.repeat(plan.local_ids, 512) * 512 + np.tile(np.arange(512), plan.n_local)   # local voxel -> global voxel
@@ -110,21 +141,30 @@ def _worker(rank, world, port, tmp):
     ex.exchange(list(hdist.F_VEL) + [10 + i for i in range(len(w.scalars))])
     outs = ix.advect_scalars(vel(), [F[10 + i] for i in range(len(w.scalars))], dt, h)
     m = np.repeat(plan.owned_local, 512)
-    np.savez(os.path.join(tmp, f"rank{rank}.npz"), vel=vel()[m], p=F[6][m], s0=outs[0][m], exchanges=ex.exchanges)
+    np.savez(os.path.join(tmp, f"rank{rank}.npz"), vel=vel()[m], p=F[6][m], s=np.stack(outs)[:, m], exchanges=ex.exchanges)
     dist.barrier()
     dist.destroy_process_group()
 
 
-@pytest.mark.parametrize("world", [2, 3])
-def test_sharded_frame_equals_single_domain_frame(tmp_path, world):
+def _bits(a):
+    return np.ascontiguousarray(a, np.float32).view(np.uint32)
+
+
+# the sphere; three_blobs at 3 ranks (ranks 1 and 2 exchange nothing but their ghost of leaf 0); block8 at 4 ranks (no interior leaf)
+@pytest.mark.parametrize("case, world", [pytest.param("sphere", 2, id="2"), pytest.param("sphere", 3, id="3"),
+                                         pytest.param("three_blobs", 3, id="three_blobs@3"), pytest.param("block8", 4, id="block8@4")])
+def test_sharded_frame_equals_single_domain_frame(tmp_path, case, world):
     from oracle import oracle as O
 
-    port = 29600 + world + (os.getpid() % 200)
-    mp.spawn(_worker, args=(world, port, str(tmp_path)), nprocs=world, join=True)
-    w = synth.smoke_sphere(40, 5)
+    with socket.socket() as sk:
+        sk.bind(("127.0.0.1", 0))
+        port = sk.getsockname()[1]
+    mp.spawn(_worker, args=(world, port, str(tmp_path), case), nprocs=world, join=True)
+    w = _frame_workload(case)
     want = O.OracleIndex(w.coords).frame(w.velocity, w.scalars, 5, w.dt, w.voxel_size)
     parts = [np.load(tmp_path / f"rank{r}.npz") for r in range(world)]
-    assert np.array_equal(np.concatenate([p["vel"] for p in parts]), want["vel"])
-    assert np.array_equal(np.concatenate([p["p"] for p in parts]), want["p"])
-    assert np.array_equal(np.concatenate([p["s0"] for p in parts]), want["scalars"][0])
+    assert np.array_equal(_bits(np.concatenate([p["vel"] for p in parts])), _bits(want["vel"]))
+    assert np.array_equal(_bits(np.concatenate([p["p"] for p in parts])), _bits(want["p"]))
+    for i in range(len(w.scalars)):
+        assert np.array_equal(_bits(np.concatenate([p["s"][i] for p in parts])), _bits(want["scalars"][i])), f"scalar {i}"
     assert int(parts[0]["exchanges"]) == 3 + 2 * 5                                # vel, adv, 2 per iteration, vel+scalars
