@@ -9,7 +9,9 @@ Two ways to run a frame are shown side by side and must agree bit for bit:
 An emitter at the plume's base (density, temperature and fuel sources and an upward velocity source, as NanoVDB grids) is added in
 front of every frame, as the SOP does with compSum (SOP_HNanoSolver.cpp:159-181): on the host blocks with io.comp_sum, on the
 resident state with Simulation.add_source. The domain stays fixed: the emitter's leaves outside it are dropped.
-With an output directory the last frame is written as a NanoVDB file + sidecar blocks (hnanosolver_b200.io) and read back.
+With an output directory the last frame is written as a NanoVDB file + sidecar blocks (hnanosolver_b200.io) and read back, and every
+field is written as a float / Vec3f .nvdb grid twice: by the host writer from the host buffers, and exported from the resident state on
+the device (Simulation.export_grid), which must give the same bytes; a pruned export (tolerance 0) is written next to it.
 """
 import os
 import sys
@@ -87,3 +89,20 @@ if out_dir:
     g2 = H.create_index_grid_from_origins(origins, h)
     assert np.array_equal(g2.nanovdb_buffer()[672:], grid.nanovdb_buffer()[672:]) and np.array_equal(back.pValues(H.VEC3F, "vel"), vel)
     print(f"wrote and re-read {out_dir}/grid.nvdb ({os.path.getsize(os.path.join(out_dir, 'grid.nvdb'))} bytes) + {back.numValueBlocks()} sidecar blocks")
+    # the cache frame as the SOP writes it (writeIndexGrid per field): from the host buffers, and exported from the resident state on
+    # the device, whole-domain (the same bytes) and pruned at tolerance 0 (leaves that hold only zeros left out). The collision SDF is
+    # an input, not a result: the launcher hands its block back zeroed, the resident state keeps it.
+    paths = hio.write_index_grids(os.path.join(out_dir, "grids"), w.origins, data, w.voxel_size)
+    pruned_dir = os.path.join(out_dir, "grids_pruned")
+    os.makedirs(pruned_dir, exist_ok=True)
+    vg = H.ValueGrid()
+    for path in paths:
+        name = os.path.basename(path)[:-len(".nvdb")]
+        if name == "collision_sdf":
+            continue
+        target = "velocity" if name == "vel" else names.index(name)
+        assert np.array_equal(sim.export_grid(target, name, -1.0, vg).download(), hio.read_nvdb(path)), name
+        pruned = os.path.join(pruned_dir, f"{name}.nvdb")
+        hio.write_nvdb(pruned, sim.export_grid(target, name, 0.0, vg).download())
+        print(f"{name:12s} whole domain {os.path.getsize(path):10d} bytes (host writer == device export), pruned at 0: "
+              f"{os.path.getsize(pruned):10d} bytes, {vg.num_leaves} of {w.num_leaves} leaves")

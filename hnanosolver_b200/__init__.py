@@ -6,5 +6,5 @@ host-side mirror of the reference's launcher interface (launchers.py, grid_data.
 from .grid_data import FLOAT, VEC3F, AllocationType, GridIndexedData  # noqa: F401
 from ._lib import CombustionParams, HnsError, HnsInvalidArgument  # noqa: F401
 from .launchers import (AdvectIndexGrid, AdvectIndexGridVelocity, CombustionKernel, Compute_Sim, CreateIndexGrid,  # noqa: F401
-                        Divergence, IndexGridHandle, Multigrid, ProjectNonDivergent, Simulation, Source, build_domain,
+                        Divergence, IndexGridHandle, Multigrid, ProjectNonDivergent, Simulation, Source, ValueGrid, build_domain,
                         create_index_grid_from_origins)

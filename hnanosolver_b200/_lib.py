@@ -80,6 +80,14 @@ SIGNATURES = {
     "hns_source_leaves_outside": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]),
     "hns_state_add_source_velocity": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "hns_state_add_source_scalar": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "hns_value_grid_create": (C.c_int, [C.POINTER(C.c_void_p)]),
+    "hns_value_grid_destroy": (None, [C.c_void_p]),
+    "hns_value_grid_bytes": (C.c_uint64, [C.c_void_p]),
+    "hns_value_grid_num_leaves": (C.c_uint64, [C.c_void_p]),
+    "hns_value_grid_device_ptr": (C.c_void_p, [C.c_void_p]),
+    "hns_value_grid_download": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
+    "hns_state_export_velocity": (C.c_int, [C.c_void_p, C.c_float, C.c_char_p, C.c_void_p, C.c_void_p]),
+    "hns_state_export_scalar": (C.c_int, [C.c_void_p, C.c_int, C.c_float, C.c_char_p, C.c_void_p, C.c_void_p]),
     "hns_state_set_combustion": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(CombustionParams)]),
     "hns_state_step": (C.c_int, [C.c_void_p, C.c_int, C.c_float, C.c_uint, C.c_void_p]),
     "hns_state_advect_velocity": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p]),

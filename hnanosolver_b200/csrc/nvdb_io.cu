@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "nvdb_layout.cuh"
 
 namespace {
 
@@ -201,23 +202,12 @@ int hns_nvdb_leaf_origins(const void* nanovdb_buffer, uint64_t bytes, int32_t* o
 // goes back: a grid with the domain's topology, every leaf buffer memcpy'd from the block, class FOG_VOLUME for float grids and
 // STAGGERED (+ VEC_CONTRAVARIANT_RELATIVE, an OpenVDB-only tag) for vector grids. The reference does this over OpenVDB grids; OpenVDB
 // is not vendored, NanoVDB is (externals/nanovdb), and its float / Vec3f grids carry the same leaf buffers, so the headless path reads
-// and writes those. Node layouts restated from externals/nanovdb/NanoVDB.h (LeafData :3660-3742, InternalData :3125-3200, RootData
-// :2620-2700) and checked with sizeof / offsetof against those headers; tests/test_nvdb_io.py reads and writes the same grids with
-// NanoVDB's own builder, accessor and file IO (oracle/_ref/libref_host.so).
+// and writes those. Node layouts: nvdb_layout.cuh (shared with the device export, export.cu); tests/test_nvdb_io.py reads and writes
+// the same grids with NanoVDB's own builder, accessor and file IO (oracle/_ref/libref_host.so).
 // =====================================================================================================================================
-namespace {
+using namespace hns::vgrid;
 
-struct ValueLayout {
-	uint32_t grid_type;      // GridType: Float 1, Vec3f 6, OnIndex 20
-	uint64_t root, tile, upper, lower, leaf;             // node sizes in bytes
-	uint64_t upper_table, lower_table, table_stride;     // InternalData::mTable and the size of its Tile union
-	uint64_t leaf_values;    // LeafData::mValues (0: none, index grids)
-	int components;
-};
-constexpr ValueLayout kFloatLayout{1, 64, 32, 270400, 33856, 2144, 8256, 1088, 8, 96, 1};
-constexpr ValueLayout kVec3fLayout{6, 96, 32, 532544, 66624, 6272, 8256, 1088, 16, 128, 3};
-constexpr ValueLayout kIndexLayout{20, 96, 32, 270400, 33856, 96, 8256, 1088, 8, 0, 0};
-constexpr uint64_t kUpperChildMask = 4128, kLowerChildMask = 544, kLeafValueMask = 16, kRootTableSize = 24;
+namespace {
 
 const ValueLayout* layout_of(uint32_t grid_type) {
 	return grid_type == 1 ? &kFloatLayout : grid_type == 6 ? &kVec3fLayout : grid_type == 20 ? &kIndexLayout : nullptr;
@@ -333,7 +323,7 @@ int hns_sidecar_from_nanovdb(const void* buffer, uint64_t bytes, const int32_t* 
 
 // size of the grid hns_sidecar_to_nanovdb emits for these leaves (components: 1 float, 3 Vec3f); 0 on a bad argument
 uint64_t hns_sidecar_nanovdb_bytes(const int32_t* domain_origins, uint64_t n_leaves, int components) {
-	const ValueLayout* lay = components == 1 ? &kFloatLayout : components == 3 ? &kVec3fLayout : nullptr;
+	const ValueLayout* lay = value_layout(components);
 	if (!lay || (n_leaves && !domain_origins)) return 0;
 	uint64_t T = 0, nLower = 0;
 	for (uint64_t l = 0; l < n_leaves; ++l) {
@@ -342,7 +332,7 @@ uint64_t hns_sidecar_nanovdb_bytes(const int32_t* domain_origins, uint64_t n_lea
 		const bool newLower = newTile || (o[0] >> 7) != (p[0] >> 7) || (o[1] >> 7) != (p[1] >> 7) || (o[2] >> 7) != (p[2] >> 7);
 		T += newTile, nLower += newLower;
 	}
-	return hns::nvdb::kGrid + hns::nvdb::kTree + lay->root + lay->tile * T + lay->upper * T + lay->lower * nLower + lay->leaf * n_leaves;
+	return GridOffsets(*lay, n_leaves, nLower, T).end;
 }
 
 // IndexGridBuilder::writeIndexGrid (GridBuilder.hpp:168-216) over NanoVDB: a float (class FogVolume) or Vec3f (class Staggered) grid with
@@ -351,7 +341,7 @@ uint64_t hns_sidecar_nanovdb_bytes(const int32_t* domain_origins, uint64_t n_lea
 int hns_sidecar_to_nanovdb(const int32_t* domain_origins, uint64_t n_leaves, const uint64_t* masks, const void* values, int components, float voxel_size,
                            const char* name, void* out_buf, uint64_t capacity) {
 	using namespace hns;
-	const ValueLayout* lay = components == 1 ? &kFloatLayout : components == 3 ? &kVec3fLayout : nullptr;
+	const ValueLayout* lay = value_layout(components);
 	if (!lay) return fail(HNS_ERR_INVALID_ARGUMENT, "components must be 1 (float) or 3 (Vec3f)");
 	if (!(voxel_size > 0.0f)) return fail(HNS_ERR_INVALID_ARGUMENT, "voxelSize must be positive.");
 	if (n_leaves && (!domain_origins || !values)) return fail(HNS_ERR_INVALID_ARGUMENT, "null argument");
@@ -371,41 +361,8 @@ int hns_sidecar_to_nanovdb(const int32_t* domain_origins, uint64_t n_leaves, con
 		const bool newTile = l == 0 || (o[0] >> 12) != (p[0] >> 12) || (o[1] >> 12) != (p[1] >> 12) || (o[2] >> 12) != (p[2] >> 12);
 		T += newTile, nLower += newTile || (o[0] >> 7) != (p[0] >> 7) || (o[1] >> 7) != (p[1] >> 7) || (o[2] >> 7) != (p[2] >> 7);
 	}
-	const uint64_t oTree = nvdb::kGrid, oRoot = oTree + nvdb::kTree, oUpper = oRoot + lay->root + lay->tile * T, oLower = oUpper + lay->upper * T,
-	               oLeaf = oLower + lay->lower * nLower;
-	const double s = double(voxel_size);
-	// GridData (GridData::init, NanoVDB.h:1834-1862)
-	uint8_t* g = buf;
-	put(g + 0, kMagicNumb);
-	put(g + 8, ~uint64_t(0));                                   // checksum: disabled
-	put(g + kOffVersion, uint32_t((32u << 21) | (7u << 10)));
-	put(g + 20, uint32_t(0x22));                                // HasBBox | IsBreadthFirst; no min/max, average, std deviation
-	put(g + kOffGridIndex, uint32_t(0));
-	put(g + kOffGridCount, uint32_t(1));
-	put(g + kOffGridSize, bytes);
-	if (name) std::strncpy(reinterpret_cast<char*>(g + kOffName), name, kNameMax - 1);
-	uint8_t* m = g + 296;                                       // Map: matF[9] invMatF[9] vecF[3] taperF matD[9] invMatD[9] vecD[3] taperD
-	for (int d = 0; d < 3; ++d) {
-		put(m + 16 * d, float(s));
-		put(m + 36 + 16 * d, 1.0f / float(s));
-		put(m + 88 + 32 * d, s);
-		put(m + 160 + 32 * d, 1.0 / s);
-	}
-	put(m + 84, 1.0f);
-	put(m + 256, 1.0);
-	for (int d = 0; d < 3; ++d) put(g + kOffVoxelSize + 8 * d, s);
-	put(g + kOffGridClass, uint32_t(components == 1 ? 2 : 3)); // GridClass::FogVolume / Staggered (GridBuilder.hpp:181-186)
-	put(g + kOffGridType, lay->grid_type);
-	put(g + 640, int64_t(bytes));                               // blind metadata: none, offset = end of the grid
-	put(g + 656, uint64_t(0));
-	put(g + 664, kMagicGrid);
-	// TreeData
-	uint8_t* t = buf + oTree;
-	put(t + 0, int64_t(oLeaf - oTree));
-	put(t + 8, int64_t(oLower - oTree));
-	put(t + 16, int64_t(oUpper - oTree));
-	put(t + 24, int64_t(oRoot - oTree));
-	put(t + 32, uint32_t(n_leaves)), put(t + 36, uint32_t(nLower)), put(t + 40, uint32_t(T));   // node counts; tile counts stay 0: no active tiles
+	const GridOffsets off(*lay, n_leaves, nLower, T);
+	const uint64_t oRoot = off.root, oUpper = off.upper, oLower = off.lower, oLeaf = off.leaf;
 	uint64_t active = 0;
 	// nodes, walking the sorted leaf list once
 	struct Box {
@@ -458,19 +415,65 @@ int hns_sidecar_to_nanovdb(const int32_t* domain_origins, uint64_t n_leaves, con
 	}
 	if (Lo) loBox.store(Lo), upBox.add(loBox.lo, loBox.hi);
 	if (U) upBox.store(U), rootBox.add(upBox.lo, upBox.hi);
-	put(t + 56, active);
-	uint8_t* r = buf + oRoot;
-	rootBox.store(r);
-	put(r + kRootTableSize, uint32_t(T));
-	for (int d = 0; d < 3; ++d) {                               // world bbox = index bbox (inclusive max + 1 voxel) x scale, as NanoVDB's builders set it
-		const double a = double(rootBox.lo[d]) * s, b = double(n_leaves ? rootBox.hi[d] + 1 : rootBox.hi[d]) * s;
-		put(g + kOffWorldBBox + 8 * d, n_leaves ? std::min(a, b) : 0.0);
-		put(g + kOffWorldBBox + 24 + 8 * d, n_leaves ? std::max(a, b) : 0.0);
-	}
+	write_grid_header(buf, *lay, n_leaves, nLower, T, voxel_size, name, rootBox.lo, rootBox.hi, active);
 	return HNS_OK;
 }
 
 }  // extern "C"
+
+namespace hns::vgrid {
+
+void write_grid_header(uint8_t* buf, const ValueLayout& lay, uint64_t L, uint64_t nLower, uint64_t T, float voxel_size, const char* name,
+                       const int32_t lo[3], const int32_t hi[3], uint64_t active) {
+	auto put = [](uint8_t* p, auto v) { std::memcpy(p, &v, sizeof(v)); };
+	const GridOffsets off(lay, L, nLower, T);
+	const uint64_t oTree = nvdb::kGrid, bytes = off.end;
+	const double s = double(voxel_size);
+	// GridData (GridData::init, NanoVDB.h:1834-1862)
+	uint8_t* g = buf;
+	put(g + 0, kMagicNumb);
+	put(g + 8, ~uint64_t(0));                                   // checksum: disabled
+	put(g + kOffVersion, uint32_t((32u << 21) | (7u << 10)));
+	put(g + 20, uint32_t(0x22));                                // HasBBox | IsBreadthFirst; no min/max, average, std deviation
+	put(g + kOffGridIndex, uint32_t(0));
+	put(g + kOffGridCount, uint32_t(1));
+	put(g + kOffGridSize, bytes);
+	if (name) std::strncpy(reinterpret_cast<char*>(g + kOffName), name, kNameMax - 1);
+	uint8_t* m = g + 296;                                       // Map: matF[9] invMatF[9] vecF[3] taperF matD[9] invMatD[9] vecD[3] taperD
+	for (int d = 0; d < 3; ++d) {
+		put(m + 16 * d, float(s));
+		put(m + 36 + 16 * d, 1.0f / float(s));
+		put(m + 88 + 32 * d, s);
+		put(m + 160 + 32 * d, 1.0 / s);
+	}
+	put(m + 84, 1.0f);
+	put(m + 256, 1.0);
+	for (int d = 0; d < 3; ++d) put(g + kOffVoxelSize + 8 * d, s);
+	put(g + kOffGridClass, uint32_t(lay.components == 1 ? 2 : 3));  // GridClass::FogVolume / Staggered (GridBuilder.hpp:181-186)
+	put(g + kOffGridType, lay.grid_type);
+	put(g + 640, int64_t(bytes));                               // blind metadata: none, offset = end of the grid
+	put(g + 656, uint64_t(0));
+	put(g + 664, kMagicGrid);
+	// TreeData
+	uint8_t* t = buf + oTree;
+	put(t + 0, int64_t(off.leaf - oTree));
+	put(t + 8, int64_t(off.lower - oTree));
+	put(t + 16, int64_t(off.upper - oTree));
+	put(t + 24, int64_t(off.root - oTree));
+	put(t + 32, uint32_t(L)), put(t + 36, uint32_t(nLower)), put(t + 40, uint32_t(T));   // node counts; tile counts stay 0: no active tiles
+	put(t + 56, active);
+	// RootData: bbox, tile count; background and statistics stay 0
+	uint8_t* r = buf + off.root;
+	std::memcpy(r, lo, 12), std::memcpy(r + 12, hi, 12);
+	put(r + kRootTableSize, uint32_t(T));
+	for (int d = 0; d < 3; ++d) {                               // world bbox = index bbox (inclusive max + 1 voxel) x scale, as NanoVDB's builders set it
+		const double a = double(lo[d]) * s, b = double(L ? hi[d] + 1 : hi[d]) * s;
+		put(g + kOffWorldBBox + 8 * d, L ? std::min(a, b) : 0.0);
+		put(g + kOffWorldBBox + 24 + 8 * d, L ? std::max(a, b) : 0.0);
+	}
+}
+
+}  // namespace hns::vgrid
 
 namespace hns {
 

@@ -360,6 +360,13 @@ class ShardedSimulation:
         stream. Collective where it writes the velocity: every rank adds the same sources (include/hns_b200.h, sources)."""
         self.sim.add_source(target, source, self._stream() if stream is None else stream)
 
+    def export_grid(self, target, name: str, tolerance: float = -1.0, out=None, stream=None):
+        """Simulation.export_grid over this rank's OWNED leaves (ghosts never, global leaf 0 only on rank 0), by default on the frame's
+        stream: a valid NanoVDB grid of the rank's slab. Not collective; the ranks' grids are not stitched together."""
+        if not self.native:
+            raise NotImplementedError("the export's owned-leaf list is the native sharded frame's plan (native=True)")
+        return self.sim.export_grid(target, name, tolerance, out, self._stream() if stream is None else stream)
+
     def frame(self, iterations: int, dt: float) -> None:
         if self.native:
             import ctypes as C

@@ -25,7 +25,7 @@ from ._lib import CombustionParams, HnsError, check, c_f32p, c_i32p, c_u64p
 from .grid_data import FLOAT, VEC3F, GridIndexedData
 
 __all__ = ["CreateIndexGrid", "Compute_Sim", "AdvectIndexGrid", "AdvectIndexGridVelocity", "ProjectNonDivergent", "Divergence",
-           "CombustionKernel", "IndexGridHandle", "Simulation", "Multigrid", "Source", "build_domain", "CombustionParams"]
+           "CombustionKernel", "IndexGridHandle", "Simulation", "Multigrid", "Source", "ValueGrid", "build_domain", "CombustionParams"]
 
 
 def _fp(a: np.ndarray):
@@ -286,6 +286,46 @@ class Source:
         return int(n.value)
 
 
+class ValueGrid:
+    """A NanoVDB float or Vec3f grid in device memory, written by Simulation.export_grid (include/hns_b200.h, export). Every export
+    into it replaces the grid; its device block only grows, so a per-frame export into one ValueGrid allocates nothing in steady state."""
+
+    def __init__(self):
+        h = C.c_void_p()
+        check(_lib.lib().hns_value_grid_create(C.byref(h)))
+        self._h = h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            _lib.lib().hns_value_grid_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def nbytes(self) -> int:
+        return int(_lib.lib().hns_value_grid_bytes(self._h))
+
+    @property
+    def num_leaves(self) -> int:
+        return int(_lib.lib().hns_value_grid_num_leaves(self._h))
+
+    @property
+    def device_ptr(self) -> int:
+        """device address of the grid (GridData first); 0 before the first export"""
+        return int(_lib.lib().hns_value_grid_device_ptr(self._h) or 0)
+
+    def download(self) -> np.ndarray:
+        """the grid as a uint8 host buffer (io.write_nvdb, io.sidecar_from_grid and Source take it)"""
+        out = np.empty(self.nbytes, np.uint8)
+        check(_lib.lib().hns_value_grid_download(self._h, out.ctypes.data_as(C.c_void_p), out.size))
+        return out
+
+
 class Simulation:
     """Device-resident state of one simulation: velocity + n_scalars float fields on an index grid."""
 
@@ -330,6 +370,20 @@ class Simulation:
             check(_lib.lib().hns_state_add_source_velocity(self._h, source._h, _stream(stream)))
         else:
             check(_lib.lib().hns_state_add_source_scalar(self._h, int(target), source._h, _stream(stream)))
+
+    def export_grid(self, target, name: str, tolerance: float = -1.0, out: ValueGrid | None = None, stream=None) -> ValueGrid:
+        """writeIndexGrid on the device: the velocity (target "velocity") as a Vec3f grid of class Staggered or scalar `target` (an int)
+        as a float grid of class FogVolume, into `out` (a new ValueGrid when None), which is returned. tolerance < 0: every leaf, every
+        voxel active; tolerance >= 0: only voxels with !(|v| <= tolerance) are active and leaves without one are left out. Ordered after
+        earlier work on `stream`; returns when the grid is complete. The state is not changed."""
+        vg = ValueGrid() if out is None else out
+        if isinstance(target, str):
+            if target != "velocity":
+                raise ValueError(f'target must be "velocity" or a scalar index, not {target!r}')
+            check(_lib.lib().hns_state_export_velocity(self._h, float(tolerance), name.encode(), vg._h, _stream(stream)))
+        else:
+            check(_lib.lib().hns_state_export_scalar(self._h, int(target), float(tolerance), name.encode(), vg._h, _stream(stream)))
+        return vg
 
     def velocity(self) -> np.ndarray:
         out = np.empty((self.n, 3), np.float32)

@@ -217,6 +217,36 @@ int hns_source_leaves_outside(const hns_source* src, const hns_grid* g, uint64_t
 int hns_state_add_source_velocity(hns_state* s, const hns_source* src, void* stream);          /* Vec3f source */
 int hns_state_add_source_scalar(hns_state* s, int index, const hns_source* src, void* stream); /* float source */
 
+/* ---------------------------------------------------------------------------------------------------------
+ * Export of resident fields: IndexGridBuilder::writeIndexGrid (src/Utils/GridBuilder.hpp:168-216, SOP_HNanoSolver.cpp:258-268) built
+ * on the device, into a NanoVDB grid in device memory that a renderer or another solver can read there, or that is downloaded for a
+ * cache file (hns_nvdb_write). A scalar becomes a float grid of class FogVolume, the velocity a Vec3f grid of class Staggered; the
+ * bytes are those hns_sidecar_to_nanovdb writes over the same leaves, values and masks: background 0, no statistics, checksum disabled.
+ *   tolerance < 0   the whole domain: every leaf, every voxel active (= hns_sidecar_to_nanovdb over the downloaded field).
+ *   tolerance >= 0  pruned: a voxel is active iff !(|v| <= tolerance) (Vec3f: any component; NaN is active). A leaf without an active
+ *                   voxel is left out, a kept leaf keeps all 512 values; nodes and root tiles left without children disappear. With
+ *                   tolerance 0 reading the grid back over the domain (hns_sidecar_from_nanovdb, fill 0) returns the field, except that a
+ *                   dropped leaf of -0.0 values comes back as +0.0. Nothing kept: the empty grid (800 bytes float, 832 bytes Vec3f).
+ * The leaves are those the state's kernels process: every leaf on one GPU, the owned leaves of a sharded state (hns_dist_set_plan;
+ * ghost leaves, and global leaf 0 on ranks other than 0, are never exported), so each rank's grid is a valid grid of its slab.
+ * The export reads the state and changes nothing in it. It is ordered after earlier work on `stream`, reads the kept-leaf and node
+ * counts back with one small copy and returns when the grid is complete. HNS_ERR_INVALID_ARGUMENT: a NaN tolerance (refused before any
+ * CUDA call), a null argument, a scalar index out of range, a value grid bound to another device than the state's. `name` is truncated
+ * to 255 bytes, as by hns_sidecar_to_nanovdb.
+ * ------------------------------------------------------------------------------------------------------- */
+typedef struct hns_value_grid hns_value_grid;   /* a NanoVDB float / Vec3f grid in device memory, refilled by every export into it */
+/* An empty value grid (no CUDA call). Its device block is allocated by the first export and grows only when an export needs more, so
+ * exporting a field every frame into the same handle allocates nothing in steady state. It binds to the device of its first export. */
+int hns_value_grid_create(hns_value_grid** out);
+void hns_value_grid_destroy(hns_value_grid* vg);
+uint64_t hns_value_grid_bytes(const hns_value_grid* vg);          /* size of the grid of the last export, 0 before the first */
+uint64_t hns_value_grid_num_leaves(const hns_value_grid* vg);
+const void* hns_value_grid_device_ptr(const hns_value_grid* vg);  /* the grid (GridData first), null before the first export */
+/* copies the grid to the host (capacity >= hns_value_grid_bytes); synchronous */
+int hns_value_grid_download(const hns_value_grid* vg, void* dst_host, uint64_t capacity);
+int hns_state_export_velocity(hns_state* s, float tolerance, const char* name, hns_value_grid* out, void* stream);
+int hns_state_export_scalar(hns_state* s, int index, float tolerance, const char* name, hns_value_grid* out, void* stream);
+
 /* Enables the combustion_oxygen + temperature_buoyancy stage of the all-in-one frame (src/Cuda/HNanoSolver.cu:190-250) on the
  * scalar fields with the given indices, and the vorticityConfinement pass (Kernel.cu:969-1025) between advect_vector and the
  * divergence when params->vorticityScale != 0 and (int)params->factorScale != 0. The reference runs that kernel in place
