@@ -88,6 +88,8 @@ SIGNATURES = {
     "hns_value_grid_download": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
     "hns_state_export_velocity": (C.c_int, [C.c_void_p, C.c_float, C.c_char_p, C.c_void_p, C.c_void_p]),
     "hns_state_export_scalar": (C.c_int, [C.c_void_p, C.c_int, C.c_float, C.c_char_p, C.c_void_p, C.c_void_p]),
+    "hns_state_domain_build": (C.c_int, [C.c_void_p, C.c_float, C.c_int, C.c_int, C.POINTER(C.c_void_p), c_i32p, C.c_uint64, C.POINTER(C.c_void_p)]),
+    "hns_state_create_remapped": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "hns_state_set_combustion": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(CombustionParams)]),
     "hns_state_step": (C.c_int, [C.c_void_p, C.c_int, C.c_float, C.c_uint, C.c_void_p]),
     "hns_state_advect_velocity": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p]),

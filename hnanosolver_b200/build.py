@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libhns_b200.so")
 SOURCES = ["topology.cu", "kernels.cu", "api.cu", "dist.cu", "nvdb_io.cu", "multigrid.cu", "advect.cu", "domain.cu", "export.cu"]
-HEADERS = ["common.cuh", "kernels.cuh", "sampling.cuh", "nvdb_layout.cuh", os.path.join("..", "..", "include", "hns_b200.h")]
+HEADERS = ["common.cuh", "kernels.cuh", "sampling.cuh", "nvdb_layout.cuh", "classify.cuh", os.path.join("..", "..", "include", "hns_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

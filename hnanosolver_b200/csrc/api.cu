@@ -501,9 +501,10 @@ int hns_source_create(const void* buffer, uint64_t bytes, hns_source** out) {
 	cudaError_t e = cudaGetDevice(&src->device);
 	if (e == cudaSuccess && L) {
 		if ((e = cudaMalloc(&src->keys, L * sizeof(ulonglong2))) == cudaSuccess && (e = cudaMalloc(&src->origins, L * sizeof(int4))) == cudaSuccess &&
-		    (e = cudaMalloc(&src->values, t.values.size() * sizeof(float))) == cudaSuccess &&
+		    (e = cudaMalloc(&src->values, t.values.size() * sizeof(float))) == cudaSuccess && (e = cudaMalloc(&src->masks, L * 64)) == cudaSuccess &&
 		    (e = cudaMemcpy(src->keys, t.keys.data(), L * sizeof(ulonglong2), cudaMemcpyHostToDevice)) == cudaSuccess &&
-		    (e = cudaMemcpy(src->origins, t.origins.data(), L * sizeof(int4), cudaMemcpyHostToDevice)) == cudaSuccess)
+		    (e = cudaMemcpy(src->origins, t.origins.data(), L * sizeof(int4), cudaMemcpyHostToDevice)) == cudaSuccess &&
+		    (e = cudaMemcpy(src->masks, t.masks.data(), L * 64, cudaMemcpyHostToDevice)) == cudaSuccess)
 			e = cudaMemcpy(src->values, t.values.data(), t.values.size() * sizeof(float), cudaMemcpyHostToDevice);
 	}
 	if (e != cudaSuccess) {
@@ -515,7 +516,7 @@ int hns_source_create(const void* buffer, uint64_t bytes, hns_source** out) {
 }
 void hns_source_destroy(hns_source* src) {
 	if (!src) return;
-	cudaFree(src->keys), cudaFree(src->origins), cudaFree(src->values);
+	cudaFree(src->keys), cudaFree(src->origins), cudaFree(src->values), cudaFree(src->masks);
 	delete src;
 }
 int hns_source_components(const hns_source* src) { return src ? src->components : 0; }

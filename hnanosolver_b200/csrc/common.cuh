@@ -92,12 +92,14 @@ __host__ __device__ inline ulonglong2 nvdb_leaf_key(int32_t x, int32_t y, int32_
 __host__ __device__ inline bool key_less(const ulonglong2& a, const ulonglong2& b) { return a.x < b.x || (a.x == b.x && a.y < b.y); }
 
 // A source grid's leaves on the host, validated and sorted by nvdb_leaf_key (nvdb_io.cu, source_tables): what hns_source_create copies
-// to the device. values: float[L][512 * components], each leaf's 512 values as the grid stores them (Vec3f: AoS).
+// to the device. values: float[L][512 * components], each leaf's 512 values as the grid stores them (Vec3f: AoS); masks: uint64[L][8], each
+// leaf's value mask (word x, bit y * 8 + z), the source's topology for hns_state_domain_build.
 struct SourceTables {
 	int components = 0;
 	std::vector<ulonglong2> keys;
 	std::vector<int4> origins;  // (x, y, z, 0)
 	std::vector<float> values;
+	std::vector<uint64_t> masks;
 };
 int source_tables(const void* buffer, uint64_t bytes, SourceTables& out);
 
@@ -254,4 +256,5 @@ struct hns_source {
 	ulonglong2* keys = nullptr;  // [L], ascending
 	int4* origins = nullptr;     // [L]
 	float* values = nullptr;     // [L][512 * components]
+	uint64_t* masks = nullptr;   // [L][8] value masks
 };

@@ -510,11 +510,12 @@ int source_tables(const void* buffer, uint64_t bytes, SourceTables& out) {
 	const int C = w.lay->components;
 	const size_t leaf_floats = size_t(512) * C;
 	out.components = C;
-	out.keys.resize(L), out.origins.resize(L), out.values.resize(L * leaf_floats);
+	out.keys.resize(L), out.origins.resize(L), out.values.resize(L * leaf_floats), out.masks.resize(L * 8);
 	for (uint64_t i = 0; i < L; ++i) {
 		const uint32_t l = order[i];
 		out.keys[i] = keys[l], out.origins[i] = origins[l];
 		std::memcpy(out.values.data() + i * leaf_floats, tree + leaf_off + l * w.lay->leaf + w.lay->leaf_values, leaf_floats * sizeof(float));
+		std::memcpy(out.masks.data() + i * 8, tree + leaf_off + l * w.lay->leaf + kLeafValueMask, 64);
 	}
 	return HNS_OK;
 }

@@ -385,6 +385,33 @@ class Simulation:
             check(_lib.lib().hns_state_export_scalar(self._h, int(target), float(tolerance), name.encode(), vg._h, _stream(stream)))
         return vg
 
+    def redomain(self, tolerance: float, padding: int, sources=(), sdf_origins=None, stream=None) -> "Simulation":
+        """The SOP's domain step for a resident state: a new Simulation on a new grid whose leaves are the velocity's leaf topology at
+        `tolerance` (as export_grid("velocity", tolerance) writes it; tolerance < 0: every leaf, every voxel) united with the leaves of
+        `sources` (Source objects), dilated by `padding` voxels, plus the collider's leaf origins `sdf_origins`. The velocity and every
+        scalar are carried over bit for bit where the old grid has the leaf; new leaves hold 0, or bytes 0x01 in the collision SDF.
+        Combustion, vorticity and the collision scalar are carried over, a multigrid solver is not (the new state solves red-black).
+        Work on `stream` is finished first; `stream` is synchronised before returning, so this object may be dropped at once."""
+        L = _lib.lib()
+        so = np.zeros((0, 3), np.int32) if sdf_origins is None else np.ascontiguousarray(np.asarray(sdf_origins, np.int32).reshape(-1, 3))
+        srcs = (C.c_void_p * max(1, len(sources)))(*[s._h.value for s in sources])
+        self.sync(stream)
+        d = C.c_void_p()
+        check(L.hns_state_domain_build(self._h, float(tolerance), int(padding), len(sources), srcs, _ip(so) if len(so) else None, so.shape[0],
+                                       C.byref(d)))
+        try:
+            g = C.c_void_p()
+            check(L.hns_domain_create_grid(d, L.hns_grid_voxel_size(self.grid._h), C.byref(g)))
+        finally:
+            L.hns_domain_destroy(d)
+        grid = IndexGridHandle(g.value)
+        h = C.c_void_p()
+        check(L.hns_state_create_remapped(self._h, grid._h, _stream(stream), C.byref(h)))
+        out = Simulation.__new__(Simulation)
+        out.grid, out.n, out.n_scalars, out._h = grid, grid.num_voxels, self.n_scalars, h
+        out.sync(stream)
+        return out
+
     def velocity(self) -> np.ndarray:
         out = np.empty((self.n, 3), np.float32)
         check(_lib.lib().hns_state_download_velocity(self._h, _fp(out)))

@@ -247,6 +247,36 @@ int hns_value_grid_download(const hns_value_grid* vg, void* dst_host, uint64_t c
 int hns_state_export_velocity(hns_state* s, float tolerance, const char* name, hns_value_grid* out, void* stream);
 int hns_state_export_scalar(hns_state* s, int index, float tolerance, const char* name, hns_value_grid* out, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * Re-domaining resident state: the domain step of SOP_HNanoSolverVerb::cook (src/SOP/HNanoSolver/SOP_HNanoSolver.cpp:188-199) and the
+ * rebuild of the sidecar over the new domain (IndexGridBuilder::build, src/Utils/GridBuilder.hpp:87-166) for a state that stays on the
+ * device, so that its domain follows the fluid between frames. Single-GPU states only: a sharded state (hns_dist_set_plan) is
+ * HNS_ERR_UNSUPPORTED. The old state is only read; it stays valid and unchanged.
+ * ------------------------------------------------------------------------------------------------------- */
+/* The new domain: hns_domain_build(origins, masks, padding, sdf_origins) where (origins, masks) is the union of
+ *   - the velocity's leaf topology as hns_state_export_velocity(s, tolerance) writes it: tolerance >= 0, a voxel is active iff
+ *     !(|v| <= tolerance) in any component (NaN is active) and leaves without an active voxel are absent; tolerance < 0, every leaf with
+ *     every voxel active;
+ *   - every source's leaves and value masks (compSum's topology union: a source outside the domain pulls the domain to itself).
+ * sources: n_sources handles (hns_source_create), none NULL; sdf_origins: HOST int32[n_sdf][3] collider leaf origins (may be NULL with
+ * n_sdf = 0). Refused before any CUDA call: a NaN tolerance, padding outside [0, 64], a null argument or source entry
+ * (HNS_ERR_INVALID_ARGUMENT); collider origins that are not multiples of 8 (HNS_ERR_TOPOLOGY) or beyond +-(2^23 - 128) voxels
+ * (HNS_ERR_UNSUPPORTED); a source on another device than the state (HNS_ERR_INVALID_ARGUMENT). An origin of the state or of a source
+ * beyond +-(2^23 - 128) voxels is HNS_ERR_UNSUPPORTED. Runs on the legacy default stream and is synchronous (it reads the leaf count
+ * back): a caller that stepped the state on another stream synchronises that stream first. The result feeds hns_domain_origins /
+ * hns_domain_create_grid. */
+int hns_state_domain_build(const hns_state* s, float tolerance, int padding, int n_sources, const hns_source* const* sources, const int32_t* sdf_origins,
+                           uint64_t n_sdf, hns_domain** out);
+/* A new state on grid g (allocated as hns_state_create(g, n_scalars of src) leaves it) with src's fields remapped onto g's leaves: per
+ * leaf of g, for the velocity and every scalar, the 512 values of src's leaf at that origin bit for bit, or, where src's grid has no
+ * leaf there, 512 values whose bytes are 0 (0x01 for the collision SDF scalar of hns_state_set_collision, GridBuilder.hpp:108): what
+ * hns_sidecar_from_nanovdb makes of a whole-domain export of the field. Carried over: the combustion configuration
+ * (hns_state_set_combustion, vorticity included) and the collision scalar. Not carried over: a multigrid pressure solver (its hierarchy
+ * belongs to the old grid; the new state solves red-black until hns_state_set_pressure_solver is called). Pressure, divergence, the
+ * advected velocity and the packed advection groups start as hns_state_create leaves them. The remap is enqueued on `stream` (one
+ * launch); src and its grid must outlive that work. HNS_ERR_INVALID_ARGUMENT: a null argument, a grid on another device than src's. */
+int hns_state_create_remapped(const hns_state* src, const hns_grid* g, void* stream, hns_state** out);
+
 /* Enables the combustion_oxygen + temperature_buoyancy stage of the all-in-one frame (src/Cuda/HNanoSolver.cu:190-250) on the
  * scalar fields with the given indices, and the vorticityConfinement pass (Kernel.cu:969-1025) between advect_vector and the
  * divergence when params->vorticityScale != 0 and (int)params->factorScale != 0. The reference runs that kernel in place
